@@ -51,7 +51,16 @@ def parse():
     ap.add_argument("--ppo-large", type=int, default=8192,
                     help="second PPO leg: 65 536 envs / 8 GPUs = 8 192 trajectories per GPU in one update (0 = skip)")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (rank 0) as DIR/<name>.npy in "
+                         "float32: a fixed, seeded sample of environments, the same for every array, all of them if they "
+                         "fit in 64 MB")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return a
 
 
 def config_dict(a, world):
@@ -66,6 +75,25 @@ def input_bytes(n, T):
     ld = (n + 3) // 4 * 4
     rows = 27 + 26 + 49 + 72 + 96 + 240 + 144 + 20 + 1 + 1 + 46 + 20 + 1 + 1 + 6 + 10
     return rows * 4 * ld * T
+
+
+DUMP_BYTES = 64 * 10**6
+
+
+def dump_outputs(out_dir, arrays, n):
+    """Write arrays (name -> (tensor, axis of the environment index)) as out_dir/<name>.npy in float32.  Every array keeps
+    the same environments: all n if they fit in DUMP_BYTES, else a sample drawn with a fixed seed, so that two builds run
+    with the same arguments can be compared file by file."""
+    import numpy as np
+    import torch
+
+    per_env = sum(4 * t.numel() // t.shape[ax] for t, ax in arrays.values())
+    k = min(n, DUMP_BYTES // per_env)
+    idx = np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, (t, ax) in arrays.items():
+        sel = torch.from_numpy(idx).to(t.device)
+        np.save(os.path.join(out_dir, name + ".npy"), t.index_select(ax, sel).float().cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -377,6 +405,16 @@ def run_b200(a):
     ms_step = ms_total / a.steps
     value = world * N * T / (ms_step * 1e-3)
     assert torch.isfinite(adv).all() and torch.isfinite(total).all(), "non-finite outputs"
+    if a.dump_outputs and rank == 0:
+        # the passes below run the step again: take its outputs now.  command row 0 is the input of the next step.
+        dump_outputs(a.dump_outputs, {
+            "action": (io["action"], 2), "log_prob": (io["log_prob"], 1), "ctrl": (io["ctrl"], 2),
+            "done": (io["done"], 1), "success": (io["success"], 1), "value": (io["value"], 1),
+            "command": (io["command"][1:], 2), "pg_carry": (io["pg_carry"], 1), "lpf": (io["lpf"], 1),
+            "actor_carry": (io["actor_carry"], 2), "critic_carry": (io["critic_carry"], 2),
+            "reward_total": (total, 1), "reward_t_single": (rcarry["t_single"], 0),
+            "reward_airtime": (rcarry["airtime"], 1), "reward_prev_contact": (rcarry["prev_contact"], 1),
+            "advantages": (adv, 1), "value_targets": (tgt, 1)}, N)
 
     # ---- per-kernel pass (CUDA events around every launch, same step) -> roofline of the dominant kernel ----------
     eng.profile(True)

@@ -13,7 +13,8 @@ can be imported in the build container or on the GPU box.  This script closes th
                                                 tests/test_oracle_cpu.py::test_reference_goldens_when_present does the same
   python tools/verify_against_ref.py            report: which [U] items are pinned, which are not, and why
 
-Nothing here is imported by the product, and nothing in the GPU tests / bench reads /root/reference at run time.
+Nothing here is imported by the product, and nothing in the tests or the bench reads the reference at run time: a
+reference checkout is found through PYTHONPATH (or baseline/_ref/), never through a fixed path outside the repository.
 An item that cannot be produced (API of the fork differs from what is assumed here) is reported with the exception text
 instead of aborting the run, so that one unknown signature does not block the other items.
 """
@@ -32,7 +33,7 @@ import numpy as np
 ROOT = Path(__file__).resolve().parent.parent
 GOLDEN = ROOT / "tests" / "golden"
 REQUIRED = ("jax", "ksim", "xax", "equinox", "distrax")
-for _p in (ROOT, ROOT / "oracle", ROOT / "baseline" / "_ref", Path("/root/reference")):
+for _p in (ROOT, ROOT / "oracle", ROOT / "baseline" / "_ref"):
     if _p.exists() and str(_p) not in sys.path:
         sys.path.append(str(_p))
 
