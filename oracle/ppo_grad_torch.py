@@ -44,15 +44,21 @@ def trunk(w, obs, carry):
 
 
 def ppo_minibatch_loss(wa, wc, actor_obs, critic_obs, action, done, old_log_probs, advantages, value_targets, old_values,
-                       p: O.OracleParams, hyper: dict):
-    """All inputs numpy [T, N, ...].  Returns (loss, (mean policy, mean value, mean entropy), log_probs, values)."""
+                       p: O.OracleParams, hyper: dict, carry0: dict | None = None):
+    """All inputs numpy [T, N, ...].  carry0: the carries at the first step, {"actor", "critic": [N, depth, 2, H],
+    "lpf_params": [N, 20]} (None = zeros, get_initial_model_carry).
+    Returns (loss, (mean policy, mean value, mean entropy), log_probs, values)."""
     T, N = done.shape
     H, depth = p.hidden_size, p.depth
     a_obs, c_obs, act = _t(actor_obs), _t(critic_obs), _t(action)
     keep = _t(1.0 - done.astype(np.float64))
-    ca = torch.zeros((N, depth, 2, H), dtype=torch.float64)
-    cc = torch.zeros((N, depth, 2, H), dtype=torch.float64)
-    lpf = torch.zeros((N, O.NUM_JOINTS), dtype=torch.float64)
+    if carry0 is None:
+        ca = torch.zeros((N, depth, 2, H), dtype=torch.float64)
+        cc = torch.zeros((N, depth, 2, H), dtype=torch.float64)
+        lpf = torch.zeros((N, O.NUM_JOINTS), dtype=torch.float64)
+    else:
+        ca, cc, lpf = _t(carry0["actor"]), _t(carry0["critic"]), _t(carry0["lpf_params"])
+        assert ca.shape == cc.shape == (N, depth, 2, H) and lpf.shape == (N, O.NUM_JOINTS)
     jb = _t(O.joint_biases(np.float64))
     lps, ents, vals = [], [], []
     for t in range(T):
@@ -82,14 +88,16 @@ def ppo_minibatch_loss(wa, wc, actor_obs, critic_obs, action, done, old_log_prob
     return -obj.mean(), (pol.mean(), vl.mean(), ent.mean()), lp, val
 
 
-def ppo_minibatch_grads(w_actor: dict, w_critic: dict, batch: dict, p: O.OracleParams, hyper: dict | None = None):
+def ppo_minibatch_grads(w_actor: dict, w_critic: dict, batch: dict, p: O.OracleParams, hyper: dict | None = None,
+                        carry0: dict | None = None):
     """batch: actor_obs [T,N,65], critic_obs [T,N,475], action [T,N,20], done [T,N] bool, old_log_probs, advantages,
-    value_targets, old_values [T,N].  Returns (loss, stats, grads_actor, grads_critic) with grads in the eqx layout."""
+    value_targets, old_values [T,N]; carry0 as in ppo_minibatch_loss.  Returns (loss, stats, grads_actor, grads_critic,
+    log_probs, values) with grads in the eqx layout."""
     hyper = hyper or {}
     wa, wc = weights_to_torch(w_actor), weights_to_torch(w_critic)
     loss, stats, lp, val = ppo_minibatch_loss(wa, wc, batch["actor_obs"], batch["critic_obs"], batch["action"], batch["done"],
                                               batch["old_log_probs"], batch["advantages"], batch["value_targets"],
-                                              batch["old_values"], p, hyper)
+                                              batch["old_values"], p, hyper, carry0)
     loss.backward()
 
     def grads(w):

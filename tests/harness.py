@@ -102,8 +102,10 @@ def scaled_err(gpu, ref, rtol=RTOL, atol=1e-6) -> float:
     return float(np.max(np.abs(gpu - ref) / (rtol * np.abs(ref) + atol)))
 
 
-def rollout_buffers(b: "Batch", hidden: int, depth: int, with_critic: bool = True) -> dict:
-    """Device buffers of kbs_rollout_io for batch b (zero-initialised carries = get_initial_model_carry)."""
+def rollout_buffers(b: "Batch", hidden: int, depth: int, with_critic: bool = True, start: dict | None = None) -> dict:
+    """Device buffers of kbs_rollout_io for batch b: zero-initialised carries (= get_initial_model_carry), or the
+    mid-episode state `start` {"actor", "critic" [N, depth, 2, H], "lpf_params" [N, 20], "pg_carry" [N, 3], "command" [N, 16]}
+    (oracle layout)."""
     T, N, ld, dev = b.T, b.N, b.ld, b.dev
     f = dict(device=dev, dtype=torch.float32)
     command = torch.zeros((T + 1, 16, ld), **f)
@@ -123,16 +125,29 @@ def rollout_buffers(b: "Batch", hidden: int, depth: int, with_critic: bool = Tru
         "success": torch.zeros((T, ld), device=dev, dtype=torch.uint8),
         "value": torch.zeros((T, ld), **f) if with_critic else None, "T": T,
     }
+    if start is not None:
+        command[0] = synth.to_soa(start["command"], 0, dev)
+        io["pg_carry"] = synth.to_soa(start["pg_carry"], 0, dev)
+        io["lpf"] = synth.to_soa(start["lpf_params"], 0, dev)
+        io["actor_carry"] = carry_from_np(start["actor"], dev)
+        if with_critic:
+            io["critic_carry"] = carry_from_np(start["critic"], dev)
     return io
 
 
-def oracle_rollout(b: "Batch", wa, wc, hidden: int, depth: int, with_critic: bool = True, p=None) -> dict:
+def oracle_rollout(b: "Batch", wa, wc, hidden: int, depth: int, with_critic: bool = True, p=None, start: dict | None = None) -> dict:
+    """O.rollout_control_steps over batch b from zero carries, or from `start` (as in rollout_buffers)."""
     p = p or O.OracleParams(hidden_size=hidden, depth=depth)
     N = b.N
-    carry = {"actor": np.zeros((N, depth, 2, hidden), np.float32), "critic": np.zeros((N, depth, 2, hidden), np.float32),
-             "lpf_params": np.zeros((N, 20), np.float32)}
-    return O.rollout_control_steps(wa, wc, b.np["state"], b.np["noise"], b.np["episode"], b.np["cmd_rand"], b.cmd0_np,
-                                   carry, np.zeros((N, 3), np.float32), p, with_critic=with_critic)
+    if start is None:
+        carry = {"actor": np.zeros((N, depth, 2, hidden), np.float32), "critic": np.zeros((N, depth, 2, hidden), np.float32),
+                 "lpf_params": np.zeros((N, 20), np.float32)}
+        cmd0, pg = b.cmd0_np, np.zeros((N, 3), np.float32)
+    else:
+        carry = {k: start[k] for k in ("actor", "critic", "lpf_params")}
+        cmd0, pg = start["command"], start["pg_carry"]
+    return O.rollout_control_steps(wa, wc, b.np["state"], b.np["noise"], b.np["episode"], b.np["cmd_rand"], cmd0,
+                                   carry, pg, p, with_critic=with_critic)
 
 
 def compare_rollout(io: dict, ref: dict, N: int, with_critic: bool = True) -> dict:
@@ -176,8 +191,10 @@ def run_rollout_case(seed: int, T: int, N: int, hidden: int, device, gemm_path=L
     return out
 
 
-def ppo_batch(rng, T, N, H, p, wa, wc):
-    """A stored minibatch with old log-probs / values taken near the current policy (so both clip branches occur)."""
+def ppo_batch(rng, T, N, H, p, wa, wc, carry0=None):
+    """A stored minibatch with old log-probs / values taken near the current policy (so both clip branches occur).
+    carry0 (oracle layout, see ppo_grad_torch.ppo_minibatch_loss): the start state the minibatch is evaluated from -- the
+    old log-probs / values must come from the same one, or every ratio lands far from 1 and the policy gradient clips to 0."""
     import ppo_grad_torch as G
 
     f = np.float32
@@ -185,23 +202,81 @@ def ppo_batch(rng, T, N, H, p, wa, wc):
          "action": (0.3 * rng.normal(size=(T, N, 20))).astype(f), "done": rng.random((T, N)) < 0.12,
          "advantages": rng.normal(size=(T, N)).astype(f), "value_targets": rng.normal(0, 0.5, (T, N)).astype(f),
          "old_log_probs": np.zeros((T, N), f), "old_values": np.zeros((T, N), f)}
-    _, _, _, _, lp, val = G.ppo_minibatch_grads(wa, wc, b, p)
+    _, _, _, _, lp, val = G.ppo_minibatch_grads(wa, wc, b, p, carry0=carry0)
     b["old_log_probs"] = (lp + rng.normal(0, 0.15, (T, N))).astype(f)
     b["old_values"] = (val + rng.normal(0, 0.25, (T, N))).astype(f)
     return b
 
 
-def run_ppo_grad_case(dev, T, N, hidden, path) -> list:
-    """kbs_ppo_grad on a seeded minibatch against torch.autograd in float64 (oracle/ppo_grad_torch.py): asserts log-probs, values
-    and loss statistics, returns the list of gradient tensors further than 3e-4 of their scale from the reference."""
+GATES = "ifgo"
+
+
+def grad_blocks(net: str, key: str, H: int) -> list:
+    """(label, row slice) blocks of one gradient tensor that the block-wise check bounds on their own scale: the i / f / g / o
+    rows of an LSTM matrix or bias, the mean rows 0..19 and std rows 20..39 of the actor's output layer."""
+    if key in ("w_ih", "w_hh", "b"):
+        return [(g, slice(k * H, (k + 1) * H)) for k, g in enumerate(GATES)]
+    if net == "actor" and key in ("w_out", "b_out"):
+        return [("mean", slice(0, 20)), ("std", slice(20, 40))]
+    return [("all", slice(None))]
+
+
+def block_bound(ref_block: np.ndarray, ref_tensor: np.ndarray) -> float:
+    """Rows of a weight-gradient GEMM each accumulate their own rows of dG, so their rounding scales with their own block."""
+    return 3e-4 * float(np.abs(ref_block).max()) + 1e-6 * float(np.abs(ref_tensor).max()) + 1e-12
+
+
+def grad_tensors(g: dict, depth: int):
+    """(name, key, layer, array) over every tensor of an eqx-layout gradient dict (numpy or torch)."""
+    a = lambda x: x.detach().cpu().numpy() if torch.is_tensor(x) else np.asarray(x)
+    for k in ("w_in", "b_in", "w_out", "b_out"):
+        yield k, k, a(g[k])
+    for l in range(depth):
+        for k in ("w_ih", "w_hh", "b"):
+            yield f"layers[{l}].{k}", k, a(g["layers"][l][k])
+
+
+def compare_grads_blockwise(got: dict, ref: dict, net: str, H: int, depth: int) -> list:
+    """Every gradient tensor within 3e-4 of its scale (+1e-9), and every block of it within block_bound.  Returns the
+    failures as strings."""
+    bad = []
+    for (name, key, g), (_, _, r) in zip(grad_tensors(got, depth), grad_tensors(ref, depth)):
+        if not np.isfinite(g).all():
+            bad.append(f"{net}.{name}: non-finite")
+            continue
+        err, scale = np.abs(g - r).max(), np.abs(r).max()
+        if not err <= 3e-4 * scale + 1e-9:
+            bad.append(f"{net}.{name}: max err {err:.3e} vs scale {scale:.3e}")
+        for lab, rows in grad_blocks(net, key, H):
+            e, bound = np.abs(g[rows] - r[rows]).max(), block_bound(r[rows], r)
+            if not e <= bound:
+                bad.append(f"{net}.{name}[{lab}]: max err {e:.3e} vs bound {bound:.3e} (block scale {np.abs(r[rows]).max():.3e})")
+    return bad
+
+
+def ppo_device_batch(b: dict, dev, carry0=None) -> dict:
+    """The library's form of a ppo_batch minibatch: SoA arrays, carries at the first step in the ABI layout."""
+    d = lambda a, dt=None: synth.to_soa(a if dt is None else a.astype(dt), 1, dev)
+    batch = {"actor_obs": d(b["actor_obs"]), "critic_obs": d(b["critic_obs"]), "action": d(b["action"]),
+             "done": d(b["done"], np.uint8), "old_log_probs": d(b["old_log_probs"]), "advantages": d(b["advantages"]),
+             "value_targets": d(b["value_targets"]), "old_values": d(b["old_values"])}
+    if carry0 is not None:
+        batch["actor_carry0"] = carry_from_np(carry0["actor"], dev)
+        batch["critic_carry0"] = carry_from_np(carry0["critic"], dev)
+        batch["lpf0"] = synth.to_soa(carry0["lpf_params"], 0, dev)
+    return batch
+
+
+def ppo_grad_compare(e, wa, wc, b: dict, p, dev, N: int, carry0=None, hyper=None) -> tuple:
+    """kbs_ppo_grad on minibatch b (from carry0, with loss hyper-parameters hyper) against torch.autograd in float64
+    (oracle/ppo_grad_torch.py): asserts log-probs, values and loss statistics; returns (the list of gradient tensors /
+    blocks outside their bound, the reference (loss, stats, grads_actor, grads_critic, log_probs, values))."""
     import ppo_grad_torch as G
 
     S = synth.from_soa
-    e, wa, wc = make_engine(hidden=hidden, gemm_path=path, device=dev)
-    p = O.OracleParams(hidden_size=hidden)
-    rng = np.random.default_rng(90 + N)
-    b = ppo_batch(rng, T, N, hidden, p, wa, wc)
-    loss, stats, ga_ref, gc_ref, lp_ref, val_ref = G.ppo_minibatch_grads(wa, wc, b, p)
+    hyper = hyper or {}
+    ref = G.ppo_minibatch_grads(wa, wc, b, p, hyper=hyper, carry0=carry0)
+    loss, stats, ga_ref, gc_ref, lp_ref, val_ref = ref
 
     def nan_like_w(w):
         z = lambda a: torch.full(a.shape, float("nan"), device=dev)
@@ -209,31 +284,25 @@ def run_ppo_grad_case(dev, T, N, hidden, path) -> list:
                 "layers": [{k: z(l[k]) for k in ("w_ih", "w_hh", "b")} for l in w["layers"]]}
 
     ga, gc = nan_like_w(wa), nan_like_w(wc)
-    d = lambda a, dt=None: synth.to_soa(a if dt is None else a.astype(dt), 1, dev)
-    batch = {"actor_obs": d(b["actor_obs"]), "critic_obs": d(b["critic_obs"]), "action": d(b["action"]),
-             "done": d(b["done"], np.uint8), "old_log_probs": d(b["old_log_probs"]), "advantages": d(b["advantages"]),
-             "value_targets": d(b["value_targets"]), "old_values": d(b["old_values"])}
-    out = e.ppo_grad(batch, ga, gc, n_envs=N)
+    out = e.ppo_grad(ppo_device_batch(b, dev, carry0), ga, gc, n_envs=N, **hyper)
     torch.cuda.synchronize()
     assert e.device_status() == 0
     close(S(out["log_probs"], N), lp_ref, "log_probs", atol=1e-4)
     close(S(out["values"], N), val_ref, "values", atol=1e-5)
     close(out["stats"].cpu().numpy(), np.array((loss,) + stats, np.float32), "loss stats", rtol=2e-5, atol=1e-5)
+    bad = (compare_grads_blockwise(ga, ga_ref, "actor", p.hidden_size, p.depth) +
+           compare_grads_blockwise(gc, gc_ref, "critic", p.hidden_size, p.depth))
+    return bad, ref
 
-    bad = []
 
-    def check(name, got, ref):
-        got = got.cpu().numpy()
-        scale = np.abs(ref).max()
-        err = np.abs(got - ref).max()
-        if not (np.isfinite(got).all() and err <= 3e-4 * scale + 1e-9):
-            bad.append(f"{name}: max err {err:.3e} vs scale {scale:.3e}")
-
-    for nm, g, r in (("actor", ga, ga_ref), ("critic", gc, gc_ref)):
-        for k in ("w_in", "b_in", "w_out", "b_out"):
-            check(f"{nm}.{k}", g[k], r[k])
-        for l in range(2):
-            for k in ("w_ih", "w_hh", "b"):
-                check(f"{nm}.layers[{l}].{k}", g["layers"][l][k], r["layers"][l][k])
-    e.close()
-    return bad
+def run_ppo_grad_case(dev, T, N, hidden, path, carry0=None, hyper=None, depth=2) -> list:
+    """kbs_ppo_grad on a seeded minibatch against torch.autograd in float64 (ppo_grad_compare): asserts log-probs, values
+    and loss statistics, returns the list of gradient tensors (or gate / mean / std blocks of them) outside their bound."""
+    e, wa, wc = make_engine(hidden=hidden, depth=depth, gemm_path=path, device=dev)
+    p = O.OracleParams(hidden_size=hidden, depth=depth)
+    rng = np.random.default_rng(90 + N)
+    b = ppo_batch(rng, T, N, hidden, p, wa, wc, carry0=carry0)
+    try:
+        return ppo_grad_compare(e, wa, wc, b, p, dev, N, carry0=carry0, hyper=hyper)[0]
+    finally:
+        e.close()

@@ -315,3 +315,67 @@ def test_reference_goldens_when_present():
         pytest.skip("no reference goldens committed: parity unpinned (oracle-defined, reference-unverified)")
     bad = {k: v for k, v in pinned.items() if v["status"] != "verified"}
     assert not bad, bad
+
+
+def _random_carry(rng, N, depth, H, dtype=np.float64):
+    """A mid-episode start state: h inside (-1, 1) as tanh leaves it, an unbounded cell state, a low-pass state of joint scale."""
+    c = np.empty((N, depth, 2, H), dtype)
+    c[:, :, 0] = rng.uniform(-0.95, 0.95, (N, depth, H))
+    c[:, :, 1] = rng.normal(0, 2.0, (N, depth, H))
+    return c
+
+
+def test_ppo_grad_reference_from_nonzero_start_state():
+    """The float64 autograd reference (oracle/ppo_grad_torch.py) from a non-zero carry0: its log-probs and values are the
+    NumPy oracle's get_ppo_variables from the same carries, and a gradient entry that only a non-zero c0 / h0 makes non-zero
+    matches a central finite difference of the loss."""
+    import torch
+
+    import ppo_grad_torch as G
+
+    T, N, H, depth = 2, 3, 8, 2
+    p = O.OracleParams(hidden_size=H, depth=depth)
+    rng = np.random.default_rng(12)
+    wa = O.init_net_weights(rng, 65, 40, H, depth, dtype=np.float64)
+    wc = O.init_net_weights(rng, 475, 1, H, depth, dtype=np.float64)
+    b = _batch(T, N, seed=5)
+    obs = [{k: v.astype(np.float64) for k, v in _obs(b, t)[0].items()} for t in range(T)]
+    cmd = np.stack([O.initial_command(b["cmd0_rand"]["mode"], b["cmd0_rand"]["u6"], b["cmd0_rand"]["u_arms"], P)] * T)
+    cmd = cmd.astype(np.float64)
+    carry0 = {"actor": _random_carry(rng, N, depth, H), "critic": _random_carry(rng, N, depth, H),
+              "lpf_params": rng.normal(0, 0.3, (N, 20))}
+    done = np.array([[True, False, False], [False, True, False]])
+    action = np.stack([o["joint_position"] for o in obs]) + 0.2 * rng.standard_normal((T, N, 20))
+    ref, _ = O.get_ppo_variables(wa, wc, obs, cmd, action, done, carry0, p, mirror=False)
+    batch = {"actor_obs": np.stack([O.actor_obs_from_dict(o, c) for o, c in zip(obs, cmd)]),
+             "critic_obs": np.stack([O.critic_obs_from_dict(o, c) for o, c in zip(obs, cmd)]),
+             "action": action, "done": done, "advantages": rng.normal(size=(T, N)), "value_targets": rng.normal(0, 0.5, (T, N))}
+    batch["old_log_probs"] = ref["log_probs"][..., 0] + rng.normal(0, 0.05, (T, N))
+    batch["old_values"] = ref["values"] + rng.normal(0, 0.05, (T, N))
+    loss, _, ga, gc, lp, val = G.ppo_minibatch_grads(wa, wc, batch, p, carry0=carry0)
+    np.testing.assert_allclose(lp, ref["log_probs"][..., 0], rtol=1e-12, atol=1e-10)
+    np.testing.assert_allclose(val, ref["values"], rtol=1e-12, atol=1e-12)
+    _, _, ga0, gc0, lp0, _ = G.ppo_minibatch_grads(wa, wc, batch, p)
+    assert np.abs(lp0 - lp).max() > 1e-3                               # carry0 reached the forward pass
+
+    def loss_at(net, layer, key, idx, delta):
+        w = {"actor": wa, "critic": wc}
+        w2 = {k: {kk: (vv if kk != "layers" else [dict(l) for l in vv]) for kk, vv in x.items()} for k, x in w.items()}
+        a = w2[net]["layers"][layer][key].copy()
+        a[idx] += delta
+        w2[net]["layers"][layer][key] = a
+        args = [batch[k] for k in ("actor_obs", "critic_obs", "action", "done", "old_log_probs", "advantages",
+                                   "value_targets", "old_values")]
+        with torch.no_grad():
+            l, _, _, _ = G.ppo_minibatch_loss(G.weights_to_torch(w2["actor"], False), G.weights_to_torch(w2["critic"], False),
+                                              *args, p, {}, carry0)
+        return float(l)
+
+    # forget-gate bias of the actor's layer 0 (env 0 is reset after step 0: the gradient of the others carries dc c0 sigma'(f)),
+    # w_hh of the critic's top layer (step 0's term is dG0^T h0): both exactly 0 from a zero start at T = 1
+    for net, layer, key, idx, g, g0 in (("actor", 0, "b", (H + 3,), ga, ga0), ("critic", 1, "w_hh", (2 * H + 1, 5), gc, gc0)):
+        eps = 1e-5
+        fd = (loss_at(net, layer, key, idx, eps) - loss_at(net, layer, key, idx, -eps)) / (2 * eps)
+        got = g["layers"][layer][key][idx]
+        assert abs(got - fd) <= 1e-6 * abs(fd) + 1e-10, (net, key, got, fd)
+        assert abs(got - g0["layers"][layer][key][idx]) > 1e-3 * abs(got), (net, key, "does not depend on carry0")
