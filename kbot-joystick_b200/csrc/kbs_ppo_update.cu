@@ -204,6 +204,15 @@ copy_block_kernel(const float* __restrict__ src, int ld, float* __restrict__ dst
   dst[idx] = src[size_t(r) * ld + c];
 }
 
+// d min(r a, clip(r) a) / d log-prob of one transition: a dr (dr = d r / d log-prob) where the unclipped term is the minimum,
+// else 0.  A non-finite advantage yields a non-finite derivative in either branch: the comparison is false for NaN, which
+// used to select the clipped branch's 0 and drop the transition from the gradient silently, so the update was applied while
+// the loss was NaN (jax.grad gives NaN there and ksim skips the update).  Caught by
+// test_gpu_ppo_update.py::test_ppo_update_non_finite_minibatch_is_skipped.
+__device__ __forceinline__ float policy_dlogp(float r, float rc, float dr, float a, bool inside) {
+  return (inside || r * a < rc * a) ? a * dr : (isfinite(a) ? 0.0f : a);
+}
+
 // The same head with one WARP per env (lane j = joint j, log-prob / entropy by warp shuffles): the one-thread-per-env form
 // above was 3.5 ms of an 18 ms update (512 threads walking 2 x T steps x 20 joints of libm math and strided loads).
 // The steps are taken in chunks of kHC: every input of a chunk is loaded first (none depends on the filter's recurrence), then
@@ -296,7 +305,7 @@ actor_head_fwd_bwd_warp_kernel(const __grid_constant__ kbs_params P, kbs_ppo_los
       const float dr = (fabsf(lr) <= L.log_clip_value) ? r : 0.0f;
       const bool inside = r >= 1.0f - L.clip_param && r <= 1.0f + L.clip_param;
       const float rc = fminf(fmaxf(r, 1.0f - L.clip_param), 1.0f + L.clip_param);
-      const float dpol = (inside || r * a < rc * a) ? a * dr : 0.0f;
+      const float dpol = policy_dlogp(r, rc, dr, a, inside);
       const float glp = -inv * dpol, gent = -inv * L.entropy_coef;
       const float keep = dn[i] ? 0.0f : 1.0f;
       float* d = dout + (t * n + e) * 64;
@@ -422,7 +431,7 @@ actor_head_fwd_bwd_block_kernel(const __grid_constant__ kbs_params P, kbs_ppo_lo
       const float dr = (fabsf(lr) <= L.log_clip_value) ? r : 0.0f;
       const bool inside = r >= 1.0f - L.clip_param && r <= 1.0f + L.clip_param;
       const float rc = fminf(fmaxf(r, 1.0f - L.clip_param), 1.0f + L.clip_param);
-      const float dpol = (inside || r * a < rc * a) ? a * dr : 0.0f;
+      const float dpol = policy_dlogp(r, rc, dr, a, inside);
       const float glp = -inv * dpol, gent = -inv * L.entropy_coef;
       float* d = dout + (t * n + e) * 64;
       float dmu = 0.0f;
@@ -473,7 +482,7 @@ actor_head_bwd_warp_kernel(const __grid_constant__ kbs_params P, kbs_ppo_loss_pa
     const float dr = (fabsf(lr) <= L.log_clip_value) ? r : 0.0f;
     const bool inside = r >= 1.0f - L.clip_param && r <= 1.0f + L.clip_param;
     const float rc = fminf(fmaxf(r, 1.0f - L.clip_param), 1.0f + L.clip_param);
-    const float dpol = (inside || r * a < rc * a) ? a * dr : 0.0f;
+    const float dpol = policy_dlogp(r, rc, dr, a, inside);
     const float glp = -inv * dpol, gent = -inv * L.entropy_coef;
     const float keep = done[t * ld + e] ? 0.0f : 1.0f;
     float* d = dout + (t * n + e) * 64;
