@@ -259,6 +259,42 @@ int kbs_adamw_step(kbs_handle* h, float* param, const float* grad, float* m, flo
  * double in a fixed order (bitwise reproducible; identical on every rank after the all-reduce). */
 int kbs_grad_norm(kbs_handle* h, const float* grad, int64_t count, float* norm_out, void* stream);
 
+/* The update phase of a PPO epoch (train.py:1763-1766: num_passes 3, batch_size 512 trajectories): num_passes passes over the
+ * stored rollout, each over a fresh random permutation of the env axis cut into n_envs / batch_size minibatches of whole
+ * trajectories [U: ksim's update loop is not vendored; this is the library's reading of it].  ppo.PpoUpdater.epoch chains
+ * kbs_ppo_variables -> kbs_gae -> per pass (kbs_minibatch_permutation -> kbs_shuffle_minibatches -> one update per
+ * minibatch), all on the device.
+ *
+ * Replaces: jax.random.permutation over the env axis [U].  perm_out int32 [n_envs] = a uniform random permutation of
+ * 0..n_envs-1, drawn on the device:
+ *   key(e)   = word 0 of Philox4x32-10(counter = (pass lo, pass hi, env0 + e, 0xFFFFFFFF), key = seed)   (the function of
+ *              kbs_generate_rollout_noise; no rollout-noise counter has 0xFFFFFFFF as its fourth word)
+ *   perm_out = the low 32 bits of the 64-bit values (key(e) << 32) | e sorted ascending (ties broken by e: always a permutation)
+ * pass_dev: device int64, read and then advanced by one (as step_dev of kbs_adamw_step), so a replayed CUDA graph draws a
+ * new permutation on every pass.  env0: the rank's global env offset (rank * n_envs): with one seed, ranks draw different
+ * permutations.  One CTA sorts in shared memory: n_envs <= KBS_MAX_PERMUTATION_ENVS, else KBS_E_SHAPE. */
+#define KBS_MAX_PERMUTATION_ENVS 16384
+int kbs_minibatch_permutation(kbs_handle* h, uint64_t seed, int64_t* pass_dev, int64_t env0, int32_t* perm_out, int64_t n_envs,
+                              void* stream);
+/* The rollout buffer cut into dense minibatches: column j of minibatch b is env perm[b * batch_size + j] of `src`.
+ *   src: the whole rollout as kbs_ppo_grad takes a minibatch (SoA at src->ld, carries [depth][2][n_envs][H]).
+ *   dst: every array [num_batches][T][F][batch_size] (done u8, the [T] fields with F = 1); carries
+ *        [num_batches][depth][2][batch_size][H], lpf0 [num_batches][20][batch_size].  Minibatch b is then an ordinary
+ *        kbs_ppo_batch with ld = batch_size at offset b of every array (whole 128-row panels keep kbs_ppo_grad's fast path).
+ *   A NULL src carry / lpf0 (zeros at the first step) requires a NULL dst one.
+ * batch_size % 4 == 0, num_batches * batch_size == n_envs <= KBS_MAX_PERMUTATION_ENVS, src->ld >= n_envs, src->ld % 4 == 0;
+ * float arrays and perm 16-byte aligned, done 4-byte aligned.  An index of perm outside [0, n_envs) is never read through:
+ * its float columns are written as NaN (done 0), so the update's non-finite skip refuses that minibatch.  One pass over
+ * the buffer: a CTA stages one [T][F] row of n_envs values in shared memory and writes its num_batches segments. */
+typedef struct kbs_ppo_minibatches {
+  float* actor_obs; float* critic_obs; float* action; uint8_t* done;
+  float* old_log_probs; float* advantages; float* value_targets; float* old_values;
+  float* actor_carry0; float* critic_carry0; float* lpf0;
+  int64_t batch_size, num_batches;
+} kbs_ppo_minibatches;
+int kbs_shuffle_minibatches(kbs_handle* h, const int32_t* perm, const kbs_ppo_batch* src, const kbs_ppo_minibatches* dst,
+                            int64_t n_envs, void* stream);
+
 /* Pins the handle's scratch allocation: while locked, a call that would have to grow (free + reallocate) the scratch
  * returns KBS_E_STATE instead -- a captured CUDA graph holds pointers into it (ppo.PpoUpdater.capture). */
 int kbs_scratch_lock(kbs_handle* h, int on);
@@ -483,7 +519,7 @@ int kbs_debug_tc_trace(kbs_handle* h, long long* trace_out, int64_t n_envs, void
 /* Same stamps for LSTM layer `layer` at step `step` of subsequent kbs_rollout calls (trace_out NULL detaches). */
 int kbs_debug_tc_trace_attach(kbs_handle* h, long long* trace_out, int64_t step, int layer);
 
-#define KBS_NUM_KERNEL_IDS 22
+#define KBS_NUM_KERNEL_IDS 24
 int kbs_profile_enable(kbs_handle* h, int on);
 int kbs_profile_read(kbs_handle* h, int max_ids, double* total_ms, int64_t* launches);
 const char* kbs_kernel_name(int id);

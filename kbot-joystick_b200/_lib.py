@@ -114,6 +114,12 @@ class KbsPpoBatch(C.Structure):
                                    "old_values", "actor_carry0", "critic_carry0", "lpf0")] + [("T", _i64), ("ld", _i64)]
 
 
+class KbsPpoMinibatches(C.Structure):
+    _fields_ = [(k, _vp) for k in ("actor_obs", "critic_obs", "action", "done", "old_log_probs", "advantages", "value_targets",
+                                   "old_values", "actor_carry0", "critic_carry0", "lpf0")] + [("batch_size", _i64),
+                                                                                             ("num_batches", _i64)]
+
+
 class KbsNetGrads(C.Structure):
     _fields_ = [("w_in", _vp), ("b_in", _vp), ("w_ih", _vp * MAX_DEPTH), ("w_hh", _vp * MAX_DEPTH), ("b", _vp * MAX_DEPTH),
                 ("w_out", _vp), ("b_out", _vp)]
@@ -127,10 +133,12 @@ EXPORTS = (
     "kbs_launch_count", "kbs_device_status", "kbs_mirror_observations", "kbs_mirror_joints", "kbs_upload_state", "kbs_com_distance", "kbs_ppo_loss_default_params", "kbs_ppo_loss", "kbs_ppo_grad", "kbs_adam_step", "kbs_torque_substeps", "kbs_profile_enable", "kbs_profile_read", "kbs_kernel_name", "kbs_debug_tc_gates", "kbs_debug_tc_trace", "kbs_debug_tc_trace_attach",
     "kbs_adamw_default_params", "kbs_adamw_step", "kbs_grad_norm", "kbs_scratch_lock", "kbs_actuator_rand_default_params",
     "kbs_sample_actuator_randomization", "kbs_device_status_reset", "kbs_ppo_grad_set_events", "kbs_generate_rollout_noise",
+    "kbs_minibatch_permutation", "kbs_shuffle_minibatches",
 )
 VERSION = 101
 STATUS_TIMEOUT_LSTM, STATUS_TIMEOUT_HEAD, STATUS_F16_RANGE = 1, 2, 0x100
-NUM_KERNEL_IDS = 22
+NUM_KERNEL_IDS = 24
+MAX_PERMUTATION_ENVS = 16384
 
 _lib = None
 
@@ -167,6 +175,8 @@ def load() -> C.CDLL:
     lib.kbs_ppo_grad_set_events.argtypes = [_vp, _vp]
     lib.kbs_generate_rollout_noise.argtypes = [_vp, C.c_uint64, _i64, P(KbsNoiseView), _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _vp]
     lib.kbs_grad_norm.argtypes = [_vp, _vp, _i64, _vp, _vp]
+    lib.kbs_minibatch_permutation.argtypes = [_vp, C.c_uint64, _vp, _i64, _vp, _i64, _vp]
+    lib.kbs_shuffle_minibatches.argtypes = [_vp, _vp, P(KbsPpoBatch), P(KbsPpoMinibatches), _i64, _vp]
     lib.kbs_scratch_lock.argtypes = [_vp, C.c_int]
     lib.kbs_device_status_reset.argtypes = [_vp]
     lib.kbs_actuator_rand_default_params.argtypes = [P(KbsActuatorRandParams)]

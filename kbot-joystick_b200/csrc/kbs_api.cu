@@ -424,7 +424,8 @@ const char* kbs_kernel_name(int id) {
       "obs_kernel", "command_kernel", "torque_kernel", "terminate_kernel", "reward_rot_kernel", "reward_terms_kernel",
       "reward_scan_kernel", "gae_kernel", "adv_norm_kernel", "policy_io_kernels", "gemm_nt_kernel(simt)",
       "lstm_cell_kernel", "actor_head_kernel", "critic_head_kernel", "pack_kernels", "lstm_layer_tc_kernel",
-      "proj_tc_kernel", "rollout_persist_kernel", "bptt_persist_kernel", "gemm_tn_tc_kernel", "sb_to_tn_kernel", "tn_reduce_kernel"};
+      "proj_tc_kernel", "rollout_persist_kernel", "bptt_persist_kernel", "gemm_tn_tc_kernel", "sb_to_tn_kernel", "tn_reduce_kernel",
+      "minibatch_permutation_kernel", "shuffle_minibatches_kernels"};
   return (id >= 0 && id < KBS_K_COUNT) ? names[id] : "?";
 }
 
@@ -824,6 +825,38 @@ int kbs_generate_rollout_noise(kbs_handle* h, uint64_t seed, int64_t step0, cons
   AL(eps_action); AL(u_switch); AL(cmd_mode); AL(cmd_u6); AL(cmd_u_arms);
   return kbs_launch_rollout_noise(h, seed, step0, noise, eps_action, u_switch, cmd_mode, cmd_u6, cmd_u_arms, T, ld, n,
                                   (cudaStream_t)stream);
+}
+
+int kbs_minibatch_permutation(kbs_handle* h, uint64_t seed, int64_t* pass_dev, int64_t env0, int32_t* perm_out, int64_t n,
+                              void* stream) {
+  REQ(h); REQ(pass_dev); REQ(perm_out);
+  if (n <= 0 || n > KBS_MAX_PERMUTATION_ENVS) return KBS_E_SHAPE;
+  if (env0 < 0) return KBS_E_PARAM;
+  if ((reinterpret_cast<uintptr_t>(pass_dev) & 7u) || (reinterpret_cast<uintptr_t>(perm_out) & 3u)) return KBS_E_ALIGN;
+  return kbs_launch_minibatch_permutation(h, seed, pass_dev, env0, perm_out, n, (cudaStream_t)stream);
+}
+
+int kbs_shuffle_minibatches(kbs_handle* h, const int32_t* perm, const kbs_ppo_batch* src, const kbs_ppo_minibatches* dst, int64_t n,
+                            void* stream) {
+  REQ(h); REQ(perm); REQ(src); REQ(dst);
+  REQ(src->actor_obs); REQ(src->critic_obs); REQ(src->action); REQ(src->done); REQ(src->old_log_probs); REQ(src->advantages);
+  REQ(src->value_targets); REQ(src->old_values);
+  REQ(dst->actor_obs); REQ(dst->critic_obs); REQ(dst->action); REQ(dst->done); REQ(dst->old_log_probs); REQ(dst->advantages);
+  REQ(dst->value_targets); REQ(dst->old_values);
+  // a start carry is copied when the rollout has one and left out (zeros at the first step) when it has none
+  if (!src->actor_carry0 != !dst->actor_carry0 || !src->critic_carry0 != !dst->critic_carry0 || !src->lpf0 != !dst->lpf0)
+    return KBS_E_NULL;
+  const int64_t bs = dst->batch_size;
+  if (src->T <= 0 || n <= 0 || n > KBS_MAX_PERMUTATION_ENVS || bs <= 0 || bs % 4 || n % bs || dst->num_batches != n / bs)
+    return KBS_E_SHAPE;
+  if (src->ld < n || (src->ld & 3)) return KBS_E_SHAPE;
+  AL(perm);
+  AL(src->actor_obs); AL(src->critic_obs); AL(src->action); AL(src->old_log_probs); AL(src->advantages); AL(src->value_targets);
+  AL(src->old_values); AL(src->actor_carry0); AL(src->critic_carry0); AL(src->lpf0);
+  AL(dst->actor_obs); AL(dst->critic_obs); AL(dst->action); AL(dst->old_log_probs); AL(dst->advantages); AL(dst->value_targets);
+  AL(dst->old_values); AL(dst->actor_carry0); AL(dst->critic_carry0); AL(dst->lpf0);
+  if ((reinterpret_cast<uintptr_t>(src->done) & 3u) || (reinterpret_cast<uintptr_t>(dst->done) & 3u)) return KBS_E_ALIGN;
+  return kbs_launch_shuffle_minibatches(h, perm, *src, *dst, n, (cudaStream_t)stream);
 }
 
 int kbs_adamw_default_params(kbs_adamw_params* p) {

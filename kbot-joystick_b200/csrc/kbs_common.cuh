@@ -47,8 +47,10 @@ struct KbsNet {
 enum KbsKernelId {
   KBS_K_OBS = 0, KBS_K_COMMAND, KBS_K_TORQUE, KBS_K_TERMINATE, KBS_K_REWARD_ROT, KBS_K_REWARD_TERMS, KBS_K_REWARD_SCAN,
   KBS_K_GAE, KBS_K_ADV_NORM, KBS_K_POLICY_IO, KBS_K_GEMM_SIMT, KBS_K_LSTM_CELL, KBS_K_ACTOR_HEAD, KBS_K_CRITIC_HEAD,
-  KBS_K_PACK, KBS_K_LSTM_TC, KBS_K_PROJ_TC, KBS_K_ROLLOUT_TC, KBS_K_BPTT_TC, KBS_K_GEMM_TN, KBS_K_PACK_TN, KBS_K_TN_REDUCE, KBS_K_COUNT
+  KBS_K_PACK, KBS_K_LSTM_TC, KBS_K_PROJ_TC, KBS_K_ROLLOUT_TC, KBS_K_BPTT_TC, KBS_K_GEMM_TN, KBS_K_PACK_TN, KBS_K_TN_REDUCE,
+  KBS_K_PERMUTATION, KBS_K_SHUFFLE, KBS_K_COUNT
 };
+static_assert(KBS_K_COUNT == KBS_NUM_KERNEL_IDS, "kbotstep.h KBS_NUM_KERNEL_IDS");
 constexpr int kKbsProfMaxPairs = 8192;
 constexpr int kKbsMaxChunks = 8;
 
@@ -81,6 +83,7 @@ struct kbs_handle {
   bool bptt_attr_set = false;
   bool fwd_save_attr_set = false;
   bool dw_attr_set = false;
+  bool minibatch_attr_set = false;            // kbs_minibatch_permutation / kbs_shuffle_minibatches shared-memory opt-in
   cudaEvent_t ev_critic_ready = nullptr;      // caller's event (kbs_ppo_grad_set_events): recorded when the critic's gradients are final
   bool scratch_locked = false;                // kbs_scratch_lock: growing the scratch is an error (a CUDA graph holds pointers)
   long long* trace_buf = nullptr;
@@ -160,6 +163,11 @@ int kbs_launch_policy_pack(kbs_handle* h, const float* ja, const float* jv, cons
                            int64_t ld, int64_t n, cudaStream_t st);
 int kbs_launch_policy_unpack(kbs_handle* h, const float* carry_aos, const float* lpf_soa, const float* mean_soa,
                              float* carry_out, float* action_out, int64_t ld, int64_t n, cudaStream_t st);
+// kbs_ppo_update.cu: the update phase's minibatch construction (arguments validated by the entry points in kbs_api.cu)
+int kbs_launch_minibatch_permutation(kbs_handle* h, uint64_t seed, int64_t* pass_dev, int64_t env0, int32_t* perm, int64_t n,
+                                     cudaStream_t st);
+int kbs_launch_shuffle_minibatches(kbs_handle* h, const int32_t* perm, const kbs_ppo_batch& src, const kbs_ppo_minibatches& dst,
+                                   int64_t n, cudaStream_t st);
 
 // kbs_net_simt.cu : fp32 FFMA datapath
 int kbs_simt_pack(kbs_handle* h, int net, const kbs_net_weights* w, cudaStream_t st);
@@ -423,6 +431,19 @@ __device__ __forceinline__ void sb_flag_range(unsigned int* status, bool bad) {
 template <int R, int KIND, bool WB = false>
 __device__ __forceinline__ void sb_store4(void* __restrict__ sb, int64_t row, int k, int kblocks, const float (&x)[4]) {
   sb_store_split<R, KIND, WB>(sb, row, k, kblocks, sb_split4<KIND>(x));
+}
+// Counter-based Philox4x32-10 (Salmon et al., SC'11): 128-bit counter c, 64-bit key k -> 4 x 32 random bits.  Shared by the
+// rollout noise (kbs_generate_rollout_noise) and the minibatch permutation (kbs_minibatch_permutation), whose counters are
+// disjoint: the permutation's fourth counter word is 0xFFFFFFFF, which no rollout-noise row index reaches.
+__device__ __forceinline__ uint4 kbs_philox4x32_10(uint4 c, uint2 k) {
+#pragma unroll
+  for (int r = 0; r < 10; ++r) {
+    const uint32_t hi0 = __umulhi(0xD2511F53u, c.x), lo0 = 0xD2511F53u * c.x;
+    const uint32_t hi1 = __umulhi(0xCD9E8D57u, c.z), lo1 = 0xCD9E8D57u * c.z;
+    c = make_uint4(hi1 ^ c.y ^ k.x, lo1, hi0 ^ c.w ^ k.y, lo0);
+    k.x += 0x9E3779B9u; k.y += 0xBB67AE85u;
+  }
+  return c;
 }
 #endif  // __CUDACC__
 

@@ -518,19 +518,9 @@ actuator_rand_kernel(const __grid_constant__ kbs_params P, const kbs_actuator_ra
 }
 
 // =====================================================================================================
-// Device-side randomness of a rollout (kbs_generate_rollout_noise): counter-based Philox4x32-10.
+// Device-side randomness of a rollout (kbs_generate_rollout_noise): counter-based Philox4x32-10 (kbs_philox4x32_10).
 // counter = (step lo, step hi, env group, row), key = seed: 4 x 32 bits per call = the 4 consecutive envs of a float4.
 // =====================================================================================================
-__device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
-#pragma unroll
-  for (int r = 0; r < 10; ++r) {
-    const uint32_t hi0 = __umulhi(0xD2511F53u, c.x), lo0 = 0xD2511F53u * c.x;
-    const uint32_t hi1 = __umulhi(0xCD9E8D57u, c.z), lo1 = 0xCD9E8D57u * c.z;
-    c = make_uint4(hi1 ^ c.y ^ k.x, lo1, hi0 ^ c.w ^ k.y, lo0);
-    k.x += 0x9E3779B9u; k.y += 0xBB67AE85u;
-  }
-  return c;
-}
 struct NoiseRows {
   float* base[9];        // eps_jpos, eps_jvel, eps_gyro, eps_pg, eps_action, u_switch, cmd_mode (as int32), cmd_u6, cmd_u_arms
   int rows[9];           // rows per step of each array
@@ -550,8 +540,8 @@ rollout_noise_kernel(const __grid_constant__ NoiseRows R, uint64_t seed, int64_t
   const int row = gr - R.first[a];
   const int64_t t = blockIdx.z;
   const uint64_t step = uint64_t(step0 + t);
-  const uint4 x = philox4x32_10(make_uint4(uint32_t(step), uint32_t(step >> 32), uint32_t(grp), uint32_t(gr)),
-                                make_uint2(uint32_t(seed), uint32_t(seed >> 32)));
+  const uint4 x = kbs_philox4x32_10(make_uint4(uint32_t(step), uint32_t(step >> 32), uint32_t(grp), uint32_t(gr)),
+                                    make_uint2(uint32_t(seed), uint32_t(seed >> 32)));
   const uint32_t w[4] = {x.x, x.y, x.z, x.w};
   float v[4];
   const int kind = R.kind[a];

@@ -1195,7 +1195,174 @@ int ppo_grad_persistent(kbs_handle* h, const kbs_ppo_loss_params& L, const kbs_p
   return KBS_OK;
 }
 
+// ---- minibatches of the update phase (kbs_minibatch_permutation, kbs_shuffle_minibatches) ------------------------------------
+
+// One CTA: Philox key of every env, bitonic sort of (key << 32) | e over the next power of two (padding = ~0, sorts last)
+// in shared memory.  All threads read *pass_dev before the first barrier; thread 0 advances it after.
+constexpr int kPermThreads = 1024;
+__global__ void __launch_bounds__(kPermThreads)
+minibatch_permutation_kernel(uint64_t seed, long long* __restrict__ pass_dev, int64_t env0, int32_t* __restrict__ perm, int n,
+                             int np2) {
+  extern __shared__ unsigned long long sk[];
+  const unsigned long long pass = (unsigned long long)pass_dev[0];
+  const uint2 key = make_uint2(uint32_t(seed), uint32_t(seed >> 32));
+  for (int e = threadIdx.x; e < np2; e += kPermThreads) {
+    unsigned long long v = ~0ull;
+    if (e < n) {
+      const uint4 x = kbs_philox4x32_10(make_uint4(uint32_t(pass), uint32_t(pass >> 32), uint32_t(env0 + e), 0xFFFFFFFFu), key);
+      v = ((unsigned long long)x.x << 32) | unsigned(e);
+    }
+    sk[e] = v;
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) pass_dev[0] = (long long)(pass + 1);
+  for (int k = 2; k <= np2; k <<= 1) {
+    for (int j = k >> 1; j > 0; j >>= 1) {
+      for (int i = threadIdx.x; i < np2 / 2; i += kPermThreads) {
+        const int lo = 2 * i - (i & (j - 1)), hi = lo + j;
+        const unsigned long long a = sk[lo], b = sk[hi];
+        if ((a > b) == ((lo & k) == 0)) { sk[lo] = b; sk[hi] = a; }
+      }
+      __syncthreads();
+    }
+  }
+  for (int i = threadIdx.x; i < n; i += kPermThreads) perm[i] = int32_t(uint32_t(sk[i]));
+}
+
+// The SoA fields of a rollout, as one list of rows: array a has rows[a] rows ([T][F] flattened) of n values at stride ld in
+// src, written as [num_batches][rows][bs] to dst.
+struct ShuffleRows {
+  const char* src[9];
+  char* dst[9];
+  int64_t first[10];     // prefix sums of the arrays' row counts
+  int esize[9];          // 4 = float, 1 = u8
+};
+constexpr int kShufThreads = 256;
+// one CTA per source row: stage the row's n values in shared memory (coalesced), then write its num_batches contiguous
+// bs-wide segments, 4 output columns per thread (bs % 4 == 0: the 4 columns are in one segment)
+__global__ void __launch_bounds__(kShufThreads)
+shuffle_rows_kernel(const __grid_constant__ ShuffleRows R, const int32_t* __restrict__ perm, int64_t ld, int n, int bs) {
+  extern __shared__ float4 srow4[];
+  const int64_t g = blockIdx.x;
+  int a = 0;
+#pragma unroll
+  for (int i = 1; i < 9; ++i) a += (g >= R.first[i]) ? 1 : 0;
+  const int64_t r = g - R.first[a], rows = R.first[a + 1] - R.first[a];
+  const int es = R.esize[a];
+  const int n16 = n * es / 16, n4 = n * es / 4;      // row bytes / 16 (float) or / 4 (u8; n % 4 == 0, ld % 4 == 0)
+  if (es == 4) {
+    const float4* s = reinterpret_cast<const float4*>(R.src[a] + r * ld * 4);
+    for (int i = threadIdx.x; i < n16; i += kShufThreads) srow4[i] = __ldcs(s + i);
+  } else {
+    const uint32_t* s = reinterpret_cast<const uint32_t*>(R.src[a] + r * ld);
+    uint32_t* d = reinterpret_cast<uint32_t*>(srow4);
+    for (int i = threadIdx.x; i < n4; i += kShufThreads) d[i] = s[i];
+  }
+  __syncthreads();
+  const float* srow = reinterpret_cast<const float*>(srow4);
+  const uint8_t* srow_b = reinterpret_cast<const uint8_t*>(srow4);
+  for (int k = threadIdx.x * 4; k < n; k += kShufThreads * 4) {
+    const int4 p = *reinterpret_cast<const int4*>(perm + k);
+    const int idx[4] = {p.x, p.y, p.z, p.w};
+    const int b = k / bs, j = k - b * bs;
+    const int64_t o = (int64_t(b) * rows + r) * bs + j;
+    if (es == 4) {
+      float v[4];
+#pragma unroll
+      for (int l = 0; l < 4; ++l) v[l] = (unsigned(idx[l]) < unsigned(n)) ? srow[idx[l]] : __int_as_float(0x7FC00000);
+      *reinterpret_cast<float4*>(R.dst[a] + o * 4) = make_float4(v[0], v[1], v[2], v[3]);
+    } else {
+      uchar4 v;
+      v.x = (unsigned(idx[0]) < unsigned(n)) ? srow_b[idx[0]] : 0;
+      v.y = (unsigned(idx[1]) < unsigned(n)) ? srow_b[idx[1]] : 0;
+      v.z = (unsigned(idx[2]) < unsigned(n)) ? srow_b[idx[2]] : 0;
+      v.w = (unsigned(idx[3]) < unsigned(n)) ? srow_b[idx[3]] : 0;
+      *reinterpret_cast<uchar4*>(R.dst[a] + o) = v;
+    }
+  }
+}
+
+// carries [D2][n][H] -> [num_batches][D2][bs][H], one warp per H-float row; blockIdx.y = net
+__global__ void __launch_bounds__(kShufThreads)
+shuffle_carry_kernel(const float* __restrict__ src0, float* __restrict__ dst0, const float* __restrict__ src1, float* __restrict__ dst1,
+                     const int32_t* __restrict__ perm, int n, int bs, int d2, int H) {
+  const float* src = blockIdx.y ? src1 : src0;
+  float* dst = blockIdx.y ? dst1 : dst0;
+  if (!src) return;
+  const int64_t o = int64_t(blockIdx.x) * (kShufThreads / 32) + (threadIdx.x >> 5);
+  if (o >= int64_t(n) * d2) return;
+  const int lane = threadIdx.x & 31;
+  const int64_t per_b = int64_t(d2) * bs;
+  const int b = int(o / per_b), rem = int(o - b * per_b), s = rem / bs, j = rem - s * bs;
+  const int e = perm[b * bs + j];
+  float4* d = reinterpret_cast<float4*>(dst + o * H);
+  if (unsigned(e) < unsigned(n)) {
+    const float4* sr = reinterpret_cast<const float4*>(src + (int64_t(s) * n + e) * H);
+    for (int i = lane; i < H / 4; i += 32) d[i] = __ldcs(sr + i);
+  } else {
+    const float q = __int_as_float(0x7FC00000);
+    for (int i = lane; i < H / 4; i += 32) d[i] = make_float4(q, q, q, q);
+  }
+}
+
+// shared-memory opt-in of both kernels for the largest n_envs, once per handle (not a call to make during graph capture)
+int minibatch_attr(kbs_handle* h) {
+  if (h->minibatch_attr_set) return KBS_OK;
+  KBS_CUDA_TRY(cudaFuncSetAttribute(minibatch_permutation_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    KBS_MAX_PERMUTATION_ENVS * int(sizeof(unsigned long long))));
+  KBS_CUDA_TRY(cudaFuncSetAttribute(shuffle_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    KBS_MAX_PERMUTATION_ENVS * int(sizeof(float))));
+  h->minibatch_attr_set = true;
+  return KBS_OK;
+}
+
 }  // namespace
+
+int kbs_launch_minibatch_permutation(kbs_handle* h, uint64_t seed, int64_t* pass_dev, int64_t env0, int32_t* perm, int64_t n,
+                                     cudaStream_t st) {
+  int np2 = 2;
+  while (np2 < n) np2 <<= 1;
+  const size_t smem = size_t(np2) * sizeof(unsigned long long);
+  if (int rc = minibatch_attr(h)) return rc;
+  static_assert(sizeof(long long) == sizeof(int64_t), "pass counter width");
+  KBS_LAUNCH(h, KBS_K_PERMUTATION, st,
+             (minibatch_permutation_kernel<<<1, kPermThreads, smem, st>>>(seed, reinterpret_cast<long long*>(pass_dev), env0, perm,
+                                                                          int(n), np2)));
+  KBS_LAUNCH_CHECK();
+  return KBS_OK;
+}
+
+int kbs_launch_shuffle_minibatches(kbs_handle* h, const int32_t* perm, const kbs_ppo_batch& src, const kbs_ppo_minibatches& dst,
+                                   int64_t n, cudaStream_t st) {
+  const int64_t T = src.T;
+  ShuffleRows R{};
+  const void* s[9] = {src.actor_obs, src.critic_obs, src.action, src.done, src.old_log_probs, src.advantages, src.value_targets,
+                      src.old_values, src.lpf0};
+  void* d[9] = {dst.actor_obs, dst.critic_obs, dst.action, dst.done, dst.old_log_probs, dst.advantages, dst.value_targets,
+                dst.old_values, dst.lpf0};
+  const int64_t rows[9] = {T * KBS_ACTOR_OBS, T * KBS_CRITIC_OBS, T * KBS_NUM_JOINTS, T, T, T, T, T, s[8] ? KBS_NUM_JOINTS : 0};
+  R.first[0] = 0;
+  for (int a = 0; a < 9; ++a) {
+    R.src[a] = static_cast<const char*>(s[a]);
+    R.dst[a] = static_cast<char*>(d[a]);
+    R.esize[a] = a == 3 ? 1 : 4;
+    R.first[a + 1] = R.first[a] + rows[a];
+  }
+  const size_t smem = size_t(n) * sizeof(float);
+  if (int rc = minibatch_attr(h)) return rc;
+  const int bs = int(dst.batch_size);
+  KBS_LAUNCH(h, KBS_K_SHUFFLE, st,
+             (shuffle_rows_kernel<<<unsigned(R.first[9]), kShufThreads, smem, st>>>(R, perm, src.ld, int(n), bs)));
+  if (src.actor_carry0 || src.critic_carry0) {
+    const int d2 = 2 * h->p.depth, H = h->p.hidden_size;
+    const unsigned gx = unsigned((n * d2 + kShufThreads / 32 - 1) / (kShufThreads / 32));
+    KBS_LAUNCH(h, KBS_K_SHUFFLE, st,
+               (shuffle_carry_kernel<<<dim3(gx, 2), kShufThreads, 0, st>>>(src.actor_carry0, dst.actor_carry0, src.critic_carry0,
+                                                                          dst.critic_carry0, perm, int(n), bs, d2, H)));
+  }
+  KBS_LAUNCH_CHECK();
+  return KBS_OK;
+}
 
 extern "C" {
 

@@ -219,6 +219,49 @@ class KbotStep:
         L.check(self.lib.kbs_adamw_step(self._h, L.ptr(param), L.ptr(grad), L.ptr(m), L.ptr(v), param.numel(), C.byref(o),
                                         L.ptr(grad_norm), L.ptr(step_dev), step, _stream()), "kbs_adamw_step")
 
+    def minibatch_permutation(self, pass_dev, n_envs: int, seed: int = 0, env0: int = 0, out=None):
+        """A uniform random permutation of the env axis (kbs_minibatch_permutation) -> int32 [n_envs] on the device.
+        pass_dev: device int64 [1] pass counter (read, then advanced by one); env0: the rank's global env offset."""
+        if out is None:
+            out = torch.empty((n_envs,), dtype=torch.int32, device=pass_dev.device)
+        L.check(self.lib.kbs_minibatch_permutation(self._h, seed, L.ptr(pass_dev), env0, L.ptr(out), n_envs, _stream()),
+                "kbs_minibatch_permutation")
+        return out
+
+    MINIBATCH_FIELDS = ("actor_obs", "critic_obs", "action", "done", "old_log_probs", "advantages", "value_targets",
+                        "old_values", "actor_carry0", "critic_carry0", "lpf0")
+
+    def minibatch_buffers(self, T: int, num_batches: int, batch_size: int, device) -> dict:
+        """Uninitialised destination of shuffle_minibatches, start carries included."""
+        e = lambda *s, dt=torch.float32: torch.empty((num_batches,) + s, dtype=dt, device=device)
+        dst = {"actor_obs": e(T, L.ACTOR_OBS, batch_size), "critic_obs": e(T, L.CRITIC_OBS, batch_size),
+               "action": e(T, L.NUM_JOINTS, batch_size), "done": e(T, batch_size, dt=torch.uint8)}
+        for k in ("old_log_probs", "advantages", "value_targets", "old_values"):
+            dst[k] = e(T, batch_size)
+        for k in ("actor_carry0", "critic_carry0"):
+            dst[k] = e(self.depth, 2, batch_size, self.hidden_size)
+        dst["lpf0"] = e(L.NUM_JOINTS, batch_size)
+        return dst
+
+    def shuffle_minibatches(self, perm, src: dict, n_envs: int, batch_size: int, dst: dict | None = None) -> dict:
+        """The rollout `src` (a ppo_grad batch over all n_envs trajectories at its ld) cut into n_envs / batch_size dense
+        minibatches (kbs_shuffle_minibatches): column j of minibatch b is env perm[b * batch_size + j].  dst (allocated when
+        None): every array [B, T, F, batch_size] ([B, T, batch_size] for the [T, ld] fields), carries [B, depth, 2,
+        batch_size, H], lpf0 [B, 20, batch_size]; the carries are present where src has them."""
+        T, _, ld = src["actor_obs"].shape
+        if dst is None:
+            dst = self.minibatch_buffers(T, n_envs // batch_size, batch_size, src["actor_obs"].device)
+            dst = {k: t for k, t in dst.items() if not k.endswith("0") or src.get(k) is not None}
+        s, d = L.KbsPpoBatch(), L.KbsPpoMinibatches()
+        for k in self.MINIBATCH_FIELDS:
+            setattr(s, k, L.ptr(src.get(k)))
+            setattr(d, k, L.ptr(dst.get(k)))
+        s.T, s.ld = T, ld
+        d.batch_size, d.num_batches = batch_size, dst["actor_obs"].shape[0]
+        L.check(self.lib.kbs_shuffle_minibatches(self._h, L.ptr(perm), C.byref(s), C.byref(d), n_envs, _stream()),
+                "kbs_shuffle_minibatches")
+        return dst
+
     def sample_actuator_randomization(self, u, episode: dict, reset=None, n_envs: int | None = None, **scales) -> None:
         """Per-episode PositionActuators randomisation (train.py:1097-1105): u [5, 20, ld] uniforms -> episode["kp"], ["kd"],
         ["tau_limit"], ["action_bias"], ["torque_bias"] ([20, ld] each, written where reset != 0 / everywhere)."""
