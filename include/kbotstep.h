@@ -439,6 +439,31 @@ typedef struct kbs_rollout_io {
 
 int kbs_rollout(kbs_handle* h, const kbs_rollout_io* io, int64_t n_envs, void* stream);
 
+/* kbs_rollout plus what crosses a call boundary and what the PPO update trains on.  kbs_rollout(h, io, n, s) is
+ * kbs_rollout_record(h, io, NULL, n, s); either pointer of `rec` may be NULL.
+ *
+ * done_prev [ld] u8 (4-byte aligned): done of the step before this call's step 0, i.e. the previous call's done[T-1].  On
+ * step 0, where done_prev[e] != 0, the lagged projected-gravity state (pg_carry) restarts at the current value, exactly as it
+ * does inside a call on the step after done[t-1].  That is the only stage that reads the previous step's done: the actor /
+ * critic carries and the action filter (lpf) are reset after step t from done[t] within the step, command[t+1] is drawn
+ * from done[t], and kbs_rewards pads t = 0 of a trajectory as the reference does (no previous step).  So a rollout split
+ * into calls, each passing the previous call's done[T-1] here, is the same rollout as one call over all steps; without it,
+ * an episode that ends on a call's last step keeps its lag state into the next episode.  T = 1 calls (one per control step
+ * around the simulator) need it at every episode end.
+ *
+ * critic_obs [T][475][ld] (16-byte aligned): the run_critic concatenation of every step, all 475 rows, as
+ * kbs_observations(critic_obs) writes it -- what kbs_ppo_variables / kbs_ppo_grad train the critic on.  It may be requested
+ * with io->value == NULL (the rows are written, the critic is not run); it needs the state rows the concatenation reads
+ * (cinert, cvel, actuator_force; else KBS_E_NULL).  Requesting it changes no other output of the call.
+ *
+ * Declared as a plain struct tag (like POSIX `struct stat` / stat()): the function owns the ordinary name. */
+struct kbs_rollout_record {
+  const uint8_t* done_prev;   /* [ld] or NULL */
+  float* critic_obs;          /* [T][475][ld] or NULL */
+};
+int kbs_rollout_record(kbs_handle* h, const kbs_rollout_io* io, const struct kbs_rollout_record* rec, int64_t n_envs,
+                       void* stream);
+
 /* Replaces: the jax.random draws the reference makes ON THE DEVICE during a rollout -- observation noise (train.py:1160, 1162,
  * 1176, 1194), the action sample (train.py:1564), the command resampling (train.py:725-737, 752-753, 782-783) -- for callers
  * that do not need bit parity with JAX's threefry streams (parity mode hands these arrays to kbs_rollout explicitly).

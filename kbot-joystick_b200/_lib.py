@@ -82,6 +82,11 @@ class KbsRolloutIO(C.Structure):
                            "term_codes", "done", "success", "value")] + [("T", _i64)]
 
 
+class KbsRolloutRecord(C.Structure):
+    """struct kbs_rollout_record (kbs_rollout_record's optional outputs / boundary input)."""
+    _fields_ = [("done_prev", _vp), ("critic_obs", _vp)]
+
+
 class KbsPpoIO(C.Structure):
     _fields_ = [(k, _vp) for k in ("actor_obs", "critic_obs", "action", "done", "actor_carry", "critic_carry", "lpf",
                                    "log_probs", "values", "entropy", "action_std", "mean")] + [("T", _i64), ("ld", _i64)] + [
@@ -133,7 +138,7 @@ EXPORTS = (
     "kbs_launch_count", "kbs_device_status", "kbs_mirror_observations", "kbs_mirror_joints", "kbs_upload_state", "kbs_com_distance", "kbs_ppo_loss_default_params", "kbs_ppo_loss", "kbs_ppo_grad", "kbs_adam_step", "kbs_torque_substeps", "kbs_profile_enable", "kbs_profile_read", "kbs_kernel_name", "kbs_debug_tc_gates", "kbs_debug_tc_trace", "kbs_debug_tc_trace_attach",
     "kbs_adamw_default_params", "kbs_adamw_step", "kbs_grad_norm", "kbs_scratch_lock", "kbs_actuator_rand_default_params",
     "kbs_sample_actuator_randomization", "kbs_device_status_reset", "kbs_ppo_grad_set_events", "kbs_generate_rollout_noise",
-    "kbs_minibatch_permutation", "kbs_shuffle_minibatches",
+    "kbs_minibatch_permutation", "kbs_shuffle_minibatches", "kbs_rollout_record",
 )
 VERSION = 101
 STATUS_TIMEOUT_LSTM, STATUS_TIMEOUT_HEAD, STATUS_F16_RANGE = 1, 2, 0x100
@@ -195,6 +200,7 @@ def load() -> C.CDLL:
     lib.kbs_gae.argtypes = [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _vp]
     lib.kbs_policy_step.argtypes = [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]
     lib.kbs_rollout.argtypes = [_vp, P(KbsRolloutIO), _i64, _vp]
+    lib.kbs_rollout_record.argtypes = [_vp, P(KbsRolloutIO), P(KbsRolloutRecord), _i64, _vp]
     lib.kbs_ppo_variables.argtypes = [_vp, P(KbsPpoIO), _i64, _vp]
     lib.kbs_launch_count.argtypes = [_vp]
     lib.kbs_launch_count.restype = _i64

@@ -90,7 +90,10 @@ constexpr int kOutLd = 64;  // row stride of the trunk output buffer
 // is evaluated for all T steps first (terminations, command law, lagged gravity, observations, input projections:
 // big HBM-bound launches), then the whole recurrence runs as ONE persistent kernel (kbs_tc_rollout_recurrent; the per-step
 // form -- 2 LSTM layer launches for both nets + a head launch per step -- stays behind KBS_TC_PER_STEP=1).
-int rollout_fused_tc(kbs_handle* h, const kbs_rollout_io* io, int64_t n, cudaStream_t st) {
+// done_prev restarts the lag scan at step 0; critic_obs (when given) replaces the per-chunk scratch of the critic's
+// observations and gets all 475 rows, the input projection still reads cinert / cvel straight from the state.
+int rollout_fused_tc(kbs_handle* h, const kbs_rollout_io* io, const uint8_t* done_prev, float* critic_obs, int64_t n,
+                     cudaStream_t st) {
   const int64_t ld = io->state.ld, T = io->T;
   const bool critic = io->value != nullptr;
   // Observation assembly + input projections can run in chunks of CT steps on the handle's aux stream while the
@@ -108,7 +111,7 @@ int rollout_fused_tc(kbs_handle* h, const kbs_rollout_io* io, int64_t n, cudaStr
   const size_t ws_f = kbs_tc_rollout_ws_floats(h, n);
   const size_t lag_f = io->pg_carry ? size_t(T) * 3 * ld : 0;
   const size_t aobs_f = io->actor_obs ? 0 : size_t(T) * KBS_ACTOR_OBS * ld;
-  const size_t cobs_f = critic ? size_t(CT) * KBS_CRITIC_OBS * ld : 0;
+  const size_t cobs_f = critic && !critic_obs ? size_t(CT) * KBS_CRITIC_OBS * ld : 0;
   const size_t xsb_f = size_t(T) * sbf;
   const size_t osb_a_f = size_t(kbs_tc_obs_sb_floats(h, KBS_NET_ACTOR, n, CT));
   const size_t osb_c_f = critic ? size_t(kbs_tc_obs_sb_floats(h, KBS_NET_CRITIC, n, CT)) : 0;
@@ -117,7 +120,7 @@ int rollout_fused_tc(kbs_handle* h, const kbs_rollout_io* io, int64_t n, cudaStr
   float* ws = h->scratch;
   float* lagged = io->pg_carry ? ws + ws_f : nullptr;
   float* aobs = io->actor_obs ? io->actor_obs : ws + ws_f + lag_f;
-  float* cobs = critic ? ws + ws_f + lag_f + aobs_f : nullptr;
+  float* cobs = critic_obs ? critic_obs : critic ? ws + ws_f + lag_f + aobs_f : nullptr;
   float* xsb_a = ws + ws_f + lag_f + aobs_f + cobs_f;
   float* xsb_c = critic ? xsb_a + xsb_f : nullptr;
   float* osb_a = xsb_a + xsb_f * (critic ? 2 : 1);
@@ -126,7 +129,8 @@ int rollout_fused_tc(kbs_handle* h, const kbs_rollout_io* io, int64_t n, cudaStr
   if ((rc = kbs_launch_terminate(h, io->state, io->term_codes, io->done, io->success, nullptr, n, st, T))) return rc;
   if (lagged) {
     if ((rc = kbs_launch_phase_a_scans(h, io->command, io->u_switch, io->cmd_mode, io->cmd_u6, io->cmd_u_arms, io->done,
-                                       io->state.sensordata, io->episode.pg_lag, io->pg_carry, lagged, T, ld, n, st)))
+                                       done_prev, io->state.sensordata, io->episode.pg_lag, io->pg_carry, lagged, T, ld, n,
+                                       st)))
       return rc;
   } else if ((rc = kbs_launch_command_scan(h, io->command, io->u_switch, io->cmd_mode, io->cmd_u6, io->cmd_u_arms, io->done,
                                            T, ld, n, st))) {
@@ -147,11 +151,12 @@ int rollout_fused_tc(kbs_handle* h, const kbs_rollout_io* io, int64_t n, cudaStr
     const kbs_state_view s = state_at(io->state, t0);
     const kbs_noise_view nz = noise_at(io->noise, t0, ld);
     float* aobs_c = aobs + t0 * KBS_ACTOR_OBS * ld;
+    float* cobs_c = critic_obs ? critic_obs + t0 * KBS_CRITIC_OBS * ld : cobs;
     if ((rc = kbs_launch_observations(h, s, &nz, &io->episode, io->command + t0 * KBS_NUM_COMMANDS * ld, nullptr, nullptr,
-                                      nullptr, aobs_c, cobs, n, aux, tc, lagged ? lagged + t0 * 3 * ld : nullptr,
-                                      /*skip_dump=*/true)))
+                                      nullptr, aobs_c, cobs_c, n, aux, tc, lagged ? lagged + t0 * 3 * ld : nullptr,
+                                      /*skip_dump=*/critic_obs == nullptr)))
       return rc;
-    const float* obs_soa[2] = {aobs_c, cobs};
+    const float* obs_soa[2] = {aobs_c, cobs_c};
     float* obs_sb[2] = {osb_a, osb_c};
     float* xsb[2] = {xsb_a + size_t(t0) * sbf, critic ? xsb_c + size_t(t0) * sbf : nullptr};
     // one chunk (default): the actor's input projection is folded into layer 0 of the persistent kernel (r.x_is_obs)
@@ -887,6 +892,11 @@ int kbs_sample_actuator_randomization(kbs_handle* h, const kbs_actuator_rand_par
 }
 
 int kbs_rollout(kbs_handle* h, const kbs_rollout_io* io, int64_t n, void* stream) {
+  return kbs_rollout_record(h, io, nullptr, n, stream);
+}
+
+int kbs_rollout_record(kbs_handle* h, const kbs_rollout_io* io, const struct kbs_rollout_record* rec, int64_t n,
+                       void* stream) {
   REQ(h); REQ(io);
   if (io->T <= 0) return KBS_E_SHAPE;
   int rc = check_state(&io->state, n, true);
@@ -895,8 +905,13 @@ int kbs_rollout(kbs_handle* h, const kbs_rollout_io* io, int64_t n, void* stream
   REQ(io->state.time); REQ(io->command); REQ(io->actor_carry); REQ(io->lpf); REQ(io->action); REQ(io->ctrl);
   REQ(io->done); REQ(io->success); REQ(io->cmd_mode); REQ(io->cmd_u6); REQ(io->cmd_u_arms); REQ(io->u_switch);
   if (io->value) { REQ(io->critic_carry); REQ(io->state.cinert); REQ(io->state.cvel); REQ(io->state.actuator_force); }
+  const uint8_t* done_prev = rec ? rec->done_prev : nullptr;
+  float* critic_obs = rec ? rec->critic_obs : nullptr;
+  if (critic_obs) { REQ(io->state.cinert); REQ(io->state.cvel); REQ(io->state.actuator_force); }
+  AL(critic_obs);
+  if (reinterpret_cast<uintptr_t>(done_prev) & 3u) return KBS_E_ALIGN;
   cudaStream_t st = (cudaStream_t)stream;
-  if (h->p.gemm_path != KBS_GEMM_SIMT_FP32) return rollout_fused_tc(h, io, n, st);
+  if (h->p.gemm_path != KBS_GEMM_SIMT_FP32) return rollout_fused_tc(h, io, done_prev, critic_obs, n, st);
   const int64_t ld = io->state.ld;
   const size_t ts = trunk_scratch_floats(h, n);
   const size_t need = ts + size_t(n) * kOutLd + size_t(KBS_ACTOR_OBS + KBS_CRITIC_OBS) * ld + 64;
@@ -911,14 +926,14 @@ int kbs_rollout(kbs_handle* h, const kbs_rollout_io* io, int64_t n, void* stream
     const float* cmd_t = io->command + t * KBS_NUM_COMMANDS * ld;
     float* cmd_n = io->command + (t + 1) * KBS_NUM_COMMANDS * ld;
     float* aobs = io->actor_obs ? io->actor_obs + t * KBS_ACTOR_OBS * ld : aobs_scratch;
+    float* cobs_t = critic_obs ? critic_obs + t * KBS_CRITIC_OBS * ld : io->value ? cobs : nullptr;
     uint8_t* done_t = io->done + t * ld;
     // terminations of the recorded state decide which carries reset after this step (train.py:1502-1506)
     if ((rc = kbs_launch_terminate(h, s, io->term_codes ? io->term_codes + t * 3 * ld : nullptr, done_t,
                                    io->success + t * ld, nullptr, n, st)))
       return rc;
-    if ((rc = kbs_launch_observations(h, s, &nz, &io->episode, cmd_t, io->pg_carry, t > 0 ? done_t - ld : nullptr,
-                                      nullptr, aobs,
-                                      io->value ? cobs : nullptr, n, st)))
+    if ((rc = kbs_launch_observations(h, s, &nz, &io->episode, cmd_t, io->pg_carry, t > 0 ? done_t - ld : done_prev,
+                                      nullptr, aobs, cobs_t, n, st)))
       return rc;
     if ((rc = trunk(h, KBS_NET_ACTOR, aobs, ld, io->actor_carry, done_t, out_rm, n, st))) return rc;
     kbs_actor_out o{};
@@ -930,7 +945,7 @@ int kbs_rollout(kbs_handle* h, const kbs_rollout_io* io, int64_t n, void* stream
       return rc;
     if ((rc = kbs_launch_torque(h, o.action, s, &io->episode, io->ctrl + t * KBS_NUM_JOINTS * ld, n, st))) return rc;
     if (io->value) {
-      if ((rc = trunk(h, KBS_NET_CRITIC, cobs, ld, io->critic_carry, done_t, out_rm, n, st))) return rc;
+      if ((rc = trunk(h, KBS_NET_CRITIC, cobs_t, ld, io->critic_carry, done_t, out_rm, n, st))) return rc;
       if ((rc = kbs_launch_critic_head(h, out_rm, kOutLd, io->value + t * ld, n, st))) return rc;
     }
     if ((rc = kbs_launch_command(h, cmd_t, cmd_n, io->u_switch + t * ld, io->cmd_mode + t * ld,

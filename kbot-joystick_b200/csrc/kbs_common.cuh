@@ -135,10 +135,10 @@ int kbs_launch_command(kbs_handle* h, const float* cmd_in, float* cmd_out, const
 int kbs_launch_command_scan(kbs_handle* h, float* command, const float* u_switch, const int32_t* mode, const float* u6,
                             const float* u_arms, const uint8_t* done, int64_t T, int64_t ld, int64_t n, cudaStream_t st);
 int kbs_launch_phase_a_scans(kbs_handle* h, float* command, const float* u_switch, const int32_t* mode, const float* u6,
-                             const float* u_arms, const uint8_t* done, const float* sensordata, const float* lag,
-                             float* pg_carry, float* lagged, int64_t T, int64_t ld, int64_t n, cudaStream_t st);
-int kbs_launch_pg_scan(kbs_handle* h, const float* sensordata, const float* lag, const uint8_t* done, float* pg_carry,
-                       float* lagged, int64_t T, int64_t ld, int64_t n, cudaStream_t st);
+                             const float* u_arms, const uint8_t* done, const uint8_t* done_prev, const float* sensordata,
+                             const float* lag, float* pg_carry, float* lagged, int64_t T, int64_t ld, int64_t n, cudaStream_t st);
+int kbs_launch_pg_scan(kbs_handle* h, const float* sensordata, const float* lag, const uint8_t* done, const uint8_t* done_prev,
+                       float* pg_carry, float* lagged, int64_t T, int64_t ld, int64_t n, cudaStream_t st);
 int kbs_launch_torque(kbs_handle* h, const float* action, const kbs_state_view& s, const kbs_episode_view* ep,
                       float* ctrl, int64_t n, cudaStream_t st);
 int kbs_launch_torque_substeps(kbs_handle* h, const float* action, float* prev_action, const float* u_drop, const float* latency,

@@ -1325,14 +1325,16 @@ command_scan_body(const kbs_params& P, int k, float* __restrict__ command /*[T+1
 }
 
 // Lagged projected gravity (ProjectedGravityObservation min_lag/max_lag): x_t = lag x_{t-1} + (1-lag) g_b(t), restarted at
-// g_b(t) on the first step of a new episode (done[t-1]).  pg_carry in/out; lagged[T][3][ld] out.
+// g_b(t) on the first step of a new episode (done[t-1]; at t = 0, done_prev[e] = the previous call's done[T-1], NULL = no
+// restart).  pg_carry in/out; lagged[T][3][ld] out.
 __device__ __forceinline__ void
 pg_scan_body(const kbs_params& P, const float* __restrict__ sensordata, const float* __restrict__ lag_p,
-               const uint8_t* __restrict__ done, float* __restrict__ pg_carry, float* __restrict__ lagged, int64_t T,
-               int64_t ld, int64_t n) {
+               const uint8_t* __restrict__ done, const uint8_t* __restrict__ done_prev, float* __restrict__ pg_carry,
+               float* __restrict__ lagged, int64_t T, int64_t ld, int64_t n) {
   const int64_t e = int64_t(blockIdx.x) * kThreads + threadIdx.x;
   if (e >= n) return;
   const float lag = lag_p ? lag_p[e] : 0.0f;
+  const bool rs0 = done_prev && done_prev[e] != 0;
   float x[3] = {pg_carry[e], pg_carry[ld + e], pg_carry[2 * ld + e]};
   // the inputs of step t do not depend on the recurrence: fetch 8 steps at a time so the load latencies overlap
   constexpr int kB = 8;
@@ -1344,7 +1346,7 @@ pg_scan_body(const kbs_params& P, const float* __restrict__ sensordata, const fl
       const int64_t t = t0 + i < T ? t0 + i : T - 1;
       const float* sd = sensordata + (t * KBS_NSENSORDATA + P.sd_imu_quat) * ld + e;
       qv[i][0] = sd[0]; qv[i][1] = sd[ld]; qv[i][2] = sd[2 * ld]; qv[i][3] = sd[3 * ld];
-      rsv[i] = (t > 0) && (done[(t - 1) * ld + e] != 0);
+      rsv[i] = t > 0 ? (done[(t - 1) * ld + e] != 0) : rs0;
     }
 #pragma unroll
     for (int i = 0; i < kB; ++i) {
@@ -1373,19 +1375,20 @@ command_scan_kernel(const __grid_constant__ kbs_params P, float* __restrict__ co
 }
 __global__ void __launch_bounds__(kThreads)
 pg_scan_kernel(const __grid_constant__ kbs_params P, const float* __restrict__ sensordata, const float* __restrict__ lag_p,
-               const uint8_t* __restrict__ done, float* __restrict__ pg_carry, float* __restrict__ lagged, int64_t T,
-               int64_t ld, int64_t n) {
-  pg_scan_body(P, sensordata, lag_p, done, pg_carry, lagged, T, ld, n);
+               const uint8_t* __restrict__ done, const uint8_t* __restrict__ done_prev, float* __restrict__ pg_carry,
+               float* __restrict__ lagged, int64_t T, int64_t ld, int64_t n) {
+  pg_scan_body(P, sensordata, lag_p, done, done_prev, pg_carry, lagged, T, ld, n);
 }
 // Both scans of the fused rollout's phase A in one launch (they only depend on `done`): blockIdx.y = 0..15 command rows,
 // 16 = the lagged-gravity scan -- two latency-bound kernels side by side instead of back to back.
 __global__ void __launch_bounds__(kThreads, 4)
 phase_a_scans_kernel(const __grid_constant__ kbs_params P, float* __restrict__ command, const float* __restrict__ u_switch,
                      const int32_t* __restrict__ mode, const float* __restrict__ u6, const float* __restrict__ u_arms,
-                     const uint8_t* __restrict__ done, const float* __restrict__ sensordata, const float* __restrict__ lag_p,
-                     float* __restrict__ pg_carry, float* __restrict__ lagged, int64_t T, int64_t ld, int64_t n) {
+                     const uint8_t* __restrict__ done, const uint8_t* __restrict__ done_prev,
+                     const float* __restrict__ sensordata, const float* __restrict__ lag_p, float* __restrict__ pg_carry,
+                     float* __restrict__ lagged, int64_t T, int64_t ld, int64_t n) {
   if (blockIdx.y < KBS_NUM_COMMANDS) command_scan_body(P, blockIdx.y, command, u_switch, mode, u6, u_arms, done, T, ld, n);
-  else pg_scan_body(P, sensordata, lag_p, done, pg_carry, lagged, T, ld, n);
+  else pg_scan_body(P, sensordata, lag_p, done, done_prev, pg_carry, lagged, T, ld, n);
 }
 
 inline unsigned groups4(int64_t n) { return unsigned((((n + 3) / 4) + kThreads - 1) / kThreads); }
@@ -1480,19 +1483,19 @@ int kbs_launch_command_scan(kbs_handle* h, float* command, const float* u_switch
 }
 
 int kbs_launch_phase_a_scans(kbs_handle* h, float* command, const float* u_switch, const int32_t* mode, const float* u6,
-                             const float* u_arms, const uint8_t* done, const float* sensordata, const float* lag,
-                             float* pg_carry, float* lagged, int64_t T, int64_t ld, int64_t n, cudaStream_t st) {
+                             const float* u_arms, const uint8_t* done, const uint8_t* done_prev, const float* sensordata,
+                             const float* lag, float* pg_carry, float* lagged, int64_t T, int64_t ld, int64_t n, cudaStream_t st) {
   KBS_LAUNCH(h, KBS_K_COMMAND, st,
              (phase_a_scans_kernel<<<dim3(unsigned((n + kThreads - 1) / kThreads), KBS_NUM_COMMANDS + 1), kThreads, 0, st>>>(
-                 h->p, command, u_switch, mode, u6, u_arms, done, sensordata, lag, pg_carry, lagged, T, ld, n)));
+                 h->p, command, u_switch, mode, u6, u_arms, done, done_prev, sensordata, lag, pg_carry, lagged, T, ld, n)));
   KBS_LAUNCH_CHECK();
   return KBS_OK;
 }
 
-int kbs_launch_pg_scan(kbs_handle* h, const float* sensordata, const float* lag, const uint8_t* done, float* pg_carry,
-                       float* lagged, int64_t T, int64_t ld, int64_t n, cudaStream_t st) {
+int kbs_launch_pg_scan(kbs_handle* h, const float* sensordata, const float* lag, const uint8_t* done, const uint8_t* done_prev,
+                       float* pg_carry, float* lagged, int64_t T, int64_t ld, int64_t n, cudaStream_t st) {
   KBS_LAUNCH(h, KBS_K_OBS, st,
-             (pg_scan_kernel<<<unsigned((n + kThreads - 1) / kThreads), kThreads, 0, st>>>(h->p, sensordata, lag, done,
+             (pg_scan_kernel<<<unsigned((n + kThreads - 1) / kThreads), kThreads, 0, st>>>(h->p, sensordata, lag, done, done_prev,
                                                                                          pg_carry, lagged, T, ld, n)));
   KBS_LAUNCH_CHECK();
   return KBS_OK;

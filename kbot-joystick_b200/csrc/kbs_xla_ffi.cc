@@ -149,20 +149,21 @@ ffi::Error CriticStepImpl(cudaStream_t stream, int64_t handle, int64_t n_envs, F
 // state [T][rows][ld] x 10; noise [T][46][ld]; episode [88][ld] = jpos_bias 20 | pg_lag 1 | pg_bias 3 | kp 20 | kd 20 | tau_limit
 // 20 | action_bias 20 ... (torque_bias: a separate [20][ld]); randomness eps_action [T][20][ld], u_switch [T][ld], cmd_mode s32
 // [T][ld], cmd_u6 [T][6][ld], cmd_u_arms [T][10][ld]; command0 [16][ld]; carries in-out.
-ffi::Error RolloutImpl(cudaStream_t stream, int64_t handle, int64_t n_envs, F32 qpos, F32 qvel, F32 sensordata, F32 xpos, F32 xquat,
-                       F32 cinert, F32 cvel, F32 actuator_force, F32 com_distance, F32 time, F32 eps_jpos, F32 eps_jvel,
-                       F32 eps_gyro, F32 eps_pg, F32 episode, F32 torque_bias, F32 eps_action, F32 u_switch, S32 cmd_mode, F32 cmd_u6,
-                       F32 cmd_u_arms, F32 command0, F32 pg_carry, F32 actor_carry, F32 critic_carry, F32 lpf, RF32 command,
-                       RF32 pg_carry_out, RF32 actor_carry_out, RF32 critic_carry_out, RF32 lpf_out, RF32 actor_obs, RF32 action,
-                       RF32 log_prob, RF32 ctrl, RS32 term_codes, RU8 done, RU8 success, RF32 value) {
+// RolloutIo: the in-out copies and the kbs_rollout_io both rollout handlers pass; false = a copy failed.
+bool RolloutIo(cudaStream_t stream, F32& qpos, F32& qvel, F32& sensordata, F32& xpos, F32& xquat, F32& cinert, F32& cvel,
+               F32& actuator_force, F32& com_distance, F32& time, F32& eps_jpos, F32& eps_jvel, F32& eps_gyro, F32& eps_pg,
+               F32& episode, F32& torque_bias, F32& eps_action, F32& u_switch, S32& cmd_mode, F32& cmd_u6, F32& cmd_u_arms,
+               F32& command0, F32& pg_carry, F32& actor_carry, F32& critic_carry, F32& lpf, RF32& command, RF32& pg_carry_out,
+               RF32& actor_carry_out, RF32& critic_carry_out, RF32& lpf_out, RF32& actor_obs, RF32& action, RF32& log_prob,
+               RF32& ctrl, RS32& term_codes, RU8& done, RU8& success, RF32& value, kbs_rollout_io& io) {
   if (!Carry(stream, pg_carry, pg_carry_out) || !Carry(stream, actor_carry, actor_carry_out) ||
       !Carry(stream, critic_carry, critic_carry_out) || !Carry(stream, lpf, lpf_out))
-    return ffi::Error::Internal("kbs_rollout: carry copy failed");
+    return false;
   const int64_t T = Dim(qpos, 0), ld = Dim(qpos, 2);
   // row 0 of the [T + 1][16][ld] command trajectory is the command at step 0 (input)
   if (cudaMemcpyAsync(command->typed_data(), command0.typed_data(), command0.size_bytes(), cudaMemcpyDeviceToDevice, stream) != cudaSuccess)
-    return ffi::Error::Internal("kbs_rollout: command copy failed");
-  kbs_rollout_io io{};
+    return false;
+  io = kbs_rollout_io{};
   io.state.qpos = qpos.typed_data(); io.state.qvel = qvel.typed_data(); io.state.sensordata = sensordata.typed_data();
   io.state.xpos = xpos.typed_data(); io.state.xquat = xquat.typed_data(); io.state.cinert = cinert.typed_data();
   io.state.cvel = cvel.typed_data(); io.state.actuator_force = actuator_force.typed_data();
@@ -180,7 +181,34 @@ ffi::Error RolloutImpl(cudaStream_t stream, int64_t handle, int64_t n_envs, F32 
   io.action = action->typed_data(); io.log_prob = log_prob->typed_data(); io.ctrl = ctrl->typed_data();
   io.term_codes = term_codes->typed_data(); io.done = done->typed_data(); io.success = success->typed_data();
   io.value = value->typed_data(); io.T = T;
+  return true;
+}
+#define KBS_ROLLOUT_PARAMS                                                                                                      \
+  F32 qpos, F32 qvel, F32 sensordata, F32 xpos, F32 xquat, F32 cinert, F32 cvel, F32 actuator_force, F32 com_distance, F32 time, \
+      F32 eps_jpos, F32 eps_jvel, F32 eps_gyro, F32 eps_pg, F32 episode, F32 torque_bias, F32 eps_action, F32 u_switch,          \
+      S32 cmd_mode, F32 cmd_u6, F32 cmd_u_arms, F32 command0, F32 pg_carry, F32 actor_carry, F32 critic_carry, F32 lpf
+#define KBS_ROLLOUT_RESULTS                                                                                                    \
+  RF32 command, RF32 pg_carry_out, RF32 actor_carry_out, RF32 critic_carry_out, RF32 lpf_out, RF32 actor_obs, RF32 action,      \
+      RF32 log_prob, RF32 ctrl, RS32 term_codes, RU8 done, RU8 success, RF32 value
+#define KBS_ROLLOUT_IO_ARGS                                                                                                    \
+  qpos, qvel, sensordata, xpos, xquat, cinert, cvel, actuator_force, com_distance, time, eps_jpos, eps_jvel, eps_gyro, eps_pg, \
+      episode, torque_bias, eps_action, u_switch, cmd_mode, cmd_u6, cmd_u_arms, command0, pg_carry, actor_carry, critic_carry,  \
+      lpf, command, pg_carry_out, actor_carry_out, critic_carry_out, lpf_out, actor_obs, action, log_prob, ctrl, term_codes,   \
+      done, success, value
+ffi::Error RolloutImpl(cudaStream_t stream, int64_t handle, int64_t n_envs, KBS_ROLLOUT_PARAMS, KBS_ROLLOUT_RESULTS) {
+  kbs_rollout_io io;
+  if (!RolloutIo(stream, KBS_ROLLOUT_IO_ARGS, io)) return ffi::Error::Internal("kbs_rollout: carry copy failed");
   return Rc(kbs_rollout(H(handle), &io, n_envs, stream));
+}
+
+// ---- the same step, continued across calls (ksim's engine loop: one step per call) and recording what the update trains on:
+//      done_prev u8 [ld] = the previous call's done[T-1] (zeros on the first call); critic_obs [T][475][ld] out ----------------
+ffi::Error RolloutRecordImpl(cudaStream_t stream, int64_t handle, int64_t n_envs, KBS_ROLLOUT_PARAMS, U8 done_prev,
+                             KBS_ROLLOUT_RESULTS, RF32 critic_obs) {
+  kbs_rollout_io io;
+  if (!RolloutIo(stream, KBS_ROLLOUT_IO_ARGS, io)) return ffi::Error::Internal("kbs_rollout_record: carry copy failed");
+  struct kbs_rollout_record rec{done_prev.typed_data(), critic_obs->typed_data()};
+  return Rc(kbs_rollout_record(H(handle), &io, &rec, n_envs, stream));
 }
 
 // ---- get_ppo_variables -> xax.scan(_ppo_scan_fn) (train.py:1435-1524) on a stored trajectory, aux_losses included ------------
@@ -322,6 +350,12 @@ XLA_FFI_DEFINE_HANDLER_SYMBOL(KbsRollout, RolloutImpl,
                                   .Arg<S32>().Arg<F32>().Arg<F32>().Arg<F32>().Arg<F32>().Arg<F32>().Arg<F32>().Arg<F32>()
                                   .Ret<F32>().Ret<F32>().Ret<F32>().Ret<F32>().Ret<F32>().Ret<F32>().Ret<F32>().Ret<F32>().Ret<F32>()
                                   .Ret<S32>().Ret<U8>().Ret<U8>().Ret<F32>());
+XLA_FFI_DEFINE_HANDLER_SYMBOL(KbsRolloutRecord, RolloutRecordImpl,
+                              KBS_BIND_N().Arg<F32>().Arg<F32>().Arg<F32>().Arg<F32>().Arg<F32>().Arg<F32>().Arg<F32>().Arg<F32>().Arg<F32>()
+                                  .Arg<F32>().Arg<F32>().Arg<F32>().Arg<F32>().Arg<F32>().Arg<F32>().Arg<F32>().Arg<F32>().Arg<F32>()
+                                  .Arg<S32>().Arg<F32>().Arg<F32>().Arg<F32>().Arg<F32>().Arg<F32>().Arg<F32>().Arg<F32>().Arg<U8>()
+                                  .Ret<F32>().Ret<F32>().Ret<F32>().Ret<F32>().Ret<F32>().Ret<F32>().Ret<F32>().Ret<F32>().Ret<F32>()
+                                  .Ret<S32>().Ret<U8>().Ret<U8>().Ret<F32>().Ret<F32>());
 XLA_FFI_DEFINE_HANDLER_SYMBOL(KbsPpoVariables, PpoVariablesImpl,
                               KBS_BIND_N().Attr<float>("actor_mirror_loss_scale").Attr<float>("critic_mirror_loss_scale")
                                   .Arg<F32>().Arg<F32>().Arg<F32>().Arg<F32>().Arg<F32>().Arg<U8>().Arg<F32>().Arg<F32>().Arg<F32>()

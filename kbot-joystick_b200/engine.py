@@ -451,7 +451,10 @@ class KbotStep:
                                                     n_envs, _stream()), "kbs_generate_rollout_noise")
 
     def rollout(self, io: dict, n_envs: int) -> None:
-        """io: tensors named as the fields of kbs_rollout_io (state/noise/episode are nested dicts)."""
+        """io: tensors named as the fields of kbs_rollout_io (state/noise/episode are nested dicts).  With io["done_prev"]
+        (u8 [ld], the previous call's done[T-1]) or io["critic_obs"] ([T, 475, ld], written) present and not None, the call
+        is kbs_rollout_record: the lag state restarts on step 0 where done_prev != 0, and every step's critic concatenation
+        is recorded."""
         r = L.KbsRolloutIO()
         ld = io["state"]["qpos"].shape[-1]
         r.state = _view(L.KbsStateView, STATE_ROWS, io["state"], ld)
@@ -462,4 +465,8 @@ class KbotStep:
                 continue
             setattr(r, k, L.ptr(io.get(k)))
         r.T = io["T"]
-        L.check(self.lib.kbs_rollout(self._h, C.byref(r), n_envs, _stream()), "kbs_rollout")
+        if io.get("done_prev") is None and io.get("critic_obs") is None:
+            L.check(self.lib.kbs_rollout(self._h, C.byref(r), n_envs, _stream()), "kbs_rollout")
+            return
+        rec = L.KbsRolloutRecord(L.ptr(io.get("done_prev")), L.ptr(io.get("critic_obs")))
+        L.check(self.lib.kbs_rollout_record(self._h, C.byref(r), C.byref(rec), n_envs, _stream()), "kbs_rollout_record")

@@ -24,7 +24,8 @@ _TARGETS = {
     "kbs_gae": "KbsGae", "kbs_terminate": "KbsTerminate", "kbs_torque": "KbsTorque",
     "kbs_sample_actuator_randomization": "KbsSampleActuatorRandomization", "kbs_policy_step": "KbsPolicyStep",
     "kbs_observations": "KbsObservations", "kbs_command_update": "KbsCommandUpdate", "kbs_actor_step": "KbsActorStep",
-    "kbs_critic_step": "KbsCriticStep", "kbs_rollout": "KbsRollout", "kbs_ppo_variables": "KbsPpoVariables",
+    "kbs_critic_step": "KbsCriticStep", "kbs_rollout": "KbsRollout",
+    "kbs_rollout_record": "KbsRolloutRecord", "kbs_ppo_variables": "KbsPpoVariables",
     "kbs_mirror_observations": "KbsMirrorObservations", "kbs_mirror_joints": "KbsMirrorJoints",
     "kbs_com_distance": "KbsComDistance", "kbs_rewards": "KbsRewards", "kbs_ppo_grad": "KbsPpoGrad",
     "kbs_grad_norm": "KbsGradNorm", "kbs_adamw_step": "KbsAdamwStep",
@@ -159,6 +160,29 @@ def rollout(handle: int, state: dict, noise: dict, episode, torque_bias, rand: d
                noise["eps_gyro"], noise["eps_pg"], episode, torque_bias, rand["eps_action"], rand["u_switch"],
                rand["cmd_mode"].astype(jnp.int32), rand["cmd_u6"], rand["cmd_u_arms"], command0, pg_carry, actor_carry, critic_carry,
                lpf, **_h(np, handle, n_envs=n_envs))
+    return dict(zip(names, res))
+
+
+def rollout_record(handle: int, state: dict, noise: dict, episode, torque_bias, rand: dict, command0, pg_carry, actor_carry,
+                   critic_carry, lpf, done_prev, n_envs: int):
+    """rollout() continued across calls (kbs_rollout_record): done_prev [ld] is the previous call's done[T-1] (zeros on the
+    first call), so the lag state restarts where an episode ended on the previous call's last step -- with one step per call,
+    as ksim's engine loop makes it, that is every episode end.  -> rollout()'s dict plus critic_obs [T, 475, ld], the
+    critic's concatenation of every step."""
+    jax, jnp, np = _j()
+    T, _, ld = state["qpos"].shape
+    f32 = jnp.float32
+    names = ("command", "pg_carry", "actor_carry", "critic_carry", "lpf", "actor_obs", "action", "log_prob", "ctrl", "term_codes",
+             "done", "success", "value", "critic_obs")
+    out = (_sds(jax, (T + 1, 16, ld), f32), _sds(jax, pg_carry.shape, f32), _sds(jax, actor_carry.shape, f32),
+           _sds(jax, critic_carry.shape, f32), _sds(jax, lpf.shape, f32), _sds(jax, (T, 65, ld), f32), _sds(jax, (T, 20, ld), f32),
+           _sds(jax, (T, ld), f32), _sds(jax, (T, 20, ld), f32), _sds(jax, (T, 3, ld), jnp.int32), _sds(jax, (T, ld), jnp.uint8),
+           _sds(jax, (T, ld), jnp.uint8), _sds(jax, (T, ld), f32), _sds(jax, (T, 475, ld), f32))
+    call = jax.ffi.ffi_call("kbs_rollout_record", out, input_output_aliases={22: 1, 23: 2, 24: 3, 25: 4})
+    res = call(*(state[k] for k, _ in STATE_ROWS), state["com_distance"], state["time"], noise["eps_jpos"], noise["eps_jvel"],
+               noise["eps_gyro"], noise["eps_pg"], episode, torque_bias, rand["eps_action"], rand["u_switch"],
+               rand["cmd_mode"].astype(jnp.int32), rand["cmd_u6"], rand["cmd_u_arms"], command0, pg_carry, actor_carry, critic_carry,
+               lpf, done_prev.astype(jnp.uint8), **_h(np, handle, n_envs=n_envs))
     return dict(zip(names, res))
 
 

@@ -58,7 +58,9 @@ class PpoUpdater:
     slice of the flat gradient is all-reduced on a communication stream while the actor's weight-gradient GEMMs still run,
     the actor's slice follows.  With `capture()` the WHOLE update -- gradients, both all-reduces, norm, AdamW, re-pack --
     is one CUDA graph (the step counter lives on the device).  `epoch()` runs the update phase of a whole PPO epoch on a
-    stored rollout (device-shuffled minibatches of whole trajectories); `capture_epoch()` records it as one CUDA graph."""
+    stored rollout (device-shuffled minibatches of whole trajectories); `capture_epoch()` records it as one CUDA graph.
+    `iteration()` runs a whole PPO iteration -- rollout, rewards, epoch -- on the rollout the library records, and
+    `capture_iteration()` records that as one CUDA graph."""
 
     def __init__(self, engine, w_actor: dict, w_critic: dict, lr: float = 5e-4, b1: float = 0.9, b2: float = 0.999,
                  eps: float = 1e-8, weight_decay: float = 1e-5, max_grad_norm: float = 10.0, **loss_hyper):
@@ -81,6 +83,7 @@ class PpoUpdater:
         self._graph = None
         self.pass_dev = torch.zeros(1, device=dev, dtype=torch.int64)    # passes drawn so far (epoch(): one permutation each)
         self._ework, self._epoch_graph = None, None
+        self._iwork, self._iter_graph = None, None
         self._repack(sync=True)
 
     def _repack(self, sync: bool = False):
@@ -212,6 +215,70 @@ class PpoUpdater:
         self._epoch_rollout = rollout
         self._epoch_args = (n_envs, batch_size, num_passes, seed)
         self._epoch_graph_work = self._ework       # the graph holds its buffers' addresses: keep them if the shapes change
+        self.eng.scratch_lock(True)
+
+    # ---- a whole iteration: rollout -> rewards -> epoch ---------------------------------------------------------------------
+    def _iteration_work(self, io: dict, n_envs: int) -> dict:
+        """What an iteration keeps besides the caller's io, allocated once per shape: the carries at the rollout's first step,
+        the recorded critic observations, the rewards, and done_prev (the previous iteration's done[T-1]; zero before the
+        first iteration, which restarts nothing, as no done_prev)."""
+        T, _, ld = io["actor_obs"].shape
+        key = (T, ld, n_envs, tuple(io["actor_carry"].shape))
+        w = self._iwork
+        if w is not None and w["key"] == key:
+            return w
+        dev = self.param.device
+        w = {"key": key, "actor_carry0": torch.empty_like(io["actor_carry"]), "critic_carry0": torch.empty_like(io["critic_carry"]),
+             "lpf0": torch.empty_like(io["lpf"]), "critic_obs": torch.empty((T, L.CRITIC_OBS, ld), device=dev),
+             "rewards": torch.empty((T, ld), device=dev), "done_prev": torch.zeros((ld,), dtype=torch.uint8, device=dev)}
+        self._iwork = w
+        return w
+
+    def _iteration(self, io: dict, reward_carry: dict, n_envs: int, batch_size: int, num_passes: int, seed: int) -> dict:
+        """One PPO iteration, enqueued on the current stream: carry snapshot -> kbs_rollout_record (value, critic_obs,
+        done_prev) -> kbs_rewards -> the epoch's update phase -> done[T-1] and command[T] carried into the next iteration."""
+        T = io["T"]
+        w = self._iteration_work(io, n_envs)
+        for k in ("actor_carry", "critic_carry", "lpf"):      # kbs_rollout advances them in place
+            w[k + "0"].copy_(io[k])
+        self.eng.rollout(dict(io, done_prev=w["done_prev"], critic_obs=w["critic_obs"]), n_envs)
+        self.eng.rewards(io["state"], io["command"][:T], io["ctrl"], io["done"], reward_carry, total=w["rewards"], n_envs=n_envs)
+        rollout = {"actor_obs": io["actor_obs"], "critic_obs": w["critic_obs"], "action": io["action"], "done": io["done"],
+                   "success": io["success"], "rewards": w["rewards"], "actor_carry0": w["actor_carry0"],
+                   "critic_carry0": w["critic_carry0"], "lpf0": w["lpf0"]}
+        out = self._epoch(rollout, n_envs, batch_size, num_passes, seed)
+        w["done_prev"].copy_(io["done"][T - 1])
+        io["command"][0].copy_(io["command"][T])
+        return dict(out, rewards=w["rewards"])
+
+    def iteration(self, io: dict, reward_carry: dict, n_envs: int, batch_size: int = 512, num_passes: int = 3,
+                  seed: int = 0) -> dict:
+        """One whole PPO iteration on the device, no host synchronisation: the rollout over io's recorded state (as
+        KbotStep.rollout; io needs actor_obs, value and critic_carry), the rewards of that trajectory (reward_carry: t_single,
+        airtime, prev_contact, advanced in place), then epoch() on what the rollout recorded.  Afterwards io is ready for the
+        next iteration: its carries, lpf and pg_carry are the final ones, command[0] = command[T], and the next rollout gets this
+        one's done[T-1], so consecutive iterations are one continuous rollout.  Refill io's state and noise in place between
+        iterations.  n_envs <= 16 384 per rank (the permutation's limit).  Returns epoch()'s "stats", "norms", "perm" and
+        "rewards" [T, ld], device tensors overwritten by the next iteration.  After capture_iteration, a call with the same io,
+        reward_carry and arguments replays the graph."""
+        if self._iter_graph is not None and io is self._iter_io and reward_carry is self._iter_reward_carry and \
+                self._iter_args == (n_envs, batch_size, num_passes, seed):
+            self._iter_graph.replay()
+            return self._iter_out
+        return self._iteration(io, reward_carry, n_envs, batch_size, num_passes, seed)
+
+    def capture_iteration(self, io: dict, reward_carry: dict, n_envs: int, batch_size: int = 512, num_passes: int = 3,
+                          seed: int = 0) -> None:
+        """Record one whole iteration() as ONE CUDA graph; later iteration() calls with the same io, reward_carry and
+        arguments replay it.  Call after one eager iteration with the same arguments (the handle's scratch has then grown to
+        what the rollout and the epoch need, and is locked here)."""
+        torch.cuda.synchronize()
+        self._iter_graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(self._iter_graph):
+            self._iter_out = self._iteration(io, reward_carry, n_envs, batch_size, num_passes, seed)
+        self._iter_io, self._iter_reward_carry = io, reward_carry
+        self._iter_args = (n_envs, batch_size, num_passes, seed)
+        self._iter_graph_work = (self._iwork, self._ework)     # the graph holds their addresses
         self.eng.scratch_lock(True)
 
     @property
