@@ -65,26 +65,33 @@ kbs_noise_view noise_at(const kbs_noise_view& z, int64_t t, int64_t ld) {
   return o;
 }
 
-// Scratch layout of one trunk evaluation: [trunk workspace (path dependent) | out_rm [n][64]].
-size_t trunk_scratch_floats(const kbs_handle* h, int64_t n) {
-  return h->p.gemm_path != KBS_GEMM_SIMT_FP32 ? kbs_tc_scratch_floats(h, n) : kbs_simt_scratch_floats(h, n);
-}
-
-int trunk(kbs_handle* h, int net, const float* obs, int64_t ld, float* carry, const uint8_t* done, float* out_rm,
-          int64_t n, cudaStream_t st) {
-  if (h->p.gemm_path == KBS_GEMM_SIMT_FP32) return kbs_simt_trunk(h, net, obs, ld, carry, done, out_rm, n, st);
-  // tensor-core path: input_proj (FFMA, K = 65 / 475) -> LSTM stack on tcgen05 -> output_proj (FFMA, N = 40 / 1)
-  const size_t H = size_t(h->p.hidden_size);
-  float* ws = h->scratch;
-  float* x_rm = ws + kbs_tc_scratch_floats(h, n) - 2 * size_t(n) * H - 256;   // tail of the TC workspace
-  float* hbuf = x_rm + size_t(n) * H;
-  int rc;
-  if ((rc = kbs_simt_in_proj(h, net, obs, ld, x_rm, n, st))) return rc;
-  if ((rc = kbs_tc_lstm_stack(h, net, x_rm, carry, done, hbuf, ws, n, false, st))) return rc;
-  return kbs_simt_out_proj(h, net, hbuf, out_rm, n, st);
-}
-
 constexpr int kOutLd = 64;  // row stride of the trunk output buffer
+
+// Workspace of one trunk evaluation: the exact-fp32 trunk's, or the tensor-core LSTM stack's plus its row-major input and
+// top-layer output [n][H]; then the trunk's output out_rm [n][kOutLd].
+struct TrunkWs { KbsSimtTrunkWs simt; KbsTcStackWs tc; float* x_rm; float* hbuf; float* out_rm; };
+TrunkWs trunk_ws(KbsScratch& s, const kbs_handle* h, int64_t n) {
+  TrunkWs w{};
+  if (h->p.gemm_path == KBS_GEMM_SIMT_FP32) {
+    w.simt = kbs_simt_trunk_ws(s, h, n);
+  } else {
+    w.tc = kbs_tc_stack_ws(s, h, n);
+    w.x_rm = s.take<float>(size_t(n) * h->p.hidden_size);
+    w.hbuf = s.take<float>(size_t(n) * h->p.hidden_size);
+  }
+  w.out_rm = s.take<float>(size_t(n) * kOutLd);
+  return w;
+}
+
+int trunk(kbs_handle* h, int net, const float* obs, int64_t ld, float* carry, const uint8_t* done, const TrunkWs& ws, int64_t n,
+          cudaStream_t st) {
+  if (h->p.gemm_path == KBS_GEMM_SIMT_FP32) return kbs_simt_trunk(h, net, obs, ld, carry, done, ws.out_rm, ws.simt, n, st);
+  // tensor-core path: input_proj (FFMA, K = 65 / 475) -> LSTM stack on tcgen05 -> output_proj (FFMA, N = 40 / 1)
+  int rc;
+  if ((rc = kbs_simt_in_proj(h, net, obs, ld, ws.x_rm, n, st))) return rc;
+  if ((rc = kbs_tc_lstm_stack(h, net, ws.x_rm, carry, done, ws.hbuf, ws.tc, n, false, st))) return rc;
+  return kbs_simt_out_proj(h, net, ws.hbuf, ws.out_rm, n, st);
+}
 
 // Fused rollout on the tensor-core path.  The state is recorded, so everything that does not depend on the networks
 // is evaluated for all T steps first (terminations, command law, lagged gravity, observations, input projections:
@@ -108,23 +115,19 @@ int rollout_fused_tc(kbs_handle* h, const kbs_rollout_io* io, const uint8_t* don
   }
   const int64_t CT = (T + chunks_cfg - 1) / chunks_cfg;
   const size_t sbf = size_t(kbs_tc_sb_floats(h, n));
-  const size_t ws_f = kbs_tc_rollout_ws_floats(h, n);
-  const size_t lag_f = io->pg_carry ? size_t(T) * 3 * ld : 0;
-  const size_t aobs_f = io->actor_obs ? 0 : size_t(T) * KBS_ACTOR_OBS * ld;
-  const size_t cobs_f = critic && !critic_obs ? size_t(CT) * KBS_CRITIC_OBS * ld : 0;
-  const size_t xsb_f = size_t(T) * sbf;
-  const size_t osb_a_f = size_t(kbs_tc_obs_sb_floats(h, KBS_NET_ACTOR, n, CT));
-  const size_t osb_c_f = critic ? size_t(kbs_tc_obs_sb_floats(h, KBS_NET_CRITIC, n, CT)) : 0;
-  int rc = kbs_scratch_reserve(h, ws_f + lag_f + aobs_f + cobs_f + xsb_f * (critic ? 2 : 1) + osb_a_f + osb_c_f + 64);
+  KbsTcRolloutArgs r{};
+  float *lagged, *aobs, *cobs, *xsb_a, *xsb_c, *osb_a, *osb_c;
+  int rc = kbs_scratch(h, [&](KbsScratch& s) {
+    r.ws = kbs_tc_rollout_ws(s, h, n, critic ? 2 : 1);
+    lagged = io->pg_carry ? s.take<float>(size_t(T) * 3 * ld) : nullptr;
+    aobs = io->actor_obs ? io->actor_obs : s.take<float>(size_t(T) * KBS_ACTOR_OBS * ld);
+    cobs = critic_obs ? critic_obs : critic ? s.take<float>(size_t(CT) * KBS_CRITIC_OBS * ld) : nullptr;
+    xsb_a = s.take<float>(size_t(T) * sbf);
+    xsb_c = critic ? s.take<float>(size_t(T) * sbf) : nullptr;
+    osb_a = s.take<float>(kbs_tc_obs_sb_floats(h, KBS_NET_ACTOR, n, CT));
+    osb_c = critic ? s.take<float>(kbs_tc_obs_sb_floats(h, KBS_NET_CRITIC, n, CT)) : nullptr;
+  });
   if (rc) return rc;
-  float* ws = h->scratch;
-  float* lagged = io->pg_carry ? ws + ws_f : nullptr;
-  float* aobs = io->actor_obs ? io->actor_obs : ws + ws_f + lag_f;
-  float* cobs = critic_obs ? critic_obs : critic ? ws + ws_f + lag_f + aobs_f : nullptr;
-  float* xsb_a = ws + ws_f + lag_f + aobs_f + cobs_f;
-  float* xsb_c = critic ? xsb_a + xsb_f : nullptr;
-  float* osb_a = xsb_a + xsb_f * (critic ? 2 : 1);
-  float* osb_c = critic ? osb_a + osb_a_f : nullptr;
 
   if ((rc = kbs_launch_terminate(h, io->state, io->term_codes, io->done, io->success, nullptr, n, st, T))) return rc;
   if (lagged) {
@@ -143,7 +146,6 @@ int rollout_fused_tc(kbs_handle* h, const kbs_rollout_io* io, const uint8_t* don
     KBS_CUDA_TRY(cudaEventRecord(h->ev_pre, st));           // scans done; previous call's readers of the staging buffers too
     KBS_CUDA_TRY(cudaStreamWaitEvent(aux, h->ev_pre, 0));
   }
-  KbsTcRolloutArgs r{};
   r.x_sb_all[0] = xsb_a; r.x_sb_all[1] = xsb_c;
   int n_chunks = 0;
   for (int64_t t0 = 0; t0 < T; t0 += CT, ++n_chunks) {
@@ -172,7 +174,6 @@ int rollout_fused_tc(kbs_handle* h, const kbs_rollout_io* io, const uint8_t* don
   r.done = io->done; r.actor_obs = aobs; r.lpf = io->lpf; r.eps_action = io->eps_action;
   r.qpos = io->state.qpos; r.qvel = io->state.qvel; r.ep = io->episode;
   r.action = io->action; r.log_prob = io->log_prob; r.ctrl = io->ctrl; r.value = io->value;
-  r.ws = ws;
   return kbs_tc_rollout_recurrent(h, r, st);
 }
 
@@ -384,18 +385,20 @@ int kbs_debug_tc_trace_attach(kbs_handle* h, long long* trace_out, int64_t step,
 int kbs_debug_tc_trace(kbs_handle* h, long long* trace_out, int64_t n, void* stream) {
   REQ(h); REQ(trace_out);
   if (n <= 0) return KBS_E_SHAPE;
-  int rc = kbs_scratch_reserve(h, kbs_tc_rollout_ws_floats(h, n) + size_t(n + 128) * h->p.hidden_size * 8);
+  KbsTcRolloutWs ws;
+  int rc = kbs_scratch(h, [&](KbsScratch& s) { ws = kbs_tc_rollout_ws(s, h, n, 1); });
   if (rc) return rc;
-  return kbs_tc_debug_trace(h, trace_out, h->scratch, n, (cudaStream_t)stream);
+  return kbs_tc_debug_trace(h, trace_out, ws, n, (cudaStream_t)stream);
 }
 
 int kbs_debug_tc_gates(kbs_handle* h, int net, int layer, const float* x_rm, const float* h_rm, float* gates_out,
                        int64_t n, void* stream) {
   REQ(h); REQ(x_rm); REQ(h_rm); REQ(gates_out);
   if (n <= 0 || layer < 0 || layer >= h->p.depth) return KBS_E_SHAPE;
-  int rc = kbs_scratch_reserve(h, kbs_tc_scratch_floats(h, n));
+  float* ws;   // x and h as SB operands
+  int rc = kbs_scratch(h, [&](KbsScratch& s) { ws = s.take<float>(2 * size_t(kbs_tc_sb_floats(h, n))); });
   if (rc) return rc;
-  return kbs_tc_debug_gates(h, net, layer, x_rm, h_rm, gates_out, h->scratch, n, (cudaStream_t)stream);
+  return kbs_tc_debug_gates(h, net, layer, x_rm, h_rm, gates_out, ws, n, (cudaStream_t)stream);
 }
 
 int kbs_profile_enable(kbs_handle* h, int on) {
@@ -567,11 +570,10 @@ int kbs_actor_step(kbs_handle* h, const float* obs, int64_t ld, float* carry, fl
   if (rc) return rc;
   AL(obs); AL(carry); AL(lpf); AL(eps); AL(action_in);
   cudaStream_t st = (cudaStream_t)stream;
-  const size_t ts = trunk_scratch_floats(h, n);
-  if ((rc = kbs_scratch_reserve(h, ts + size_t(n) * kOutLd))) return rc;
-  float* out_rm = h->scratch + ts;
-  if ((rc = trunk(h, KBS_NET_ACTOR, obs, ld, carry, done, out_rm, n, st))) return rc;
-  return kbs_launch_actor_head(h, out_rm, kOutLd, obs, ld, lpf, eps, action_in, done, *out, n, st);
+  TrunkWs ws;
+  if ((rc = kbs_scratch(h, [&](KbsScratch& s) { ws = trunk_ws(s, h, n); }))) return rc;
+  if ((rc = trunk(h, KBS_NET_ACTOR, obs, ld, carry, done, ws, n, st))) return rc;
+  return kbs_launch_actor_head(h, ws.out_rm, kOutLd, obs, ld, lpf, eps, action_in, done, *out, n, st);
 }
 
 int kbs_critic_step(kbs_handle* h, const float* obs, int64_t ld, float* carry, const uint8_t* done, float* value,
@@ -581,11 +583,10 @@ int kbs_critic_step(kbs_handle* h, const float* obs, int64_t ld, float* carry, c
   if (rc) return rc;
   AL(obs); AL(carry);
   cudaStream_t st = (cudaStream_t)stream;
-  const size_t ts = trunk_scratch_floats(h, n);
-  if ((rc = kbs_scratch_reserve(h, ts + size_t(n) * kOutLd))) return rc;
-  float* out_rm = h->scratch + ts;
-  if ((rc = trunk(h, KBS_NET_CRITIC, obs, ld, carry, done, out_rm, n, st))) return rc;
-  return kbs_launch_critic_head(h, out_rm, kOutLd, value, n, st);
+  TrunkWs ws;
+  if ((rc = kbs_scratch(h, [&](KbsScratch& s) { ws = trunk_ws(s, h, n); }))) return rc;
+  if ((rc = trunk(h, KBS_NET_CRITIC, obs, ld, carry, done, ws, n, st))) return rc;
+  return kbs_launch_critic_head(h, ws.out_rm, kOutLd, value, n, st);
 }
 
 int kbs_torque(kbs_handle* h, const float* action, const kbs_state_view* s, const kbs_episode_view* ep,
@@ -660,104 +661,99 @@ int kbs_policy_step(kbs_handle* h, const float* joint_angles, const float* joint
       // records [n][d2 * H + 20] are converted straight to / from the kernel's operand layouts: one pass each way
       // instead of flat -> [d2][n][H] -> SB / FB (and back), which was 2/3 of the step's HBM traffic at large n.
       const int carry_w = d2 * H + 20;
-      const size_t ws_f = kbs_tc_rollout_ws_floats(h, n);
-      const size_t xsb_f = size_t(kbs_tc_sb_floats(h, n));
-      const size_t osb_f = size_t(kbs_tc_obs_sb_floats(h, KBS_NET_ACTOR, n, 1));
-      int rc = kbs_scratch_reserve(h, ws_f + xsb_f + osb_f + size_t(KBS_ACTOR_OBS + 20 + 20) * ld + 64);
+      KbsTcRolloutArgs r{};
+      float *xsb, *osb, *obs, *lpf, *act;
+      int rc = kbs_scratch(h, [&](KbsScratch& s) {
+        r.ws = kbs_tc_rollout_ws(s, h, n, 1);
+        xsb = s.take<float>(kbs_tc_sb_floats(h, n));
+        osb = s.take<float>(kbs_tc_obs_sb_floats(h, KBS_NET_ACTOR, n, 1));
+        obs = s.take<float>(size_t(KBS_ACTOR_OBS) * ld);
+        lpf = s.take<float>(size_t(20) * ld);
+        act = s.take<float>(size_t(20) * ld);
+      });
       if (rc) return rc;
-      float* ws = h->scratch;
-      float* xsb = ws + ws_f;
-      float* osb = xsb + xsb_f;
-      float* obs = osb + osb_f;
-      float* lpf = obs + size_t(KBS_ACTOR_OBS) * ld;
-      float* act = lpf + 20 * ld;
       if ((rc = kbs_launch_policy_pack(h, joint_angles, joint_vel, projected_gravity, gyro, command, carry_in, obs, nullptr,
                                        lpf, ld, n, st)))
         return rc;
       const float* obs_soa[2] = {obs, nullptr};
       float* obs_sb[2] = {osb, nullptr};
       float* x_all[2] = {xsb, nullptr};
-      KbsTcRolloutArgs r{};
       if ((rc = kbs_tc_input_proj_all(h, 1, obs_soa, obs_sb, x_all, ld, n, 1, st, nullptr, nullptr, &r))) return rc;
       r.n = n; r.ld = ld; r.T = 1; r.with_critic = false;
       r.carry[0] = const_cast<float*>(carry_in); r.carry_out[0] = carry_out; r.carry_ld = carry_w;
       r.actor_obs = obs; r.lpf = lpf; r.action = act;
-      r.ws = ws;
       if ((rc = kbs_tc_rollout_recurrent(h, r, st))) return rc;
       return kbs_launch_policy_unpack(h, nullptr, lpf, act, carry_out, action_out, ld, n, st);
     }
   }
-  const size_t ts = trunk_scratch_floats(h, n);
-  const size_t need = ts + size_t(n) * kOutLd + size_t(KBS_ACTOR_OBS + 20 + 20) * ld + size_t(d2) * n * H + 64;
-  int rc = kbs_scratch_reserve(h, need);
+  TrunkWs ws;
+  float *obs, *lpf, *mean, *carry;
+  int rc = kbs_scratch(h, [&](KbsScratch& s) {
+    ws = trunk_ws(s, h, n);
+    obs = s.take<float>(size_t(KBS_ACTOR_OBS) * ld);
+    lpf = s.take<float>(size_t(20) * ld);
+    mean = s.take<float>(size_t(20) * ld);
+    carry = s.take<float>(size_t(d2) * n * H);
+  });
   if (rc) return rc;
-  float* out_rm = h->scratch + ts;
-  float* obs = out_rm + size_t(n) * kOutLd;
-  float* lpf = obs + size_t(KBS_ACTOR_OBS) * ld;
-  float* mean = lpf + 20 * ld;
-  float* carry = mean + 20 * ld;
   if ((rc = kbs_launch_policy_pack(h, joint_angles, joint_vel, projected_gravity, gyro, command, carry_in, obs, carry,
                                    lpf, ld, n, st)))
     return rc;
-  if ((rc = trunk(h, KBS_NET_ACTOR, obs, ld, carry, nullptr, out_rm, n, st))) return rc;
+  if ((rc = trunk(h, KBS_NET_ACTOR, obs, ld, carry, nullptr, ws, n, st))) return rc;
   kbs_actor_out o{};
   o.mean = mean;
-  if ((rc = kbs_launch_actor_head(h, out_rm, kOutLd, obs, ld, lpf, nullptr, nullptr, nullptr, o, n, st))) return rc;
+  if ((rc = kbs_launch_actor_head(h, ws.out_rm, kOutLd, obs, ld, lpf, nullptr, nullptr, nullptr, o, n, st))) return rc;
   return kbs_launch_policy_unpack(h, carry, lpf, mean, carry_out, action_out, ld, n, st);
 }
 
-// One pass of _ppo_scan_fn's networks over a stored trajectory (actor [+ critic]); `base` = first float of the handle's
-// scratch this pass may use (the mirror pass of kbs_ppo_variables keeps its intermediate outputs below it).
-static int ppo_variables_pass(kbs_handle* h, const kbs_ppo_io* io, int64_t n, cudaStream_t st, size_t base, size_t* end_out,
-                              bool dry) {
+// Workspace of ppo_variables_pass: the exact-fp32 trunk's, or the tensor-core recurrence's and the input projections' of all T
+// steps for actor [+ critic].
+struct VarsWs { TrunkWs trunk; KbsTcRolloutWs rollout; float* xsb[2]; float* osb[2]; };
+VarsWs vars_ws(KbsScratch& s, const kbs_handle* h, const kbs_ppo_io* io, int64_t n) {
+  VarsWs w{};
+  if (h->p.gemm_path == KBS_GEMM_SIMT_FP32) { w.trunk = trunk_ws(s, h, n); return w; }
+  const int nets = io->critic_obs ? 2 : 1;
+  w.rollout = kbs_tc_rollout_ws(s, h, n, nets);
+  for (int k = 0; k < nets; ++k) w.xsb[k] = s.take<float>(size_t(io->T) * kbs_tc_sb_floats(h, n));
+  for (int k = 0; k < nets; ++k) w.osb[k] = s.take<float>(kbs_tc_obs_sb_floats(h, k, n, io->T));
+  return w;
+}
+
+// One pass of _ppo_scan_fn's networks over a stored trajectory (actor [+ critic]).
+static int ppo_variables_pass(kbs_handle* h, const kbs_ppo_io* io, const VarsWs& ws, int64_t n, cudaStream_t st) {
   int rc;
   const bool critic = io->critic_obs != nullptr;
   const int64_t ld = io->ld, T = io->T;
   if (h->p.gemm_path == KBS_GEMM_SIMT_FP32) {
     // stage-by-stage form (exact-fp32 datapath): T x (actor step, critic step)
-    const size_t ts = trunk_scratch_floats(h, n);
-    if (end_out) *end_out = ts + size_t(n) * kOutLd;          // the trunk's workspace layout starts at the scratch base
-    if (dry) return KBS_OK;
-    float* out_rm = h->scratch + ts;
     for (int64_t t = 0; t < T; ++t) {
       const uint8_t* done_t = io->done + t * ld;
-      if ((rc = trunk(h, KBS_NET_ACTOR, io->actor_obs + t * KBS_ACTOR_OBS * ld, ld, io->actor_carry, done_t, out_rm, n, st)))
+      if ((rc = trunk(h, KBS_NET_ACTOR, io->actor_obs + t * KBS_ACTOR_OBS * ld, ld, io->actor_carry, done_t, ws.trunk, n, st)))
         return rc;
       kbs_actor_out o{};
       o.log_prob = io->log_probs ? io->log_probs + t * ld : nullptr;
       o.entropy = io->entropy ? io->entropy + t * ld : nullptr;
       o.std = io->action_std ? io->action_std + t * KBS_NUM_JOINTS * ld : nullptr;
       o.mean = io->mean ? io->mean + t * KBS_NUM_JOINTS * ld : nullptr;
-      if ((rc = kbs_launch_actor_head(h, out_rm, kOutLd, io->actor_obs + t * KBS_ACTOR_OBS * ld, ld, io->lpf, nullptr,
+      if ((rc = kbs_launch_actor_head(h, ws.trunk.out_rm, kOutLd, io->actor_obs + t * KBS_ACTOR_OBS * ld, ld, io->lpf, nullptr,
                                       io->action + t * KBS_NUM_JOINTS * ld, done_t, o, n, st)))
         return rc;
       if (critic) {
-        if ((rc = trunk(h, KBS_NET_CRITIC, io->critic_obs + t * KBS_CRITIC_OBS * ld, ld, io->critic_carry, done_t, out_rm,
+        if ((rc = trunk(h, KBS_NET_CRITIC, io->critic_obs + t * KBS_CRITIC_OBS * ld, ld, io->critic_carry, done_t, ws.trunk,
                         n, st)))
           return rc;
-        if ((rc = kbs_launch_critic_head(h, out_rm, kOutLd, io->values + t * ld, n, st))) return rc;
+        if ((rc = kbs_launch_critic_head(h, ws.trunk.out_rm, kOutLd, io->values + t * ld, n, st))) return rc;
       }
     }
     return KBS_OK;
   }
   // tensor-core form: input projections of all T steps (critic: one launch; actor: folded into layer 0), then the persistent
   // recurrence kernel with the stored actions (log-prob / entropy / std / mean of the stored action instead of sampling)
-  const size_t sbf = size_t(kbs_tc_sb_floats(h, n));
-  const size_t ws_f = kbs_tc_rollout_ws_floats(h, n), xsb_f = size_t(T) * sbf;
-  const size_t osb_a_f = size_t(kbs_tc_obs_sb_floats(h, KBS_NET_ACTOR, n, T));
-  const size_t osb_c_f = critic ? size_t(kbs_tc_obs_sb_floats(h, KBS_NET_CRITIC, n, T)) : 0;
-  if (end_out) *end_out = base + ws_f + xsb_f * (critic ? 2 : 1) + osb_a_f + osb_c_f + 64;
-  if (dry) return KBS_OK;
-  float* ws = h->scratch + base;
-  float* xsb_a = ws + ws_f;
-  float* xsb_c = critic ? xsb_a + xsb_f : nullptr;
-  float* osb_a = xsb_a + xsb_f * (critic ? 2 : 1);
-  float* osb_c = critic ? osb_a + osb_a_f : nullptr;
   KbsTcRolloutArgs r{};
   {
     const float* obs_soa[2] = {io->actor_obs, io->critic_obs};
-    float* obs_sb[2] = {osb_a, osb_c};
-    float* xsb[2] = {xsb_a, xsb_c};
+    float* obs_sb[2] = {ws.osb[0], critic ? ws.osb[1] : nullptr};
+    float* xsb[2] = {ws.xsb[0], critic ? ws.xsb[1] : nullptr};
     if ((rc = kbs_tc_input_proj_all(h, critic ? 2 : 1, obs_soa, obs_sb, xsb, ld, n, T, st, nullptr, nullptr, &r))) return rc;
   }
   r.n = n; r.ld = ld; r.T = T; r.with_critic = critic;
@@ -766,7 +762,7 @@ static int ppo_variables_pass(kbs_handle* h, const kbs_ppo_io* io, int64_t n, cu
   r.action_in = io->action; r.log_prob = io->log_probs; r.entropy = io->entropy; r.action_std = io->action_std;
   r.mean = io->mean;
   r.value = io->values;
-  r.ws = ws;
+  r.ws = ws.rollout;
   return kbs_tc_rollout_recurrent(h, r, st);
 }
 
@@ -792,28 +788,31 @@ int kbs_ppo_variables(kbs_handle* h, const kbs_ppo_io* io, int64_t n, void* stre
   const int64_t ld = io->ld, T = io->T;
   const bool tc = h->p.gemm_path != KBS_GEMM_SIMT_FP32;
   if (tc && io->mean && !kbs_tc_persistent_available(h, n, T, critic ? 2 : 1)) return KBS_E_SHAPE;
-  // scratch: [mirror intermediates: mean, mean_m [T][20][ld], value_m, lp_m, ent_m [T][ld]] | pass workspace.  The exact-fp32
-  // trunk addresses its workspace from the scratch base, so there the intermediates sit behind it instead.
-  const size_t mir_f = mirror ? (2 * size_t(T) * KBS_NUM_JOINTS * ld + 3 * size_t(T) * ld + 255) / 256 * 256 : 0;
-  size_t pass_end = 0;
-  if ((rc = ppo_variables_pass(h, io, n, st, tc ? mir_f : 0, &pass_end, true))) return rc;
-  if ((rc = kbs_scratch_reserve(h, pass_end + (tc ? 0 : mir_f) + 64))) return rc;
-  float* mir = mirror ? (tc ? h->scratch : h->scratch + pass_end) : nullptr;
+  // the mirror pass's intermediates: mean, mean_m [T][20][ld], value_m, lp_m, ent_m [T][ld]; then both passes' workspace
+  float *mean = nullptr, *mean_m = nullptr, *value_m = nullptr, *lp_m = nullptr, *ent_m = nullptr;
+  VarsWs ws;
+  rc = kbs_scratch(h, [&](KbsScratch& s) {
+    if (mirror) {
+      mean = s.take<float>(size_t(T) * KBS_NUM_JOINTS * ld);
+      mean_m = s.take<float>(size_t(T) * KBS_NUM_JOINTS * ld);
+      value_m = s.take<float>(size_t(T) * ld);
+      lp_m = s.take<float>(size_t(T) * ld);
+      ent_m = s.take<float>(size_t(T) * ld);
+    }
+    ws = vars_ws(s, h, io, n);
+  });
+  if (rc) return rc;
   kbs_ppo_io a = *io;
-  if (mirror && !a.mean) a.mean = mir;
-  if ((rc = ppo_variables_pass(h, &a, n, st, tc ? mir_f : 0, nullptr, false))) return rc;
+  if (mirror && !a.mean) a.mean = mean;
+  if ((rc = ppo_variables_pass(h, &a, ws, n, st))) return rc;
   if (!mirror) return KBS_OK;
   // the mirrored passes (train.py:1462-1481): same networks, mirrored observations, their own carries
-  float* mean_m = mir + size_t(T) * KBS_NUM_JOINTS * ld;
-  float* value_m = mean_m + size_t(T) * KBS_NUM_JOINTS * ld;
-  float* lp_m = value_m + size_t(T) * ld;
-  float* ent_m = lp_m + size_t(T) * ld;
   kbs_ppo_io m = *io;
   m.actor_obs = io->actor_obs_mirror; m.critic_obs = io->critic_obs_mirror;
   m.actor_carry = io->actor_mirror_carry; m.critic_carry = io->critic_mirror_carry; m.lpf = io->lpf_mirror;
   m.log_probs = lp_m; m.entropy = ent_m; m.values = io->critic_obs_mirror ? value_m : nullptr; m.action_std = nullptr;
   m.mean = mean_m;
-  if ((rc = ppo_variables_pass(h, &m, n, st, tc ? mir_f : 0, nullptr, false))) return rc;
+  if ((rc = ppo_variables_pass(h, &m, ws, n, st))) return rc;
   return kbs_launch_mirror_loss(h, a.mean, mean_m, io->values, value_m, io->action_mirror_loss,
                                 io->critic_obs_mirror ? io->value_mirror_loss : nullptr, io->actor_mirror_loss_scale,
                                 io->critic_mirror_loss_scale, T, ld, n, st);
@@ -913,12 +912,14 @@ int kbs_rollout_record(kbs_handle* h, const kbs_rollout_io* io, const struct kbs
   cudaStream_t st = (cudaStream_t)stream;
   if (h->p.gemm_path != KBS_GEMM_SIMT_FP32) return rollout_fused_tc(h, io, done_prev, critic_obs, n, st);
   const int64_t ld = io->state.ld;
-  const size_t ts = trunk_scratch_floats(h, n);
-  const size_t need = ts + size_t(n) * kOutLd + size_t(KBS_ACTOR_OBS + KBS_CRITIC_OBS) * ld + 64;
-  if ((rc = kbs_scratch_reserve(h, need))) return rc;
-  float* out_rm = h->scratch + ts;
-  float* aobs_scratch = out_rm + size_t(n) * kOutLd;
-  float* cobs = aobs_scratch + size_t(KBS_ACTOR_OBS) * ld;
+  TrunkWs ws;
+  float *aobs_scratch, *cobs;
+  rc = kbs_scratch(h, [&](KbsScratch& s) {
+    ws = trunk_ws(s, h, n);
+    aobs_scratch = s.take<float>(size_t(KBS_ACTOR_OBS) * ld);
+    cobs = s.take<float>(size_t(KBS_CRITIC_OBS) * ld);
+  });
+  if (rc) return rc;
 
   for (int64_t t = 0; t < io->T; ++t) {
     const kbs_state_view s = state_at(io->state, t);
@@ -935,18 +936,18 @@ int kbs_rollout_record(kbs_handle* h, const kbs_rollout_io* io, const struct kbs
     if ((rc = kbs_launch_observations(h, s, &nz, &io->episode, cmd_t, io->pg_carry, t > 0 ? done_t - ld : done_prev,
                                       nullptr, aobs, cobs_t, n, st)))
       return rc;
-    if ((rc = trunk(h, KBS_NET_ACTOR, aobs, ld, io->actor_carry, done_t, out_rm, n, st))) return rc;
+    if ((rc = trunk(h, KBS_NET_ACTOR, aobs, ld, io->actor_carry, done_t, ws, n, st))) return rc;
     kbs_actor_out o{};
     o.action = io->action + t * KBS_NUM_JOINTS * ld;
     o.log_prob = io->log_prob ? io->log_prob + t * ld : nullptr;
-    if ((rc = kbs_launch_actor_head(h, out_rm, kOutLd, aobs, ld, io->lpf,
+    if ((rc = kbs_launch_actor_head(h, ws.out_rm, kOutLd, aobs, ld, io->lpf,
                                     io->eps_action ? io->eps_action + t * KBS_NUM_JOINTS * ld : nullptr, nullptr, done_t,
                                     o, n, st)))
       return rc;
     if ((rc = kbs_launch_torque(h, o.action, s, &io->episode, io->ctrl + t * KBS_NUM_JOINTS * ld, n, st))) return rc;
     if (io->value) {
-      if ((rc = trunk(h, KBS_NET_CRITIC, cobs_t, ld, io->critic_carry, done_t, out_rm, n, st))) return rc;
-      if ((rc = kbs_launch_critic_head(h, out_rm, kOutLd, io->value + t * ld, n, st))) return rc;
+      if ((rc = trunk(h, KBS_NET_CRITIC, cobs_t, ld, io->critic_carry, done_t, ws, n, st))) return rc;
+      if ((rc = kbs_launch_critic_head(h, ws.out_rm, kOutLd, io->value + t * ld, n, st))) return rc;
     }
     if ((rc = kbs_launch_command(h, cmd_t, cmd_n, io->u_switch + t * ld, io->cmd_mode + t * ld,
                                  io->cmd_u6 + t * 6 * ld, io->cmd_u_arms + t * 10 * ld, done_t, ld, n, st)))

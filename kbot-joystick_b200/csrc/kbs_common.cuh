@@ -112,8 +112,30 @@ int kbs_side_stream_init(kbs_handle* h);   // kbs_api.cu: lazily creates side_st
 int kbs_status_init(kbs_handle* h);
 int kbs_status_publish(kbs_handle* h, cudaStream_t st);
 int kbs_enter(kbs_handle* h);
-// scratch management (kbs_api.cu)
+// scratch management (kbs_api.cu): grows the handle's allocation (KBS_E_STATE while kbs_scratch_lock holds it)
 int kbs_scratch_reserve(kbs_handle* h, size_t floats);
+
+// Bump allocator over the handle's scratch.  An entry point states its layout once, as code that only takes pieces (no
+// launches, no branches on which pass it is in); kbs_scratch runs it with a null base to add up the total, grows the
+// scratch to that, and runs it again on the real base to hand out the pointers.  Every piece is rounded up to 256 bytes.
+struct KbsScratch {
+  char* base;
+  size_t bytes = 0;
+  template <class T> T* take(size_t count) {
+    T* p = base ? reinterpret_cast<T*>(base + bytes) : nullptr;
+    bytes += (count * sizeof(T) + 255) / 256 * 256;
+    return p;
+  }
+};
+template <class Layout>
+int kbs_scratch(kbs_handle* h, Layout&& layout) {
+  KbsScratch size{nullptr};
+  layout(size);
+  if (const int rc = kbs_scratch_reserve(h, size.bytes / sizeof(float))) return rc;
+  KbsScratch s{reinterpret_cast<char*>(h->scratch)};
+  layout(s);
+  return KBS_OK;
+}
 
 // ---- stage launchers implemented across the translation units -------------------------------------
 // kbs_elementwise.cu
@@ -171,9 +193,10 @@ int kbs_launch_shuffle_minibatches(kbs_handle* h, const int32_t* perm, const kbs
 
 // kbs_net_simt.cu : fp32 FFMA datapath
 int kbs_simt_pack(kbs_handle* h, int net, const kbs_net_weights* w, cudaStream_t st);
+struct KbsSimtTrunkWs { float* x; float* gates; float* hbuf; };   // [n][H], [n][4H], [n][H]
+KbsSimtTrunkWs kbs_simt_trunk_ws(KbsScratch& s, const kbs_handle* h, int64_t n);
 int kbs_simt_trunk(kbs_handle* h, int net, const float* obs_soa, int64_t ld, float* carry, const uint8_t* done,
-                   float* out_rowmajor /*[n][nout_pad]*/, int64_t n, cudaStream_t st);
-size_t kbs_simt_scratch_floats(const kbs_handle* h, int64_t n);
+                   float* out_rowmajor /*[n][nout_pad]*/, const KbsSimtTrunkWs& ws, int64_t n, cudaStream_t st);
 
 int kbs_simt_gemm_nt(kbs_handle* h, const float* A, int64_t lda, const float* W, int ldw, const float* bias, float* C, int ldc,
                      int64_t M, int Npad, int K, int accumulate, cudaStream_t st, int batch = 1, int64_t a_ts = 0, int64_t c_ts = 0);
@@ -184,9 +207,15 @@ int kbs_simt_out_proj(kbs_handle* h, int net, const float* h_rm, float* out_rm, 
 
 // kbs_net_tc.cu : tcgen05 3xTF32 datapath
 int kbs_tc_pack(kbs_handle* h, int net, cudaStream_t st);
-size_t kbs_tc_scratch_floats(const kbs_handle* h, int64_t n);
+// workspace of kbs_tc_lstm_stack: x_sb ping/pong [2], h_sb [depth][2 (in, out)] x act SB; fb [depth][c, h] x np*H
+struct KbsTcStackWs { char* x_sb; char* h_sb; float* fb; };
+KbsTcStackWs kbs_tc_stack_ws(KbsScratch& s, const kbs_handle* h, int64_t n);
 int kbs_tc_lstm_stack(kbs_handle* h, int net, const float* x_rm, float* carry, const uint8_t* done, float* out_h_rm,
-                      float* ws, int64_t n, bool carry_sb_valid, cudaStream_t st);
+                      const KbsTcStackWs& ws, int64_t n, bool carry_sb_valid, cudaStream_t st);
+// workspace of kbs_tc_rollout_recurrent, per net: hsb, xmid [depth][2] x act SB; h2rm [2 parity][n][H]; fb [depth][c, h] x np*H;
+// flags [depth + 1][panels]
+struct KbsTcRolloutWs { char* hsb[2]; char* xmid[2]; float* h2rm[2]; float* fb[2]; unsigned int* flags[2]; };
+KbsTcRolloutWs kbs_tc_rollout_ws(KbsScratch& s, const kbs_handle* h, int64_t n, int nets);
 // recurrent phase of the fused rollout (kbs_net_tc.cu)
 struct KbsTcRolloutArgs {
   int64_t n, ld, T;
@@ -217,11 +246,10 @@ struct KbsTcRolloutArgs {
   // save_g [T][depth][4] x np*H, sraw [T][20][ld]; carry[] may be nullptr (zeros); the final carries are not written back.
   int save;
   char* xmid_hist[2]; char* hsb_hist[2]; float* c_hist[2]; float* save_g[2]; float* sraw;
-  float* ws;                  // kbs_tc_rollout_ws_floats
+  KbsTcRolloutWs ws;          // kbs_tc_rollout_ws for (with_critic ? 2 : 1) nets
   int64_t chunk_len;          // > 0: before step t with t % chunk_len == 0, wait for chunk_events[t / chunk_len]
   cudaEvent_t* chunk_events;  //      (the input projections of that chunk of steps, produced on another stream)
 };
-size_t kbs_tc_rollout_ws_floats(const kbs_handle* h, int64_t n);
 int64_t kbs_tc_sb_floats(const kbs_handle* h, int64_t n);
 int64_t kbs_tc_obs_sb_floats(const kbs_handle* h, int net, int64_t n, int64_t T);
 // cinert / cvel != nullptr: the critic's privileged dump (features 80..447) is read from the recorded state
@@ -233,7 +261,7 @@ bool kbs_tc_fused_input(const kbs_handle* h, int net, int64_t n, int64_t T, int 
 int kbs_tc_rollout_recurrent(kbs_handle* h, const KbsTcRolloutArgs& r, cudaStream_t st);
 // true when kbs_tc_rollout_recurrent will take the persistent kernel for this shape (all T steps in one launch)
 bool kbs_tc_persistent_available(const kbs_handle* h, int64_t n, int64_t T, int nets);
-int kbs_tc_debug_trace(kbs_handle* h, long long* trace_out, float* ws, int64_t n, cudaStream_t st);
+int kbs_tc_debug_trace(kbs_handle* h, long long* trace_out, const KbsTcRolloutWs& ws, int64_t n, cudaStream_t st);
 // tensor-core GEMMs of the PPO update
 int kbs_tc_gates_fwd(kbs_handle* h, int net, int layer, const void* x_sb, const void* h_sb, float* gates_out, int64_t n,
                      cudaStream_t st);

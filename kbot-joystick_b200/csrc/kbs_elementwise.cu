@@ -1420,10 +1420,10 @@ static int ppo_loss_blocks(const kbs_handle* h, const kbs_ppo_loss_io& io) {
 }
 
 int kbs_launch_ppo_loss(kbs_handle* h, const kbs_ppo_loss_params& L, const kbs_ppo_loss_io& io, int64_t n, cudaStream_t st) {
-  const int blocks = ppo_loss_blocks(h, io);
-  int rc = kbs_scratch_reserve(h, size_t(blocks) * 8 + 16);
+  double* partials;
+  const int rc = kbs_scratch(h, [&](KbsScratch& s) { partials = s.take<double>(size_t(ppo_loss_blocks(h, io)) * 4); });
   if (rc) return rc;
-  return kbs_launch_ppo_loss_at(h, L, io, n, reinterpret_cast<double*>(h->scratch), st);
+  return kbs_launch_ppo_loss_at(h, L, io, n, partials, st);
 }
 
 // partials: >= 4 * 4 * num_sms doubles of caller-provided device scratch
@@ -1568,12 +1568,12 @@ int kbs_launch_terminate(kbs_handle* h, const kbs_state_view& s, int32_t* codes,
 int kbs_launch_rewards(kbs_handle* h, const kbs_traj_view& tr, const kbs_reward_carry& carry, float* total,
                        float* components, int64_t n, cudaStream_t st) {
   const int64_t ld = tr.state.ld, T = tr.T;
-  // scratch: is_rot [ld] + flags [T][ld] bytes
-  const size_t bytes = size_t(ld) * size_t(T + 1);
-  int rc = kbs_scratch_reserve(h, (bytes + 3) / 4 + 4);
+  uint8_t *is_rot, *flags;   // [ld], [T][ld]
+  const int rc = kbs_scratch(h, [&](KbsScratch& s) {
+    is_rot = s.take<uint8_t>(size_t(ld));
+    flags = s.take<uint8_t>(size_t(T) * ld);
+  });
   if (rc) return rc;
-  uint8_t* is_rot = reinterpret_cast<uint8_t*>(h->scratch);
-  uint8_t* flags = is_rot + ld;
   KBS_LAUNCH(h, KBS_K_REWARD_ROT, st, (reward_rot_kernel<<<groups4(n), kThreads, 0, st>>>(tr.command, is_rot, T, ld, n)));
   dim3 grid(unsigned((n + kThreads - 1) / kThreads), unsigned(T));
   KBS_LAUNCH(h, KBS_K_REWARD_TERMS, st,

@@ -357,20 +357,18 @@ int kbs_simt_gemm_tn(kbs_handle* h, const float* A, int lda, const float* B, int
   return KBS_OK;
 }
 
-size_t kbs_simt_scratch_floats(const kbs_handle* h, int64_t n) {
-  const size_t H = size_t(h->p.hidden_size);
-  return size_t(n) * (H + 4 * H + H) + 64;
+KbsSimtTrunkWs kbs_simt_trunk_ws(KbsScratch& s, const kbs_handle* h, int64_t n) {
+  const size_t nH = size_t(n) * h->p.hidden_size;
+  return {s.take<float>(nH), s.take<float>(4 * nH), s.take<float>(nH)};   // braced list: taken left to right
 }
 
 // out_rowmajor: [n][nout_pad = 64]
 int kbs_simt_trunk(kbs_handle* h, int net, const float* obs_soa, int64_t ld, float* carry, const uint8_t* done,
-                   float* out_rm, int64_t n, cudaStream_t st) {
+                   float* out_rm, const KbsSimtTrunkWs& ws, int64_t n, cudaStream_t st) {
   const KbsNet& N = h->net[net];
   if (!N.packed) return KBS_E_STATE;
   const int H = h->p.hidden_size;
-  float* x = h->scratch;
-  float* gates = x + size_t(n) * H;
-  float* hbuf = gates + size_t(n) * 4 * H;
+  float* x = ws.x; float* gates = ws.gates; float* hbuf = ws.hbuf;
   const unsigned mb = unsigned((n + BM - 1) / BM);
   KBS_LAUNCH(h, KBS_K_GEMM_SIMT, st,
              (gemm_nt_kernel<true><<<dim3(mb, H / BN), 256, 0, st>>>(obs_soa, ld, N.w_in, N.kin_pad, N.b_in, x, H, n,

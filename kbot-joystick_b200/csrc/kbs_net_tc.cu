@@ -3186,11 +3186,9 @@ static int pack_rows(kbs_handle* h, const float* src, int64_t ld, char* sb, int6
 // bytes of one [n][H] SB activation buffer
 static size_t act_sb_bytes(const kbs_handle* h, int64_t n) { return kbs_sb_bytes_kind(tc_kind(h), pad_rows(n), h->p.hidden_size); }
 
-// scratch (floats) of the per-step TC trunk: x_sb ping/pong + h_sb in/out per layer + x row-major + hbuf row-major
-size_t kbs_tc_scratch_floats(const kbs_handle* h, int64_t n) {
-  const size_t H = size_t(h->p.hidden_size);
-  return act_sb_bytes(h, n) / 4 * (2 + 2 * size_t(h->p.depth)) + 2 * size_t(h->p.depth) * size_t(pad_rows(n)) * H +
-         2 * size_t(n) * H + 256;
+KbsTcStackWs kbs_tc_stack_ws(KbsScratch& s, const kbs_handle* h, int64_t n) {
+  const size_t sbb = act_sb_bytes(h, n), depth = size_t(h->p.depth);
+  return {s.take<char>(2 * sbb), s.take<char>(2 * depth * sbb), s.take<float>(2 * depth * size_t(pad_rows(n)) * h->p.hidden_size)};
 }
 
 static int fb_convert(kbs_handle* h, float* rm, float* fb, int64_t n, int64_t np, int H, int to_fb, cudaStream_t st) {
@@ -3224,19 +3222,18 @@ static void fill_lstm_args(const kbs_handle* h, int net, int l, LayerArgs& a) {
 }
 
 // Runs depth LSTM layers on the tensor cores.  x_rm: [n][H] row-major layer-0 input (input_proj output);
-// carry: ABI layout [depth][2][n][H]; out_h_rm: [n][H] row-major un-reset top-layer output.  ws: kbs_tc_scratch_floats.
+// carry: ABI layout [depth][2][n][H]; out_h_rm: [n][H] row-major un-reset top-layer output.
 int kbs_tc_lstm_stack(kbs_handle* h, int net, const float* x_rm, float* carry, const uint8_t* done, float* out_h_rm,
-                      float* ws, int64_t n, bool carry_sb_valid, cudaStream_t st) {
+                      const KbsTcStackWs& ws, int64_t n, bool carry_sb_valid, cudaStream_t st) {
   const KbsNet& N = h->net[net];
   if (!N.packed || !N.tc_image) return KBS_E_STATE;
   const int H = h->p.hidden_size, depth = h->p.depth;
   const int64_t np = pad_rows(n);
   const size_t sbb = act_sb_bytes(h, n);
-  char* wsb = reinterpret_cast<char*>(ws);
-  char* x_sb[2] = {wsb, wsb + sbb};
-  char* h_sb = wsb + 2 * sbb;   // [depth][2 (in, out)]: the column-tile CTAs of a panel all read h_{t-1} while their
+  char* x_sb[2] = {ws.x_sb, ws.x_sb + sbb};
+  char* h_sb = ws.h_sb;         // [depth][2 (in, out)]: the column-tile CTAs of a panel all read h_{t-1} while their
                                 // epilogues write h_t, so in and out must be distinct buffers
-  float* fb = reinterpret_cast<float*>(h_sb + sbb * 2 * depth);   // [depth][c, h] x np*H: state in the kernel's FB layout
+  float* fb = ws.fb;            // [depth][c, h] x np*H: state in the kernel's FB layout
   const size_t fbf = size_t(np) * H;
   pack_rows(h, x_rm, H, x_sb[0], n, np, H, st);
   for (int l = 0; l < depth; ++l)
@@ -3941,15 +3938,18 @@ size_t kbs_tc_rows_sb_bytes(const kbs_handle* h, int64_t n, int K) { return kbs_
 int kbs_tc_kind_of(const kbs_handle* h) { return tc_kind(h); }
 
 // ---- fused rollout: tensor-core input projection of all T steps + the recurrent phase --------------------------------
-// Workspace per net: h_sb [depth][2 parity] | x_mid_sb [2] | h2_rm [n][H] (floats)
-static size_t rollout_flag_bytes(const kbs_handle* h, int64_t n) {
-  return (size_t(h->p.depth + 1) * size_t(pad_rows(n) / kPanelRows) * 4 + 255) / 256 * 256;
+KbsTcRolloutWs kbs_tc_rollout_ws(KbsScratch& s, const kbs_handle* h, int64_t n, int nets) {
+  const size_t sbb = act_sb_bytes(h, n), depth = size_t(h->p.depth), H = size_t(h->p.hidden_size), np = size_t(pad_rows(n));
+  KbsTcRolloutWs w{};
+  for (int k = 0; k < nets; ++k) {
+    w.hsb[k] = s.take<char>(2 * depth * sbb);
+    w.xmid[k] = s.take<char>(2 * depth * sbb);    // the per-step launch path uses the first two
+    w.h2rm[k] = s.take<float>(2 * size_t(n) * H);  // top-layer output (per-step path)
+    w.fb[k] = s.take<float>(2 * depth * np * H);
+    w.flags[k] = s.take<unsigned int>((depth + 1) * (np / kPanelRows));
+  }
+  return w;
 }
-static size_t rollout_ws_per_net_bytes(const kbs_handle* h, int64_t n) {
-  return act_sb_bytes(h, n) * (4 * size_t(h->p.depth)) + 2 * size_t(n) * h->p.hidden_size * 4 +
-         2 * size_t(h->p.depth) * size_t(pad_rows(n)) * h->p.hidden_size * 4 + rollout_flag_bytes(h, n) + 256;
-}
-size_t kbs_tc_rollout_ws_floats(const kbs_handle* h, int64_t n) { return 2 * rollout_ws_per_net_bytes(h, n) / 4; }
 int64_t kbs_tc_sb_floats(const kbs_handle* h, int64_t n) { return int64_t(act_sb_bytes(h, n) / 4); }
 // floats of the SB observation staging buffer of `net` for T steps
 int64_t kbs_tc_obs_sb_floats(const kbs_handle* h, int net, int64_t n, int64_t T) {
@@ -4075,17 +4075,10 @@ int kbs_tc_rollout_recurrent(kbs_handle* h, const KbsTcRolloutArgs& r, cudaStrea
     h->head_attr_set = true;
   }
   const int64_t n = r.n, ld = r.ld, np = pad_rows(n);
-  const size_t sbb = act_sb_bytes(h, n), per_net = rollout_ws_per_net_bytes(h, n);
-  char* hsb[2]; char* xmid[2]; float* h2rm[2]; float* fb[2]; unsigned int* flags[2];
+  const size_t sbb = act_sb_bytes(h, n);
+  char* hsb[2] = {r.ws.hsb[0], r.ws.hsb[1]}; char* xmid[2] = {r.ws.xmid[0], r.ws.xmid[1]};
+  float* const* h2rm = r.ws.h2rm; float* const* fb = r.ws.fb; unsigned int* const* flags = r.ws.flags;
   const size_t fbf = size_t(np) * H;
-  for (int k = 0; k < nets; ++k) {
-    char* base = reinterpret_cast<char*>(r.ws) + per_net * k;
-    hsb[k] = base;                                   // [depth][2] x sbb
-    xmid[k] = base + sbb * 2 * depth;                // [depth][2] x sbb (the per-step launch path uses the first two)
-    h2rm[k] = reinterpret_cast<float*>(xmid[k] + 2 * depth * sbb);   // [2 parity] x n*H: top-layer output (per-step path)
-    fb[k] = h2rm[k] + 2 * size_t(n) * H;             // [depth][c, h] x np*H, FB layout
-    flags[k] = reinterpret_cast<unsigned int*>(fb[k] + 2 * size_t(depth) * fbf);
-  }
   const char* legacy_env = getenv("KBS_TC_PER_STEP");          // A/B and cross-check against the per-step launches
   const int legacy = (legacy_env && !r.save) ? atoi(legacy_env) : 0;
   const bool persistent = !legacy && kbs_tc_persistent_available(h, n, r.T, nets);
@@ -4141,7 +4134,7 @@ int kbs_tc_rollout_recurrent(kbs_handle* h, const KbsTcRolloutArgs& r, cudaStrea
       for (int l = 0; l < depth; ++l) { N.w_sb[l] = layer_w_p(h, k, l); N.bias_t[l] = layer_bias_p(h, k, l); }
       if (r.x_is_obs[k]) { N.w_sb[0] = fused_w(h, k); N.bias_t[0] = fused_bias(h, k); }
       N.w_head = head_w(h, k); N.bias_head = head_bias(h, k);
-      KBS_CUDA_TRY(cudaMemsetAsync(flags[k], 0, rollout_flag_bytes(h, n), st));
+      KBS_CUDA_TRY(cudaMemsetAsync(flags[k], 0, size_t(depth + 1) * panels * sizeof(unsigned int), st));
     }
     a.nets = nets; a.depth = depth; a.H = H; a.panels = panels; a.tiles = tiles;
     a.n = n; a.ld = ld; a.T = r.T; a.sbb = sbb;
@@ -4287,21 +4280,22 @@ int kbs_tc_rollout_recurrent(kbs_handle* h, const KbsTcRolloutArgs& r, cudaStrea
 // Debug: one LSTM-mode layer launch for both nets on scratch data with per-CTA clock64 stamps.
 // trace_out (device) [2 * tiles * panels][8]: start, setup done, first stage landed, MMAs issued, accumulators ready,
 // epilogue done, smid, unused.
-int kbs_tc_debug_trace(kbs_handle* h, long long* trace_out, float* ws, int64_t n, cudaStream_t st) {
+// Both nets run on zeroed layer-0 buffers of the rollout workspace of net 0.
+int kbs_tc_debug_trace(kbs_handle* h, long long* trace_out, const KbsTcRolloutWs& ws, int64_t n, cudaStream_t st) {
   const int H = h->p.hidden_size;
   for (int k = 0; k < 2; ++k)
     if (!h->net[k].packed || !h->net[k].tc_image) return KBS_E_STATE;
   const int64_t np = pad_rows(n);
   const size_t sbb = act_sb_bytes(h, n);
-  char* wsb = reinterpret_cast<char*>(ws);
-  KBS_CUDA_TRY(cudaMemsetAsync(wsb, 0, sbb * 4 + size_t(np) * H * 4 * 3, st));
-  float* rm = reinterpret_cast<float*>(wsb + sbb * 4);
+  KBS_CUDA_TRY(cudaMemsetAsync(ws.hsb[0], 0, sbb * 2, st));
+  KBS_CUDA_TRY(cudaMemsetAsync(ws.xmid[0], 0, sbb * 2, st));
+  KBS_CUDA_TRY(cudaMemsetAsync(ws.fb[0], 0, size_t(np) * H * 4 * 2, st));
   LayerArgs2 a2{};
   for (int k = 0; k < 2; ++k) {
     LayerArgs& a = a2.net[k];
     fill_lstm_args(h, k, 0, a);
-    a.x_sb = wsb; a.h_sb_in = wsb + sbb; a.h_sb_out = wsb + 2 * sbb; a.x_next_sb = wsb + 3 * sbb;
-    a.c = rm; a.h_carry = rm + size_t(np) * H; a.h_next_rm = nullptr; a.done = nullptr; a.n = n;
+    a.x_sb = ws.xmid[0]; a.h_sb_in = ws.hsb[0]; a.h_sb_out = ws.hsb[0] + sbb; a.x_next_sb = ws.xmid[0] + sbb;
+    a.c = ws.fb[0]; a.h_carry = ws.fb[0] + size_t(np) * H; a.h_next_rm = nullptr; a.done = nullptr; a.n = n;
     a.trace = trace_out;
     a.panels = int(np / kPanelRows);
   }

@@ -681,25 +681,6 @@ struct NetWork {      // per-net workspace (floats), carved from the handle's sc
   char* tn_a; char* tn_b; float* tn_partial; float* tn_zero; char* tn_ones;
 };
 
-size_t net_work_floats(const kbs_handle* h, int net, int64_t T, int64_t n, bool tc) {
-  const size_t H = size_t(h->p.hidden_size), rows = size_t(T) * size_t(n);
-  const size_t kp = size_t(round_up_i(h->net[net].num_in, 64));
-  const size_t depth = size_t(h->p.depth);
-  size_t f = rows * kp + rows * H * 2 /*x0, dh_top*/ + rows * 2 * H /*dxh0*/ + rows * 64 * 2 + depth * size_t(n) * 2 * H;
-  f += depth * (rows * 4 * H * 2 + rows * H * 4 + 2 * 4 * H * H + 256);
-  f += 64 * H;
-  if (tc) {
-    const size_t sbH = kbs_tc_rows_sb_bytes(h, n, int(H)) / 4, sb4H = kbs_tc_rows_sb_bytes(h, n, int(4 * H)) / 4;
-    f += size_t(T) * sbH * (1 + 2 * depth) + sb4H + 1024;
-    const KbsTnPlan plan = kbs_tc_tn_plan(h, int64_t(rows));
-    const size_t m_panels = 4 * H / 128, b_tiles = (kp > 2 * H ? kp : 2 * H) / 128 + 1;
-    f += (m_panels + b_tiles) * plan.col_bytes / 4 + size_t(plan.ksplit) * m_panels * 128 * (b_tiles * 128) + 1024 + 4096 + 4096;
-  }
-  return f + 4096;
-}
-
-float* carve(float*& p, size_t floats) { float* r = p; p += (floats + 63) / 64 * 64; return r; }
-
 template <int KIND>
 int run_net_k(kbs_handle* h, int net, const kbs_ppo_batch& b, const float* carry0, NetWork& w, float* gates_pre, float* dc_rec,
               float* part, int splits, int64_t n, cudaStream_t st, bool backward, const kbs_net_grads* g, bool tc) {
@@ -902,73 +883,55 @@ struct PersistWork {
   char* tna_dG[KBS_MAX_DEPTH];      // A operands: dG of each layer re-packed (by the backward kernel's transposer CTAs): 4 H / 128 panels
 };
 
-size_t persist_work_floats(const kbs_handle* h, int net, int64_t T, int64_t n) {
-  const size_t H = size_t(h->p.hidden_size), depth = size_t(h->p.depth);
-  const size_t np = size_t((n + 127) / 128 * 128), npH = np * H, rows = size_t(T) * size_t(n);
-  const size_t sbf = kbs_tc_rows_sb_bytes(h, n, int(H)) / 4, sb4f = kbs_tc_rows_sb_bytes(h, n, int(4 * H)) / 4;
-  const KbsTnPlan plan = kbs_tc_tn_plan(h, int64_t(T) * int64_t(np));
-  const size_t kpp = size_t(round_up_i(h->net[net].num_in + 1, 128));
-  const size_t m_panels = 4 * H / 128, b_tiles = (kpp > 2 * H ? kpp : 2 * H) / 128 + 1;
-  size_t f = size_t(T) * sbf /*x_sb*/ + depth * size_t(T) * sbf /*xmid*/ + depth * size_t(T + 1) * sbf /*hsb*/ +
-             depth * size_t(T + 1) * npH /*c_hist*/ + size_t(T) * depth * 4 * npH /*save_g*/ + depth * size_t(T + 1) * sb4f /*dG*/ +
-             depth * size_t(T) * npH /*dx*/ + size_t(T) * sbf /*dx0*/ + depth * npH /*dc*/ + rows * H /*dh_top*/ + rows * 64 /*dout*/ +
-             64 * H + kbs_tc_bptt_flag_bytes(h, n) / 4 + rows * H /*h_top_rm*/ + rows * 64 /*out*/ + kbs_tc_fwd_save_flag_bytes(h, n) / 4;
-  f += m_panels * plan.col_bytes / 4 + size_t(plan.ksplit) * m_panels * 128 * (b_tiles * 128) + 1024 + 4096;
-  f += (depth * (2 * H / 128) + H / 128 + kpp / 128 + depth * (4 * H / 128)) * plan.col_bytes / 4;
-  return f + 64 * 40;       // carve() rounds every piece up to 64 floats
-}
-
 int ppo_grad_persistent(kbs_handle* h, const kbs_ppo_loss_params& L, const kbs_ppo_batch& b, const kbs_net_grads* const* grads,
                         float* log_probs, float* values, float* entropy, float* stats_out, int64_t n, cudaStream_t st) {
   const int H = h->p.hidden_size, depth = h->p.depth;
   const int64_t T = b.T, ld = b.ld, rows = T * n, np = (n + 127) / 128 * 128;
   const size_t npH = size_t(np) * H;
   const size_t sbb = kbs_tc_rows_sb_bytes(h, n, H), sb4 = kbs_tc_rows_sb_bytes(h, n, 4 * H);
-  const size_t ws_f = kbs_tc_rollout_ws_floats(h, n);
-  const size_t osb_f[2] = {size_t(kbs_tc_obs_sb_floats(h, 0, n, T)), size_t(kbs_tc_obs_sb_floats(h, 1, n, T))};
-  const size_t head_f = 3 * size_t(T) * KBS_NUM_JOINTS * ld + size_t(KBS_NUM_JOINTS) * ld + 64;
-  const size_t total = ws_f + osb_f[0] + osb_f[1] + head_f + persist_work_floats(h, 0, T, n) + persist_work_floats(h, 1, T, n) +
-                       size_t(16) * 4096 + 8192;
-  int rc = kbs_scratch_reserve(h, total);
-  if (rc) return rc;
-  float* p = h->scratch;
-  float* ws = carve(p, ws_f);
-  float* osb[2] = {carve(p, osb_f[0]), carve(p, osb_f[1])};
-  float* y_s = carve(p, size_t(T) * KBS_NUM_JOINTS * ld);
-  float* sd_s = carve(p, size_t(T) * KBS_NUM_JOINTS * ld);
-  float* sraw_s = carve(p, size_t(T) * KBS_NUM_JOINTS * ld);
-  float* lpf = carve(p, size_t(KBS_NUM_JOINTS) * ld);
-  double* loss_part = reinterpret_cast<double*>(carve(p, 8192));
   const KbsTnPlan plan = kbs_tc_tn_plan(h, T * np);
+  KbsTcRolloutWs rws;
+  float* osb[2]; float *y_s, *sd_s, *sraw_s, *lpf;
+  double* loss_part;
   PersistWork w[2];
-  for (int k = 0; k < 2; ++k) {
-    const size_t kpp = size_t(round_up_i(h->net[k].num_in + 1, 128));
-    const size_t m_panels = size_t(4 * H / 128), b_tiles = (kpp > size_t(2 * H) ? kpp : size_t(2 * H)) / 128 + 1;
-    w[k].x_sb = reinterpret_cast<char*>(carve(p, size_t(T) * sbb / 4));
-    w[k].xmid = reinterpret_cast<char*>(carve(p, size_t(depth) * T * sbb / 4));
-    w[k].hsb = reinterpret_cast<char*>(carve(p, size_t(depth) * (T + 1) * sbb / 4));
-    w[k].c_hist = carve(p, size_t(depth) * (T + 1) * npH);
-    w[k].save_g = carve(p, size_t(T) * depth * 4 * npH);
-    w[k].dG = reinterpret_cast<char*>(carve(p, size_t(depth) * (T + 1) * sb4 / 4));
-    w[k].dx = carve(p, size_t(depth) * T * npH);
-    w[k].dx0 = reinterpret_cast<char*>(carve(p, size_t(T) * sbb / 4));
-    w[k].dc = carve(p, size_t(depth) * npH);
-    w[k].dh_top = carve(p, size_t(rows) * H);
-    w[k].dout = carve(p, size_t(rows) * 64);
-    w[k].w_outT = carve(p, size_t(64) * H);
-    w[k].bflags = reinterpret_cast<unsigned int*>(carve(p, kbs_tc_bptt_flag_bytes(h, n) / 4));
-    w[k].h_top_rm = carve(p, size_t(rows) * H);
-    w[k].out = carve(p, size_t(rows) * 64);
-    w[k].fflags = reinterpret_cast<unsigned int*>(carve(p, kbs_tc_fwd_save_flag_bytes(h, n) / 4));
-    w[k].tn_a = reinterpret_cast<char*>(carve(p, m_panels * plan.col_bytes / 4));
-    w[k].tn_partial = carve(p, size_t(plan.ksplit) * m_panels * 128 * (b_tiles * 128));
-    w[k].tn_zero = carve(p, 1024);
-    w[k].tn_ones = reinterpret_cast<char*>(carve(p, 4096));
-    for (int l = 0; l < depth; ++l) w[k].tnb_layer[l] = reinterpret_cast<char*>(carve(p, size_t(2 * H / 128) * plan.col_bytes / 4));
-    w[k].tnb_top = reinterpret_cast<char*>(carve(p, size_t(H / 128) * plan.col_bytes / 4));
-    w[k].tnb_obs = reinterpret_cast<char*>(carve(p, kpp / 128 * plan.col_bytes / 4));
-    for (int l = 0; l < depth; ++l) w[k].tna_dG[l] = reinterpret_cast<char*>(carve(p, size_t(4 * H / 128) * plan.col_bytes / 4));
-  }
+  int rc = kbs_scratch(h, [&](KbsScratch& s) {
+    rws = kbs_tc_rollout_ws(s, h, n, 2);
+    for (int k = 0; k < 2; ++k) osb[k] = s.take<float>(kbs_tc_obs_sb_floats(h, k, n, T));
+    y_s = s.take<float>(size_t(T) * KBS_NUM_JOINTS * ld);
+    sd_s = s.take<float>(size_t(T) * KBS_NUM_JOINTS * ld);
+    sraw_s = s.take<float>(size_t(T) * KBS_NUM_JOINTS * ld);
+    lpf = s.take<float>(size_t(KBS_NUM_JOINTS) * ld);
+    loss_part = s.take<double>(4096);
+    for (int k = 0; k < 2; ++k) {
+      const size_t kpp = size_t(round_up_i(h->net[k].num_in + 1, 128));
+      const size_t m_panels = size_t(4 * H / 128), b_tiles = (kpp > size_t(2 * H) ? kpp : size_t(2 * H)) / 128 + 1;
+      w[k].x_sb = s.take<char>(size_t(T) * sbb);
+      w[k].xmid = s.take<char>(size_t(depth) * T * sbb);
+      w[k].hsb = s.take<char>(size_t(depth) * (T + 1) * sbb);
+      w[k].c_hist = s.take<float>(size_t(depth) * (T + 1) * npH);
+      w[k].save_g = s.take<float>(size_t(T) * depth * 4 * npH);
+      w[k].dG = s.take<char>(size_t(depth) * (T + 1) * sb4);
+      w[k].dx = s.take<float>(size_t(depth) * T * npH);
+      w[k].dx0 = s.take<char>(size_t(T) * sbb);
+      w[k].dc = s.take<float>(size_t(depth) * npH);
+      w[k].dh_top = s.take<float>(size_t(rows) * H);
+      w[k].dout = s.take<float>(size_t(rows) * 64);
+      w[k].w_outT = s.take<float>(size_t(64) * H);
+      w[k].bflags = s.take<unsigned int>(kbs_tc_bptt_flag_bytes(h, n) / 4);
+      w[k].h_top_rm = s.take<float>(size_t(rows) * H);
+      w[k].out = s.take<float>(size_t(rows) * 64);
+      w[k].fflags = s.take<unsigned int>(kbs_tc_fwd_save_flag_bytes(h, n) / 4);
+      w[k].tn_a = s.take<char>(m_panels * plan.col_bytes);
+      w[k].tn_partial = s.take<float>(size_t(plan.ksplit) * m_panels * 128 * (b_tiles * 128));
+      w[k].tn_zero = s.take<float>(1024);
+      w[k].tn_ones = s.take<char>(4096 * sizeof(float));
+      for (int l = 0; l < depth; ++l) w[k].tnb_layer[l] = s.take<char>(size_t(2 * H / 128) * plan.col_bytes);
+      w[k].tnb_top = s.take<char>(size_t(H / 128) * plan.col_bytes);
+      w[k].tnb_obs = s.take<char>(kpp / 128 * plan.col_bytes);
+      for (int l = 0; l < depth; ++l) w[k].tna_dG[l] = s.take<char>(size_t(4 * H / 128) * plan.col_bytes);
+    }
+  });
+  if (rc) return rc;
   // ---- forward ----
   // narrow-tile kernel (lstm_fwd_save_kernel: LSTM stacks only, heads as a batched GEMM + per-env scan afterwards) unless
   // KBS_PPO_FWD_WIDE=1 asks for rollout_persist_kernel<SAVE> (128 x 256 tiles, heads fused: the first version, kept for A/B)
@@ -1075,7 +1038,7 @@ int ppo_grad_persistent(kbs_handle* h, const kbs_ppo_loss_params& L, const kbs_p
     else KBS_CUDA_TRY(cudaMemsetAsync(lpf, 0, size_t(KBS_NUM_JOINTS) * ld * 4, st));
     r.lpf = lpf;
     r.action_in = b.action; r.log_prob = log_probs; r.entropy = entropy; r.action_std = sd_s; r.mean = y_s; r.value = values;
-    r.ws = ws;
+    r.ws = rws;
     r.save = 1; r.sraw = sraw_s;
     for (int k = 0; k < 2; ++k) { r.xmid_hist[k] = w[k].xmid; r.hsb_hist[k] = w[k].hsb; r.c_hist[k] = w[k].c_hist; r.save_g[k] = w[k].save_g; }
     if ((rc = kbs_tc_rollout_recurrent(h, r, st))) return rc;
@@ -1395,58 +1358,55 @@ int kbs_ppo_grad(kbs_handle* h, const kbs_ppo_loss_params* params, const kbs_ppo
   const int kp_max = round_up_i(KBS_CRITIC_OBS, 64);
   const bool tc = h->p.gemm_path != KBS_GEMM_SIMT_FP32;
   const size_t part_f = size_t(chunks) * 4 * H + size_t(splits) * size_t(4 * H) * size_t(kp_max) + size_t(H) * kp_max + 64 * H + 4096;
-  const size_t shared_f = 2 * (sH * 4 /*gates_pre*/ + size_t(depth) * sH /*dc_rec*/ + part_f + 1024) +
-                          2 * size_t(T) * KBS_NUM_JOINTS * ld /*y_s, sd_s*/;
-  const size_t total_f = shared_f + net_work_floats(h, 0, T, n, tc) + net_work_floats(h, 1, T, n, tc) + 8192;
-  int rc = kbs_scratch_reserve(h, total_f);
-  if (rc) return rc;
-  float* p = h->scratch;
-  float* gates_pre[2]; float* dc_rec[2]; float* part[2];
-  for (int k = 0; k < 2; ++k) {            // per net: actor and critic run concurrently on two streams
-    gates_pre[k] = carve(p, sH * 4);
-    dc_rec[k] = carve(p, size_t(depth) * sH);
-    part[k] = carve(p, part_f);
-  }
-  float* y_s = carve(p, size_t(T) * KBS_NUM_JOINTS * ld);
-  float* sd_s = carve(p, size_t(T) * KBS_NUM_JOINTS * ld);
+  float* gates_pre[2]; float* dc_rec[2]; float* part[2]; float *y_s, *sd_s;
   NetWork w[2];
-  for (int k = 0; k < 2; ++k) {
-    const size_t kp = size_t(round_up_i(h->net[k].num_in, 64));
-    w[k].obs_rm = carve(p, size_t(rows) * kp);
-    w[k].x0 = carve(p, size_t(rows) * H);
-    w[k].dh_top = carve(p, size_t(rows) * H);
-    w[k].dxh0 = carve(p, size_t(rows) * 2 * H);
-    w[k].out = carve(p, size_t(rows) * 64);
-    w[k].dout = carve(p, size_t(rows) * 64);
-    for (int l = 0; l < depth; ++l) {
-      w[k].dxh[l] = carve(p, sH * 2);
-      w[k].ga[l] = carve(p, size_t(rows) * 4 * H);
-      w[k].dG[l] = carve(p, size_t(rows) * 4 * H);
-      w[k].cs[l] = carve(p, size_t(rows) * H);
-      w[k].hs[l] = carve(p, size_t(rows) * H);
-      w[k].h_in[l] = carve(p, size_t(rows) * H);
-      w[k].c_in[l] = carve(p, size_t(rows) * H);
-      w[k].w_ihT[l] = carve(p, size_t(4) * H * H);
-      w[k].w_hhT[l] = carve(p, size_t(4) * H * H);
+  int rc = kbs_scratch(h, [&](KbsScratch& s) {
+    for (int k = 0; k < 2; ++k) {            // per net: actor and critic run concurrently on two streams
+      gates_pre[k] = s.take<float>(sH * 4);
+      dc_rec[k] = s.take<float>(size_t(depth) * sH);
+      part[k] = s.take<float>(part_f);
     }
-    w[k].w_outT = carve(p, size_t(64) * H);
-    if (tc) {
-      const size_t sbH = kbs_tc_rows_sb_bytes(h, n, H) / 4, sb4H = kbs_tc_rows_sb_bytes(h, n, 4 * H) / 4;
-      w[k].x0_sb = reinterpret_cast<char*>(carve(p, size_t(T) * sbH));
+    y_s = s.take<float>(size_t(T) * KBS_NUM_JOINTS * ld);
+    sd_s = s.take<float>(size_t(T) * KBS_NUM_JOINTS * ld);
+    for (int k = 0; k < 2; ++k) {
+      const size_t kp = size_t(round_up_i(h->net[k].num_in, 64));
+      w[k].obs_rm = s.take<float>(size_t(rows) * kp);
+      w[k].x0 = s.take<float>(size_t(rows) * H);
+      w[k].dh_top = s.take<float>(size_t(rows) * H);
+      w[k].dxh0 = s.take<float>(size_t(rows) * 2 * H);
+      w[k].out = s.take<float>(size_t(rows) * 64);
+      w[k].dout = s.take<float>(size_t(rows) * 64);
       for (int l = 0; l < depth; ++l) {
-        w[k].hs_sb[l] = reinterpret_cast<char*>(carve(p, size_t(T) * sbH));
-        w[k].h_in_sb[l] = reinterpret_cast<char*>(carve(p, size_t(T) * sbH));
+        w[k].dxh[l] = s.take<float>(sH * 2);
+        w[k].ga[l] = s.take<float>(size_t(rows) * 4 * H);
+        w[k].dG[l] = s.take<float>(size_t(rows) * 4 * H);
+        w[k].cs[l] = s.take<float>(size_t(rows) * H);
+        w[k].hs[l] = s.take<float>(size_t(rows) * H);
+        w[k].h_in[l] = s.take<float>(size_t(rows) * H);
+        w[k].c_in[l] = s.take<float>(size_t(rows) * H);
+        w[k].w_ihT[l] = s.take<float>(size_t(4) * H * H);
+        w[k].w_hhT[l] = s.take<float>(size_t(4) * H * H);
       }
-      w[k].dG_sb = reinterpret_cast<char*>(carve(p, sb4H));
-      const KbsTnPlan plan = kbs_tc_tn_plan(h, rows);
-      const size_t m_panels = size_t(4 * H / 128), b_tiles = size_t((int(kp) > 2 * H ? int(kp) : 2 * H) / 128 + 1);
-      w[k].tn_a = reinterpret_cast<char*>(carve(p, m_panels * plan.col_bytes / 4));
-      w[k].tn_b = reinterpret_cast<char*>(carve(p, b_tiles * plan.col_bytes / 4));
-      w[k].tn_partial = carve(p, size_t(plan.ksplit) * m_panels * 128 * (b_tiles * 128));
-      w[k].tn_zero = carve(p, 1024);
-      w[k].tn_ones = reinterpret_cast<char*>(carve(p, 4096));
+      w[k].w_outT = s.take<float>(size_t(64) * H);
+      if (tc) {
+        const size_t sbH = kbs_tc_rows_sb_bytes(h, n, H), sb4H = kbs_tc_rows_sb_bytes(h, n, 4 * H);
+        w[k].x0_sb = s.take<char>(size_t(T) * sbH);
+        for (int l = 0; l < depth; ++l) {
+          w[k].hs_sb[l] = s.take<char>(size_t(T) * sbH);
+          w[k].h_in_sb[l] = s.take<char>(size_t(T) * sbH);
+        }
+        w[k].dG_sb = s.take<char>(sb4H);
+        const KbsTnPlan plan = kbs_tc_tn_plan(h, rows);
+        const size_t m_panels = size_t(4 * H / 128), b_tiles = size_t((int(kp) > 2 * H ? int(kp) : 2 * H) / 128 + 1);
+        w[k].tn_a = s.take<char>(m_panels * plan.col_bytes);
+        w[k].tn_b = s.take<char>(b_tiles * plan.col_bytes);
+        w[k].tn_partial = s.take<float>(size_t(plan.ksplit) * m_panels * 128 * (b_tiles * 128));
+        w[k].tn_zero = s.take<float>(1024);
+        w[k].tn_ones = s.take<char>(4096 * sizeof(float));
+      }
     }
-  }
+  });
+  if (rc) return rc;
   // The two networks share nothing until the loss statistics: the critic runs on the handle's side stream, forked from
   // and joined into the caller's stream with events (capturable: the whole call can be replayed as one CUDA graph).
   { const int rc0 = kbs_side_stream_init(h); if (rc0) return rc0; }
