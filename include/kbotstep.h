@@ -464,6 +464,79 @@ struct kbs_rollout_record {
 int kbs_rollout_record(kbs_handle* h, const kbs_rollout_io* io, const struct kbs_rollout_record* rec, int64_t n_envs,
                        void* stream);
 
+/* The online rollout: one control step per call, the form a simulator loop around mjx.step drives (state t+1 depends on
+ * the ctrl of step t).  What crosses a step boundary stays on the device in a caller-owned STEP STATE: one device buffer of
+ * kbs_step_state_bytes bytes, 256-byte aligned (any cudaMalloc'd or torch-allocated buffer is).  The library keeps none of
+ * it in its scratch, which every other entry point reuses between steps.  It holds:
+ *   - the actor and critic carries in the operand layouts the rollout kernels read and write: on the tensor-core datapaths
+ *     the split-blocked h operand in two slots with a device word naming the slot the next step reads, and the fp32 c and h;
+ *     on SIMT the ABI carries;
+ *   - lpf, pg_carry, the current command row and done_prev (the previous step's done);
+ *   - the step index t (device int64): every kbs_rollout_step reads it and then advances it by one, like step_dev of
+ *     kbs_adamw_step, so one captured CUDA graph of the step serves every step of an iteration.
+ * Its per-env rows are at ld = n_envs rounded up to a multiple of 4; the arrays kbs_rollout_step takes use that ld too. */
+typedef struct kbs_step_state {
+  void* buf;                  /* device, 256-byte aligned */
+  uint64_t bytes;             /* size of buf: >= kbs_step_state_bytes(h, n_envs, with_critic) */
+  int64_t n_envs;
+  int32_t with_critic;        /* room for the critic's carries (kbs_rollout_step with value != NULL needs it) */
+} kbs_step_state;
+int kbs_step_state_bytes(kbs_handle* h, int64_t n_envs, int with_critic, uint64_t* bytes);
+
+/* ABI form of what a step state carries.  On load any pointer may be NULL (= zeros: get_initial_model_carry, no previous
+ * done); on store NULL = not written. */
+typedef struct kbs_step_carry {
+  float* actor_carry;         /* AoS [depth][2][n][H] */
+  float* critic_carry;        /* AoS [depth][2][n][H] (with_critic states only) */
+  float* lpf;                 /* [20][ld] */
+  float* pg_carry;            /* [3][ld] */
+  float* command;             /* [16][ld]: the command of the next step (row 0 of a rollout's command) */
+  uint8_t* done_prev;         /* [ld], 4-byte aligned: the done of the step before the next one */
+} kbs_step_carry;
+/* Fills the state from `in` and sets t = 0 and the h slot to 0. */
+int kbs_step_state_load(kbs_handle* h, const kbs_step_state* st, const kbs_step_carry* in, void* stream);
+/* The reverse, leaving the state as it is.  After the same steps, the carries, lpf, pg_carry and command are bitwise what
+ * kbs_rollout_record leaves in io (command: row T), and done_prev is its done[T-1]. */
+int kbs_step_state_store(kbs_handle* h, const kbs_step_state* st, const kbs_step_carry* out, void* stream);
+/* Sets the step index back to 0 and changes nothing else: the next iteration of an online rollout records into slot 0 again.
+ * It does not repair a state that a step past T left behind (see kbs_rollout_step): load that one again. */
+int kbs_step_state_rewind(kbs_handle* h, const kbs_step_state* st, void* stream);
+
+/* One control step of the online rollout.  Inputs are this step's [F][ld] arrays.  Outputs are trajectories; slot t is
+ * written, t being the state's step index read on the device.  The stages are those of kbs_rollout_record, and T calls from a
+ * loaded state give bitwise the outputs of one T-step kbs_rollout_record call (with done_prev, and critic_obs where asked)
+ * from the same carries. */
+typedef struct kbs_step_io {
+  kbs_state_view state;       /* this step: [F][ld] */
+  kbs_noise_view noise;       /* this step: [..][ld] */
+  kbs_episode_view episode;   /* per env */
+  const float* eps_action;    /* [20][ld] N(0,1) or NULL (argmax) */
+  const float* u_switch;      /* [ld] */
+  const int32_t* cmd_mode;    /* [ld] */
+  const float* cmd_u6;        /* [6][ld] */
+  const float* cmd_u_arms;    /* [10][ld] */
+  /* trajectories [T][..][ld], slot t written */
+  float* command;             /* [T+1][16][ld]: rows t (the state's command) and t+1 (the next one) */
+  float* actor_obs;           /* [T][65][ld] or NULL */
+  float* critic_obs;          /* [T][475][ld] or NULL (needs cinert, cvel, actuator_force in state) */
+  float* action;              /* [T][20][ld] */
+  float* log_prob;            /* [T][ld] or NULL */
+  float* ctrl;                /* [T][20][ld] */
+  int32_t* term_codes;        /* [T][3][ld] or NULL */
+  uint8_t* done;              /* [T][ld] */
+  uint8_t* success;           /* [T][ld] */
+  float* value;               /* [T][ld] or NULL (the critic is not run); needs a with_critic state and cinert, cvel,
+                                 actuator_force */
+  kbs_state_view traj_state;  /* [T][F][ld]: copies of this step's state fields (what kbs_rewards reads afterwards); a NULL
+                                 field is not recorded, and needs a non-NULL state field otherwise; ld ignored */
+  int64_t T;                  /* trajectory length */
+} kbs_step_io;
+/* The step's index is only known on the device.  A step that finds t >= T records nothing and leaves t as it is; it sets
+ * KBS_STATUS_STEP_RANGE in the health word, so the next fused call returns KBS_E_DEVICE.  The carries in the state did
+ * advance: load it again.  On the tensor-core datapaths the recurrence is the persistent kernel with T = 1 (KBS_E_SHAPE for an
+ * n_envs it cannot take). */
+int kbs_rollout_step(kbs_handle* h, const kbs_step_state* st, const kbs_step_io* io, void* stream);
+
 /* Replaces: the jax.random draws the reference makes ON THE DEVICE during a rollout -- observation noise (train.py:1160, 1162,
  * 1176, 1194), the action sample (train.py:1564), the command resampling (train.py:725-737, 752-753, 782-783) -- for callers
  * that do not need bit parity with JAX's threefry streams (parity mode hands these arrays to kbs_rollout explicitly).
@@ -527,6 +600,7 @@ int kbs_device_status(kbs_handle* h, int* status_out);
 #define KBS_STATUS_TIMEOUT_LSTM 1
 #define KBS_STATUS_TIMEOUT_HEAD 2
 #define KBS_STATUS_F16_RANGE 0x100
+#define KBS_STATUS_STEP_RANGE 0x200   /* kbs_rollout_step found its step index t >= T */
 int kbs_device_status_reset(kbs_handle* h);
 
 /* Per-kernel device timing for bench.py's roofline line: while enabled, every kernel launch of this handle is
@@ -544,7 +618,7 @@ int kbs_debug_tc_trace(kbs_handle* h, long long* trace_out, int64_t n_envs, void
 /* Same stamps for LSTM layer `layer` at step `step` of subsequent kbs_rollout calls (trace_out NULL detaches). */
 int kbs_debug_tc_trace_attach(kbs_handle* h, long long* trace_out, int64_t step, int layer);
 
-#define KBS_NUM_KERNEL_IDS 24
+#define KBS_NUM_KERNEL_IDS 25
 int kbs_profile_enable(kbs_handle* h, int on);
 int kbs_profile_read(kbs_handle* h, int max_ids, double* total_ms, int64_t* launches);
 const char* kbs_kernel_name(int id);

@@ -87,6 +87,24 @@ class KbsRolloutRecord(C.Structure):
     _fields_ = [("done_prev", _vp), ("critic_obs", _vp)]
 
 
+class KbsStepState(C.Structure):
+    """kbs_step_state: the caller-owned device buffer of the online rollout and what it was sized for."""
+    _fields_ = [("buf", _vp), ("bytes", C.c_uint64), ("n_envs", _i64), ("with_critic", C.c_int32)]
+
+
+class KbsStepCarry(C.Structure):
+    """kbs_step_carry: the ABI form of what a step state carries (load / store)."""
+    _fields_ = [(k, _vp) for k in ("actor_carry", "critic_carry", "lpf", "pg_carry", "command", "done_prev")]
+
+
+class KbsStepIO(C.Structure):
+    """kbs_step_io: one step's inputs, and the trajectories whose slot t it writes."""
+    _fields_ = [("state", KbsStateView), ("noise", KbsNoiseView), ("episode", KbsEpisodeView)] + [
+        (k, _vp) for k in ("eps_action", "u_switch", "cmd_mode", "cmd_u6", "cmd_u_arms", "command", "actor_obs", "critic_obs",
+                           "action", "log_prob", "ctrl", "term_codes", "done", "success", "value")] + [
+        ("traj_state", KbsStateView), ("T", _i64)]
+
+
 class KbsPpoIO(C.Structure):
     _fields_ = [(k, _vp) for k in ("actor_obs", "critic_obs", "action", "done", "actor_carry", "critic_carry", "lpf",
                                    "log_probs", "values", "entropy", "action_std", "mean")] + [("T", _i64), ("ld", _i64)] + [
@@ -138,11 +156,12 @@ EXPORTS = (
     "kbs_launch_count", "kbs_device_status", "kbs_mirror_observations", "kbs_mirror_joints", "kbs_upload_state", "kbs_com_distance", "kbs_ppo_loss_default_params", "kbs_ppo_loss", "kbs_ppo_grad", "kbs_adam_step", "kbs_torque_substeps", "kbs_profile_enable", "kbs_profile_read", "kbs_kernel_name", "kbs_debug_tc_gates", "kbs_debug_tc_trace", "kbs_debug_tc_trace_attach",
     "kbs_adamw_default_params", "kbs_adamw_step", "kbs_grad_norm", "kbs_scratch_lock", "kbs_actuator_rand_default_params",
     "kbs_sample_actuator_randomization", "kbs_device_status_reset", "kbs_ppo_grad_set_events", "kbs_generate_rollout_noise",
-    "kbs_minibatch_permutation", "kbs_shuffle_minibatches", "kbs_rollout_record",
+    "kbs_minibatch_permutation", "kbs_shuffle_minibatches", "kbs_rollout_record", "kbs_step_state_bytes", "kbs_step_state_load",
+    "kbs_step_state_store", "kbs_step_state_rewind", "kbs_rollout_step",
 )
 VERSION = 101
-STATUS_TIMEOUT_LSTM, STATUS_TIMEOUT_HEAD, STATUS_F16_RANGE = 1, 2, 0x100
-NUM_KERNEL_IDS = 24
+STATUS_TIMEOUT_LSTM, STATUS_TIMEOUT_HEAD, STATUS_F16_RANGE, STATUS_STEP_RANGE = 1, 2, 0x100, 0x200
+NUM_KERNEL_IDS = 25
 MAX_PERMUTATION_ENVS = 16384
 
 _lib = None
@@ -202,6 +221,11 @@ def load() -> C.CDLL:
     lib.kbs_rollout.argtypes = [_vp, P(KbsRolloutIO), _i64, _vp]
     lib.kbs_rollout_record.argtypes = [_vp, P(KbsRolloutIO), P(KbsRolloutRecord), _i64, _vp]
     lib.kbs_ppo_variables.argtypes = [_vp, P(KbsPpoIO), _i64, _vp]
+    lib.kbs_step_state_bytes.argtypes = [_vp, _i64, C.c_int, P(C.c_uint64)]
+    lib.kbs_step_state_load.argtypes = [_vp, P(KbsStepState), P(KbsStepCarry), _vp]
+    lib.kbs_step_state_store.argtypes = [_vp, P(KbsStepState), P(KbsStepCarry), _vp]
+    lib.kbs_step_state_rewind.argtypes = [_vp, P(KbsStepState), _vp]
+    lib.kbs_rollout_step.argtypes = [_vp, P(KbsStepState), P(KbsStepIO), _vp]
     lib.kbs_launch_count.argtypes = [_vp]
     lib.kbs_launch_count.restype = _i64
     lib.kbs_device_status.argtypes = [_vp, P(C.c_int)]

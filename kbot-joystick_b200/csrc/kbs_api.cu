@@ -99,35 +99,50 @@ int trunk(kbs_handle* h, int net, const float* obs, int64_t ld, float* carry, co
 // form -- 2 LSTM layer launches for both nets + a head launch per step -- stays behind KBS_TC_PER_STEP=1).
 // done_prev restarts the lag scan at step 0; critic_obs (when given) replaces the per-chunk scratch of the critic's
 // observations and gets all 475 rows, the input projection still reads cinert / cvel straight from the state.
-int rollout_fused_tc(kbs_handle* h, const kbs_rollout_io* io, const uint8_t* done_prev, float* critic_obs, int64_t n,
-                     cudaStream_t st) {
+// Observation assembly + input projections can run in chunks of CT steps on the handle's aux stream while the
+// recurrence of the previous chunk runs on the caller's stream (KBS_ROLLOUT_CHUNKS = 2..8).  MEASURED: slower
+// (9.97 vs 8.89 ms per 100-step rollout): the persistent recurrence kernel wants every SM to itself, so the
+// concurrent kernels delay its CTAs more than they hide.  Default = 1 chunk: phase A first, then the recurrence.
+int rollout_chunks() {
+  const char* e = getenv("KBS_ROLLOUT_CHUNKS");
+  const int c = e ? atoi(e) : 1;
+  return (c < 1 || c > kKbsMaxChunks) ? 1 : c;
+}
+
+// Workspace of rollout_fused_tc: the recurrence's, the lag states of all T steps (when pg_carry is carried), the actor's
+// observations when the caller keeps none, the critic's when it records none, and the operands of the input projections.
+struct FusedTcWs { KbsTcRolloutWs r; float *lagged, *aobs, *cobs, *xsb_a, *xsb_c, *osb_a, *osb_c; };
+FusedTcWs fused_tc_ws(KbsScratch& s, const kbs_handle* h, int64_t n, int64_t ld, int64_t T, int chunks, bool critic, bool pg,
+                      bool own_aobs, bool own_cobs) {
+  const int64_t CT = (T + chunks - 1) / chunks;
+  const size_t sbf = size_t(kbs_tc_sb_floats(h, n));
+  FusedTcWs w{};
+  w.r = kbs_tc_rollout_ws(s, h, n, critic ? 2 : 1);
+  w.lagged = pg ? s.take<float>(size_t(T) * 3 * ld) : nullptr;
+  w.aobs = own_aobs ? nullptr : s.take<float>(size_t(T) * KBS_ACTOR_OBS * ld);
+  w.cobs = (critic && !own_cobs) ? s.take<float>(size_t(CT) * KBS_CRITIC_OBS * ld) : nullptr;
+  w.xsb_a = s.take<float>(size_t(T) * sbf);
+  w.xsb_c = critic ? s.take<float>(size_t(T) * sbf) : nullptr;
+  w.osb_a = s.take<float>(kbs_tc_obs_sb_floats(h, KBS_NET_ACTOR, n, CT));
+  w.osb_c = critic ? s.take<float>(kbs_tc_obs_sb_floats(h, KBS_NET_CRITIC, n, CT)) : nullptr;
+  return w;
+}
+
+// res (kbs_rollout_step): the carries are resident in a step state (KbsTcRolloutArgs::res_*), io->*_carry are not read.
+int rollout_fused_tc(kbs_handle* h, const kbs_rollout_io* io, const uint8_t* done_prev, float* critic_obs, const FusedTcWs& w,
+                     int chunks_cfg, const KbsTcRolloutArgs* res, int64_t n, cudaStream_t st) {
   const int64_t ld = io->state.ld, T = io->T;
   const bool critic = io->value != nullptr;
-  // Observation assembly + input projections can run in chunks of CT steps on the handle's aux stream while the
-  // recurrence of the previous chunk runs on the caller's stream (KBS_ROLLOUT_CHUNKS = 2..8).  MEASURED: slower
-  // (9.97 vs 8.89 ms per 100-step rollout): the persistent recurrence kernel wants every SM to itself, so the
-  // concurrent kernels delay its CTAs more than they hide.  Default = 1 chunk: phase A first, then the recurrence.
-  int chunks_cfg = 1;
-  {
-    const char* e = getenv("KBS_ROLLOUT_CHUNKS");
-    chunks_cfg = e ? atoi(e) : 1;
-    if (chunks_cfg < 1 || chunks_cfg > kKbsMaxChunks) chunks_cfg = 1;
-  }
   const int64_t CT = (T + chunks_cfg - 1) / chunks_cfg;
   const size_t sbf = size_t(kbs_tc_sb_floats(h, n));
   KbsTcRolloutArgs r{};
-  float *lagged, *aobs, *cobs, *xsb_a, *xsb_c, *osb_a, *osb_c;
-  int rc = kbs_scratch(h, [&](KbsScratch& s) {
-    r.ws = kbs_tc_rollout_ws(s, h, n, critic ? 2 : 1);
-    lagged = io->pg_carry ? s.take<float>(size_t(T) * 3 * ld) : nullptr;
-    aobs = io->actor_obs ? io->actor_obs : s.take<float>(size_t(T) * KBS_ACTOR_OBS * ld);
-    cobs = critic_obs ? critic_obs : critic ? s.take<float>(size_t(CT) * KBS_CRITIC_OBS * ld) : nullptr;
-    xsb_a = s.take<float>(size_t(T) * sbf);
-    xsb_c = critic ? s.take<float>(size_t(T) * sbf) : nullptr;
-    osb_a = s.take<float>(kbs_tc_obs_sb_floats(h, KBS_NET_ACTOR, n, CT));
-    osb_c = critic ? s.take<float>(kbs_tc_obs_sb_floats(h, KBS_NET_CRITIC, n, CT)) : nullptr;
-  });
-  if (rc) return rc;
+  if (res) { for (int k = 0; k < 2; ++k) { r.res_hsb[k] = res->res_hsb[k]; r.res_fb[k] = res->res_fb[k]; } r.res_hsb_slot = res->res_hsb_slot; }
+  r.ws = w.r;
+  float* lagged = w.lagged;
+  float* aobs = io->actor_obs ? io->actor_obs : w.aobs;
+  float* cobs = critic_obs ? critic_obs : w.cobs;
+  float *xsb_a = w.xsb_a, *xsb_c = w.xsb_c, *osb_a = w.osb_a, *osb_c = w.osb_c;
+  int rc;
 
   if ((rc = kbs_launch_terminate(h, io->state, io->term_codes, io->done, io->success, nullptr, n, st, T))) return rc;
   if (lagged) {
@@ -156,7 +171,7 @@ int rollout_fused_tc(kbs_handle* h, const kbs_rollout_io* io, const uint8_t* don
     float* cobs_c = critic_obs ? critic_obs + t0 * KBS_CRITIC_OBS * ld : cobs;
     if ((rc = kbs_launch_observations(h, s, &nz, &io->episode, io->command + t0 * KBS_NUM_COMMANDS * ld, nullptr, nullptr,
                                       nullptr, aobs_c, cobs_c, n, aux, tc, lagged ? lagged + t0 * 3 * ld : nullptr,
-                                      /*skip_dump=*/critic_obs == nullptr)))
+                                      /*skip_dump=*/critic_obs == nullptr, /*one_step=*/res != nullptr)))
       return rc;
     const float* obs_soa[2] = {aobs_c, cobs_c};
     float* obs_sb[2] = {osb_a, osb_c};
@@ -176,6 +191,18 @@ int rollout_fused_tc(kbs_handle* h, const kbs_rollout_io* io, const uint8_t* don
   r.action = io->action; r.log_prob = io->log_prob; r.ctrl = io->ctrl; r.value = io->value;
   return kbs_tc_rollout_recurrent(h, r, st);
 }
+
+// Workspace of rollout_simt: the trunk's, and one step of observations the caller does not keep.
+struct SimtRolloutWs { TrunkWs trunk; float* aobs; float* cobs; };
+SimtRolloutWs simt_rollout_ws(KbsScratch& s, const kbs_handle* h, int64_t n, int64_t ld) {
+  SimtRolloutWs w{};
+  w.trunk = trunk_ws(s, h, n);
+  w.aobs = s.take<float>(size_t(KBS_ACTOR_OBS) * ld);
+  w.cobs = s.take<float>(size_t(KBS_CRITIC_OBS) * ld);
+  return w;
+}
+int rollout_simt(kbs_handle* h, const kbs_rollout_io* io, const uint8_t* done_prev, float* critic_obs, const SimtRolloutWs& w,
+                 int64_t n, cudaStream_t st, bool one_step = false);
 
 }  // namespace
 
@@ -433,7 +460,7 @@ const char* kbs_kernel_name(int id) {
       "reward_scan_kernel", "gae_kernel", "adv_norm_kernel", "policy_io_kernels", "gemm_nt_kernel(simt)",
       "lstm_cell_kernel", "actor_head_kernel", "critic_head_kernel", "pack_kernels", "lstm_layer_tc_kernel",
       "proj_tc_kernel", "rollout_persist_kernel", "bptt_persist_kernel", "gemm_tn_tc_kernel", "sb_to_tn_kernel", "tn_reduce_kernel",
-      "minibatch_permutation_kernel", "shuffle_minibatches_kernels"};
+      "step_record_kernel", "minibatch_permutation_kernel", "shuffle_minibatches_kernels"};
   return (id >= 0 && id < KBS_K_COUNT) ? names[id] : "?";
 }
 
@@ -910,17 +937,35 @@ int kbs_rollout_record(kbs_handle* h, const kbs_rollout_io* io, const struct kbs
   AL(critic_obs);
   if (reinterpret_cast<uintptr_t>(done_prev) & 3u) return KBS_E_ALIGN;
   cudaStream_t st = (cudaStream_t)stream;
-  if (h->p.gemm_path != KBS_GEMM_SIMT_FP32) return rollout_fused_tc(h, io, done_prev, critic_obs, n, st);
   const int64_t ld = io->state.ld;
-  TrunkWs ws;
-  float *aobs_scratch, *cobs;
-  rc = kbs_scratch(h, [&](KbsScratch& s) {
-    ws = trunk_ws(s, h, n);
-    aobs_scratch = s.take<float>(size_t(KBS_ACTOR_OBS) * ld);
-    cobs = s.take<float>(size_t(KBS_CRITIC_OBS) * ld);
-  });
-  if (rc) return rc;
+  if (h->p.gemm_path != KBS_GEMM_SIMT_FP32) {
+    const int chunks = rollout_chunks();
+    FusedTcWs w;
+    if ((rc = kbs_scratch(h, [&](KbsScratch& s) {
+           w = fused_tc_ws(s, h, n, ld, io->T, chunks, io->value != nullptr, io->pg_carry != nullptr, io->actor_obs != nullptr,
+                           critic_obs != nullptr);
+         })))
+      return rc;
+    return rollout_fused_tc(h, io, done_prev, critic_obs, w, chunks, nullptr, n, st);
+  }
+  SimtRolloutWs ws;
+  if ((rc = kbs_scratch(h, [&](KbsScratch& s) { ws = simt_rollout_ws(s, h, n, ld); }))) return rc;
+  return rollout_simt(h, io, done_prev, critic_obs, ws, n, st);
+}
 
+}  // extern "C"
+
+namespace {
+
+// The exact-fp32 rollout: T x (terminate, observations, actor trunk + head, torque, [critic trunk + head], command)
+// one_step: kbs_rollout_step's T = 1 call (the observation kernel's one-step launch shape)
+int rollout_simt(kbs_handle* h, const kbs_rollout_io* io, const uint8_t* done_prev, float* critic_obs, const SimtRolloutWs& w,
+                 int64_t n, cudaStream_t st, bool one_step) {
+  const int64_t ld = io->state.ld;
+  const TrunkWs& ws = w.trunk;
+  float* aobs_scratch = w.aobs;
+  float* cobs = w.cobs;
+  int rc;
   for (int64_t t = 0; t < io->T; ++t) {
     const kbs_state_view s = state_at(io->state, t);
     const kbs_noise_view nz = noise_at(io->noise, t, ld);
@@ -934,7 +979,7 @@ int kbs_rollout_record(kbs_handle* h, const kbs_rollout_io* io, const struct kbs
                                    io->success + t * ld, nullptr, n, st)))
       return rc;
     if ((rc = kbs_launch_observations(h, s, &nz, &io->episode, cmd_t, io->pg_carry, t > 0 ? done_t - ld : done_prev,
-                                      nullptr, aobs, cobs_t, n, st)))
+                                      nullptr, aobs, cobs_t, n, st, 1, nullptr, false, one_step)))
       return rc;
     if ((rc = trunk(h, KBS_NET_ACTOR, aobs, ld, io->actor_carry, done_t, ws, n, st))) return rc;
     kbs_actor_out o{};
@@ -954,6 +999,238 @@ int kbs_rollout_record(kbs_handle* h, const kbs_rollout_io* io, const struct kbs
       return rc;
   }
   return KBS_OK;
+}
+
+}  // namespace
+
+// ---- the online rollout: one control step per call on a caller-owned step state ----------------------------------------------
+namespace {
+
+struct StepHeader { int64_t t; int32_t hsb_slot; uint32_t ticket; };
+// Layout of a step state, carved from the caller's buffer like scratch (rows at ld = round_up4(n)).
+struct StepState {
+  StepHeader* hdr; uint8_t* done_prev; float* command /* [2][16][ld]: current, next */; float* lpf; float* pg_carry;
+  KbsTcStepNet tc[2]; float* carry[2];
+};
+StepState step_state(KbsScratch& s, const kbs_handle* h, int64_t n, bool critic) {
+  const int64_t ld = round_up4(n);
+  StepState w{};
+  w.hdr = s.take<StepHeader>(1);
+  w.done_prev = s.take<uint8_t>(size_t(ld));
+  w.command = s.take<float>(size_t(2) * KBS_NUM_COMMANDS * ld);
+  w.lpf = s.take<float>(size_t(KBS_NUM_JOINTS) * ld);
+  w.pg_carry = s.take<float>(size_t(3) * ld);
+  for (int k = 0; k < (critic ? 2 : 1); ++k) {
+    if (h->p.gemm_path == KBS_GEMM_SIMT_FP32) w.carry[k] = s.take<float>(size_t(h->p.depth) * 2 * n * h->p.hidden_size);
+    else w.tc[k] = kbs_tc_step_net(s, h, n);
+  }
+  return w;
+}
+
+uint64_t step_state_bytes(const kbs_handle* h, int64_t n, bool critic) {
+  KbsScratch s{nullptr};
+  step_state(s, h, n, critic);
+  return s.bytes;
+}
+
+// the descriptor's checks, then the layout on its buffer
+int step_state_at(const kbs_handle* h, const kbs_step_state* st, StepState* w) {
+  REQ(st); REQ(st->buf);
+  if (st->n_envs <= 0) return KBS_E_SHAPE;
+  if (reinterpret_cast<uintptr_t>(st->buf) & 255u) return KBS_E_ALIGN;
+  if (st->bytes < step_state_bytes(h, st->n_envs, st->with_critic != 0)) return KBS_E_SHAPE;
+  if (h->p.gemm_path != KBS_GEMM_SIMT_FP32 && !kbs_tc_persistent_available(h, st->n_envs, 1, st->with_critic ? 2 : 1))
+    return KBS_E_SHAPE;
+  KbsScratch s{static_cast<char*>(st->buf)};
+  *w = step_state(s, h, st->n_envs, st->with_critic != 0);
+  return KBS_OK;
+}
+
+int check_step_carry(const kbs_step_state* st, const kbs_step_carry* c) {
+  REQ(c);
+  if (c->critic_carry && !st->with_critic) return KBS_E_PARAM;
+  AL(c->actor_carry); AL(c->critic_carry); AL(c->lpf); AL(c->pg_carry); AL(c->command);
+  if (reinterpret_cast<uintptr_t>(c->done_prev) & 3u) return KBS_E_ALIGN;
+  return KBS_OK;
+}
+
+// dst <- src (bytes), or zeros when src is NULL
+int copy_or_zero(void* dst, const void* src, size_t bytes, cudaStream_t st) {
+  if (src) KBS_CUDA_TRY(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, st));
+  else KBS_CUDA_TRY(cudaMemsetAsync(dst, 0, bytes, st));
+  return KBS_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int kbs_step_state_bytes(kbs_handle* h, int64_t n, int with_critic, uint64_t* bytes) {
+  REQ(h); REQ(bytes);
+  if (n <= 0) return KBS_E_SHAPE;
+  *bytes = step_state_bytes(h, n, with_critic != 0);
+  return KBS_OK;
+}
+
+int kbs_step_state_load(kbs_handle* h, const kbs_step_state* st, const kbs_step_carry* in, void* stream) {
+  REQ(h);
+  StepState w;
+  int rc = step_state_at(h, st, &w);
+  if (rc || (rc = check_step_carry(st, in)) || (rc = kbs_enter(h))) return rc;
+  cudaStream_t s = (cudaStream_t)stream;
+  const int64_t n = st->n_envs, ld = round_up4(n);
+  KBS_CUDA_TRY(cudaMemsetAsync(w.hdr, 0, sizeof(StepHeader), s));
+  if ((rc = copy_or_zero(w.done_prev, in->done_prev, size_t(ld), s))) return rc;
+  if ((rc = copy_or_zero(w.command, in->command, size_t(KBS_NUM_COMMANDS) * ld * 4, s))) return rc;
+  KBS_CUDA_TRY(cudaMemsetAsync(w.command + size_t(KBS_NUM_COMMANDS) * ld, 0, size_t(KBS_NUM_COMMANDS) * ld * 4, s));
+  if ((rc = copy_or_zero(w.lpf, in->lpf, size_t(KBS_NUM_JOINTS) * ld * 4, s))) return rc;
+  if ((rc = copy_or_zero(w.pg_carry, in->pg_carry, size_t(3) * ld * 4, s))) return rc;
+  float* carry[2] = {in->actor_carry, in->critic_carry};
+  for (int k = 0; k < (st->with_critic ? 2 : 1); ++k) {
+    if (h->p.gemm_path == KBS_GEMM_SIMT_FP32)
+      rc = copy_or_zero(w.carry[k], carry[k], size_t(h->p.depth) * 2 * n * h->p.hidden_size * 4, s);
+    else
+      rc = kbs_tc_step_carry(h, carry[k], w.tc[k], n, true, s);
+    if (rc) return rc;
+  }
+  return KBS_OK;
+}
+
+int kbs_step_state_store(kbs_handle* h, const kbs_step_state* st, const kbs_step_carry* out, void* stream) {
+  REQ(h);
+  StepState w;
+  int rc = step_state_at(h, st, &w);
+  if (rc || (rc = check_step_carry(st, out)) || (rc = kbs_enter(h))) return rc;
+  cudaStream_t s = (cudaStream_t)stream;
+  const int64_t n = st->n_envs, ld = round_up4(n);
+  auto copy = [&](void* dst, const void* src, size_t bytes) -> int {
+    if (dst) KBS_CUDA_TRY(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, s));
+    return KBS_OK;
+  };
+  if ((rc = copy(out->done_prev, w.done_prev, size_t(ld)))) return rc;
+  if ((rc = copy(out->command, w.command, size_t(KBS_NUM_COMMANDS) * ld * 4))) return rc;
+  if ((rc = copy(out->lpf, w.lpf, size_t(KBS_NUM_JOINTS) * ld * 4))) return rc;
+  if ((rc = copy(out->pg_carry, w.pg_carry, size_t(3) * ld * 4))) return rc;
+  float* carry[2] = {out->actor_carry, out->critic_carry};
+  for (int k = 0; k < (st->with_critic ? 2 : 1); ++k) {
+    if (!carry[k]) continue;
+    if (h->p.gemm_path == KBS_GEMM_SIMT_FP32)
+      rc = copy(carry[k], w.carry[k], size_t(h->p.depth) * 2 * n * h->p.hidden_size * 4);
+    else
+      rc = kbs_tc_step_carry(h, carry[k], w.tc[k], n, false, s);
+    if (rc) return rc;
+  }
+  return KBS_OK;
+}
+
+int kbs_step_state_rewind(kbs_handle* h, const kbs_step_state* st, void* stream) {
+  REQ(h);
+  StepState w;
+  if (const int rc = step_state_at(h, st, &w)) return rc;
+  KBS_CUDA_TRY(cudaMemsetAsync(&w.hdr->t, 0, sizeof(int64_t), (cudaStream_t)stream));
+  return KBS_OK;
+}
+
+int kbs_rollout_step(kbs_handle* h, const kbs_step_state* st, const kbs_step_io* io, void* stream) {
+  REQ(h); REQ(io);
+  StepState w;
+  int rc = step_state_at(h, st, &w);
+  if (rc) return rc;
+  const int64_t n = st->n_envs, ld = round_up4(n);
+  if (io->T <= 0) return KBS_E_SHAPE;
+  if ((rc = check_state(&io->state, n, true))) return rc;
+  if (io->state.ld != ld) return KBS_E_SHAPE;
+  if ((rc = kbs_enter(h))) return rc;
+  REQ(io->state.time); REQ(io->command); REQ(io->action); REQ(io->ctrl); REQ(io->done); REQ(io->success);
+  REQ(io->cmd_mode); REQ(io->cmd_u6); REQ(io->cmd_u_arms); REQ(io->u_switch);
+  if (io->value || io->critic_obs) { REQ(io->state.cinert); REQ(io->state.cvel); REQ(io->state.actuator_force); }
+  if (io->value && !st->with_critic) return KBS_E_PARAM;
+  if (!h->net[KBS_NET_ACTOR].packed || (io->value && !h->net[KBS_NET_CRITIC].packed)) return KBS_E_STATE;
+  if (io->noise.eps_jpos) { REQ(io->noise.eps_jvel); REQ(io->noise.eps_gyro); REQ(io->noise.eps_pg); }
+  AL(io->noise.eps_jpos); AL(io->noise.eps_jvel); AL(io->noise.eps_gyro); AL(io->noise.eps_pg);
+  AL(io->eps_action); AL(io->u_switch); AL(io->cmd_mode); AL(io->cmd_u6); AL(io->cmd_u_arms);
+  AL(io->command); AL(io->actor_obs); AL(io->critic_obs); AL(io->action); AL(io->log_prob); AL(io->ctrl); AL(io->term_codes);
+  AL(io->value);
+  if ((reinterpret_cast<uintptr_t>(io->done) & 3u) || (reinterpret_cast<uintptr_t>(io->success) & 3u)) return KBS_E_ALIGN;
+  // the recorded state: (step field, trajectory field, rows)
+  const kbs_state_view& a = io->state;
+  const kbs_state_view& b = io->traj_state;
+  const struct { const float* src; const float* dst; int rows; } rows[] = {
+      {a.qpos, b.qpos, KBS_NQ}, {a.qvel, b.qvel, KBS_NV}, {a.sensordata, b.sensordata, KBS_NSENSORDATA},
+      {a.xpos, b.xpos, 3 * KBS_NBODY}, {a.xquat, b.xquat, 4 * KBS_NBODY}, {a.cinert, b.cinert, 10 * KBS_NBODY},
+      {a.cvel, b.cvel, 6 * KBS_NBODY}, {a.actuator_force, b.actuator_force, KBS_NUM_JOINTS}, {a.com_distance, b.com_distance, 1},
+      {a.time, b.time, 1}};
+  for (const auto& r : rows) {
+    if (r.dst && !r.src) return KBS_E_NULL;
+    AL(r.dst);
+  }
+  cudaStream_t s = (cudaStream_t)stream;
+  const bool tc = h->p.gemm_path != KBS_GEMM_SIMT_FP32, critic = io->value != nullptr;
+
+  // this step's outputs in scratch (the rollout kernels' addressing stays that of a T = 1 call), then one record pass
+  float *aobs, *cobs, *action, *log_prob, *ctrl, *value;
+  int32_t* codes;
+  uint8_t *done, *success;
+  FusedTcWs tw;
+  SimtRolloutWs sw;
+  rc = kbs_scratch(h, [&](KbsScratch& sc) {
+    aobs = sc.take<float>(size_t(KBS_ACTOR_OBS) * ld);
+    cobs = io->critic_obs ? sc.take<float>(size_t(KBS_CRITIC_OBS) * ld) : nullptr;
+    action = sc.take<float>(size_t(KBS_NUM_JOINTS) * ld);
+    log_prob = sc.take<float>(size_t(ld));
+    ctrl = sc.take<float>(size_t(KBS_NUM_JOINTS) * ld);
+    value = critic ? sc.take<float>(size_t(ld)) : nullptr;
+    codes = io->term_codes ? sc.take<int32_t>(size_t(3) * ld) : nullptr;
+    done = sc.take<uint8_t>(size_t(ld));
+    success = sc.take<uint8_t>(size_t(ld));
+    if (tc) tw = fused_tc_ws(sc, h, n, ld, 1, 1, critic, true, true, io->critic_obs != nullptr);
+    else sw = simt_rollout_ws(sc, h, n, ld);
+  });
+  if (rc) return rc;
+  kbs_rollout_io r1{};
+  r1.state = io->state; r1.noise = io->noise; r1.episode = io->episode;
+  r1.eps_action = io->eps_action; r1.u_switch = io->u_switch; r1.cmd_mode = io->cmd_mode; r1.cmd_u6 = io->cmd_u6;
+  r1.cmd_u_arms = io->cmd_u_arms;
+  r1.command = w.command; r1.pg_carry = w.pg_carry; r1.lpf = w.lpf;
+  r1.actor_carry = w.carry[0]; r1.critic_carry = w.carry[1];          // SIMT; the tensor-core kernels read w.tc in place
+  r1.actor_obs = aobs; r1.action = action; r1.log_prob = log_prob; r1.ctrl = ctrl; r1.term_codes = codes;
+  r1.done = done; r1.success = success; r1.value = value; r1.T = 1;
+  if (tc) {
+    KbsTcRolloutArgs res{};
+    for (int k = 0; k < 2; ++k) { res.res_hsb[k] = w.tc[k].hsb; res.res_fb[k] = w.tc[k].fb; }
+    res.res_hsb_slot = &w.hdr->hsb_slot;
+    rc = rollout_fused_tc(h, &r1, w.done_prev, cobs, tw, 1, &res, n, s);
+  } else {
+    rc = rollout_simt(h, &r1, w.done_prev, cobs, sw, n, s, /*one_step=*/true);
+  }
+  if (rc) return rc;
+
+  KbsStepRecord R{};
+  int j = 0;
+  auto job = [&](const void* src, void* dst, int64_t words) {
+    if (!dst) return;
+    R.job[j].src = src; R.job[j].dst = dst; R.job[j].words = words; R.job[j].dst_step = words; ++j;
+  };
+  job(aobs, io->actor_obs, KBS_ACTOR_OBS * ld);
+  job(cobs, io->critic_obs, KBS_CRITIC_OBS * ld);
+  job(action, io->action, KBS_NUM_JOINTS * ld);
+  job(log_prob, io->log_prob, ld);
+  job(ctrl, io->ctrl, KBS_NUM_JOINTS * ld);
+  job(value, io->value, ld);
+  job(codes, io->term_codes, 3 * ld);
+  job(done, io->done, ld / 4);
+  job(success, io->success, ld / 4);
+  for (const auto& rr : rows) job(rr.src, const_cast<float*>(rr.dst), rr.rows * ld);
+  job(done, w.done_prev, ld / 4);
+  R.job[j - 1].dst_step = 0;                                           // done_prev: no time axis
+  R.job[j].src = w.command; R.job[j].dst = io->command; R.job[j].words = KBS_NUM_COMMANDS * ld;
+  R.job[j].dst_step = KBS_NUM_COMMANDS * ld; R.job[j].shift = 1; ++j;
+  R.jobs = j;
+  R.T = io->T; R.t = &w.hdr->t; R.hsb_slot = tc ? &w.hdr->hsb_slot : nullptr; R.ticket = &w.hdr->ticket;
+  if ((rc = kbs_status_init(h))) return rc;
+  R.status = h->persist_status;
+  if ((rc = kbs_launch_step_record(h, R, s))) return rc;
+  return kbs_status_publish(h, s);
 }
 
 }  // extern "C"

@@ -48,7 +48,7 @@ enum KbsKernelId {
   KBS_K_OBS = 0, KBS_K_COMMAND, KBS_K_TORQUE, KBS_K_TERMINATE, KBS_K_REWARD_ROT, KBS_K_REWARD_TERMS, KBS_K_REWARD_SCAN,
   KBS_K_GAE, KBS_K_ADV_NORM, KBS_K_POLICY_IO, KBS_K_GEMM_SIMT, KBS_K_LSTM_CELL, KBS_K_ACTOR_HEAD, KBS_K_CRITIC_HEAD,
   KBS_K_PACK, KBS_K_LSTM_TC, KBS_K_PROJ_TC, KBS_K_ROLLOUT_TC, KBS_K_BPTT_TC, KBS_K_GEMM_TN, KBS_K_PACK_TN, KBS_K_TN_REDUCE,
-  KBS_K_PERMUTATION, KBS_K_SHUFFLE, KBS_K_COUNT
+  KBS_K_STEP_RECORD, KBS_K_PERMUTATION, KBS_K_SHUFFLE, KBS_K_COUNT
 };
 static_assert(KBS_K_COUNT == KBS_NUM_KERNEL_IDS, "kbotstep.h KBS_NUM_KERNEL_IDS");
 constexpr int kKbsProfMaxPairs = 8192;
@@ -142,7 +142,8 @@ int kbs_scratch(kbs_handle* h, Layout&& layout) {
 int kbs_launch_observations(kbs_handle* h, const kbs_state_view& s, const kbs_noise_view* nz,
                             const kbs_episode_view* ep, const float* command, float* pg_carry,
                             const uint8_t* pg_reset, float* computed, float* actor_obs, float* critic_obs, int64_t n,
-                            cudaStream_t st, int64_t T = 1, const float* pg_lagged = nullptr, bool skip_dump = false);
+                            cudaStream_t st, int64_t T = 1, const float* pg_lagged = nullptr, bool skip_dump = false,
+                            bool one_step = false);   // one_step (T = 1): the launch shape of kbs_rollout_step
 int kbs_launch_ppo_loss(kbs_handle* h, const kbs_ppo_loss_params& L, const kbs_ppo_loss_io& io, int64_t n, cudaStream_t st);
 int kbs_launch_ppo_loss_at(kbs_handle* h, const kbs_ppo_loss_params& L, const kbs_ppo_loss_io& io, int64_t n, double* partials,
                            cudaStream_t st);
@@ -185,6 +186,15 @@ int kbs_launch_policy_pack(kbs_handle* h, const float* ja, const float* jv, cons
                            int64_t ld, int64_t n, cudaStream_t st);
 int kbs_launch_policy_unpack(kbs_handle* h, const float* carry_aos, const float* lpf_soa, const float* mean_soa,
                              float* carry_out, float* action_out, int64_t ld, int64_t n, cudaStream_t st);
+// the online step's record into slot t (kbs_rollout_step): jobs of 32-bit words, dst advanced by t * dst_step words;
+// shift = the command job (src = the state's [2][16][ld] rows, words = 16 ld; dst = the [T+1] trajectory)
+struct KbsStepJob { const void* src; void* dst; int64_t words, dst_step; int shift, block0; };
+constexpr int kKbsStepMaxJobs = 24;
+struct KbsStepRecord {
+  KbsStepJob job[kKbsStepMaxJobs]; int jobs;
+  int64_t T; int64_t* t; int* hsb_slot; unsigned int* ticket; unsigned int* status;
+};
+int kbs_launch_step_record(kbs_handle* h, KbsStepRecord a, cudaStream_t st);
 // kbs_ppo_update.cu: the update phase's minibatch construction (arguments validated by the entry points in kbs_api.cu)
 int kbs_launch_minibatch_permutation(kbs_handle* h, uint64_t seed, int64_t* pass_dev, int64_t env0, int32_t* perm, int64_t n,
                                      cudaStream_t st);
@@ -247,9 +257,17 @@ struct KbsTcRolloutArgs {
   int save;
   char* xmid_hist[2]; char* hsb_hist[2]; float* c_hist[2]; float* save_g[2]; float* sraw;
   KbsTcRolloutWs ws;          // kbs_tc_rollout_ws for (with_critic ? 2 : 1) nets
+  // res_hsb_slot != nullptr (kbs_rollout_step, T = 1, persistent kernel only): the carries are resident in a step state in
+  // the kernel's own layouts -- per net hsb [depth][2] x sb and fb [depth][c, h] x np*H, and the device word naming the hsb
+  // slot this launch reads -- so nothing is converted on either side; carry[] is not read
+  char* res_hsb[2]; float* res_fb[2]; const int* res_hsb_slot;
   int64_t chunk_len;          // > 0: before step t with t % chunk_len == 0, wait for chunk_events[t / chunk_len]
   cudaEvent_t* chunk_events;  //      (the input projections of that chunk of steps, produced on another stream)
 };
+// the online step's resident carries of one net (kbs_net_tc.cu): pieces of the caller's step state, carved like scratch
+struct KbsTcStepNet { char* hsb; float* fb; };
+KbsTcStepNet kbs_tc_step_net(KbsScratch& s, const kbs_handle* h, int64_t n);
+int kbs_tc_step_carry(kbs_handle* h, float* carry, const KbsTcStepNet& w, int64_t n, bool to_state, cudaStream_t st);
 int64_t kbs_tc_sb_floats(const kbs_handle* h, int64_t n);
 int64_t kbs_tc_obs_sb_floats(const kbs_handle* h, int net, int64_t n, int64_t T);
 // cinert / cvel != nullptr: the critic's privileged dump (features 80..447) is read from the recorded state

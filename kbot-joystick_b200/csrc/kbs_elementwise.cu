@@ -68,9 +68,23 @@ __device__ __forceinline__ void encode_pg(const float (&g)[3], float (&o)[5]) {
 // observations: get_observations table + run_actor / run_critic concats.
 // train.py:1155-1204, 682-707, 1329-1431.  grid = (env groups, 1 + copy sections).
 // =====================================================================================================
-constexpr int kCopyRowsPerSection = 46;  // 368 pure-copy rows (cinert 230 + cvel 138) in 8 sections
-constexpr int kObsSections = 4;          // computed rows of one env-step in 4 sections (see obs_kernel)
+// Sections of obs_kernel.  The trajectory form (T steps per launch): joints in 2 sections, IMU + command in one, feet + the
+// critic's small copies in one, then the 368 pure-copy rows (cinert 230 + cvel 138) in 8 sections.  The one-step form
+// (kbs_rollout_step: a few thousand envs, one step per launch) cuts the same rows 6x finer -- one joint per section, the command
+// apart from the IMU, 8 copy rows per section -- so one step fills the SMs instead of running on a few blocks per SM.
+template <bool ONE_STEP> struct ObsSections {
+  static constexpr int kJoint = ONE_STEP ? 20 : 2;           // joint sections, KBS_NUM_JOINTS / kJoint joints each
+  static constexpr int kImu = kJoint;
+  static constexpr int kCmd = ONE_STEP ? kImu + 1 : kImu;     // the trajectory form does both in one section
+  static constexpr int kFeet = kCmd + 1;
+  static constexpr int kComputed = kFeet + 1;                 // sections before the copy sections
+  static constexpr int kCopyRows = ONE_STEP ? 8 : 46;
+  static constexpr int kCopy = 368 / kCopyRows;
+};
+constexpr int kCopyRowsPerSection = 46;  // mirror_obs_kernel's copy sections (the trajectory form's)
+static_assert(368 % ObsSections<true>::kCopyRows == 0 && 368 % ObsSections<false>::kCopyRows == 0, "copy sections");
 
+template <bool ONE_STEP>
 __global__ void __launch_bounds__(kThreads)
 obs_kernel(const __grid_constant__ kbs_params P, kbs_state_view s, kbs_noise_view nz,
            const kbs_episode_view ep, const float* __restrict__ command, float* __restrict__ pg_carry,
@@ -94,15 +108,16 @@ obs_kernel(const __grid_constant__ kbs_params P, kbs_state_view s, kbs_noise_vie
     if (critic_obs) critic_obs += t * KBS_CRITIC_OBS * ld;
   }
 
-  // blockIdx.y = section: the rows of one env-step are independent, so they are spread over kObsSections x as many
-  // threads (one thread doing all ~250 rows of its 4 envs left 21 warps per SM and 2.4 TB/s).
+  // blockIdx.y = section: the rows of one env-step are independent, so they are spread over the sections x as many
+  // threads (one thread doing all ~250 rows of its 4 envs left 21 warps per SM and 2.4 TB/s).  Trajectory form:
   //   0 / 1: joints 0-9 / 10-19   2: IMU + command slots   3: feet positions + the critic's small copies   4..: dump
+  using S = ObsSections<ONE_STEP>;
   const int sec = blockIdx.y;
-  if (sec >= kObsSections) {
+  if (sec >= S::kComputed) {
     // critic privileged dump: center_of_mass_inertia = cinert[1:], center_of_mass_velocity = cvel[1:]
-    const int i0 = (sec - kObsSections) * kCopyRowsPerSection;
+    const int i0 = (sec - S::kComputed) * S::kCopyRows;
 #pragma unroll 8
-    for (int i = i0; i < i0 + kCopyRowsPerSection; ++i) {
+    for (int i = i0; i < i0 + S::kCopyRows; ++i) {
       if (i < 230) kbs_copy4(s.cinert, 10 + i, critic_obs, 80 + i, ld, n0);
       else if (i < 368) kbs_copy4(s.cvel, 6 + (i - 230), critic_obs, 310 + (i - 230), ld, n0);
     }
@@ -112,9 +127,10 @@ obs_kernel(const __grid_constant__ kbs_params P, kbs_state_view s, kbs_noise_vie
   const bool has_noise = nz.eps_jpos != nullptr;
 
   // joints: slots 0-19 / 20-39
-  if (sec < 2) {
+  if (sec < S::kJoint) {
+  constexpr int kPer = KBS_NUM_JOINTS / S::kJoint;
 #pragma unroll 5
-  for (int j = sec * 10; j < sec * 10 + 10; ++j) {
+  for (int j = sec * kPer; j < sec * kPer + kPer; ++j) {
     float q[4], qd[4], jb[4] = {0, 0, 0, 0}, e1[4] = {0, 0, 0, 0}, e2[4] = {0, 0, 0, 0};
     kbs_ld4(s.qpos, 7 + j, ld, n0, q);
     kbs_ld4(s.qvel, 6 + j, ld, n0, qd);
@@ -139,7 +155,7 @@ obs_kernel(const __grid_constant__ kbs_params P, kbs_state_view s, kbs_noise_vie
   }
 
   // IMU: projected gravity (clean + lagged/biased/noisy twin) and gyro
-  if (sec == 2) {
+  if (sec == S::kImu) {
     float iq[4][4], gy[3][4];
 #pragma unroll
     for (int k = 0; k < 4; ++k) kbs_ld4(s.sensordata, P.sd_imu_quat + k, ld, n0, iq[k]);
@@ -201,10 +217,11 @@ obs_kernel(const __grid_constant__ kbs_params P, kbs_state_view s, kbs_noise_vie
       for (int k = 0; k < 5; ++k) kbs_st4(critic_obs, 40 + k, ld, n0, enc_c[k]);
       for (int k = 0; k < 3; ++k) kbs_st4(critic_obs, 45 + k, ld, n0, gy[k]);
     }
+    if (S::kCmd != S::kImu) return;
   }
 
   // zero_cmd flag + command: slots 48, 49-64
-  if (sec == 2) {
+  if (sec == S::kCmd) {
   float c[16][4];
 #pragma unroll
   for (int k = 0; k < 16; ++k) kbs_ld4(command, k, ld, n0, c[k]);
@@ -1399,15 +1416,23 @@ inline unsigned groups4(int64_t n) { return unsigned((((n + 3) / 4) + kThreads -
 int kbs_launch_observations(kbs_handle* h, const kbs_state_view& s, const kbs_noise_view* nz,
                             const kbs_episode_view* ep, const float* command, float* pg_carry,
                             const uint8_t* pg_reset, float* computed, float* actor_obs, float* critic_obs, int64_t n,
-                            cudaStream_t st, int64_t T, const float* pg_lagged, bool skip_dump) {
+                            cudaStream_t st, int64_t T, const float* pg_lagged, bool skip_dump, bool one_step) {
   kbs_noise_view z{};
   kbs_episode_view e{};
   if (nz) z = *nz;
   if (ep) e = *ep;
   // skip_dump: the caller reads cinert / cvel straight from the state (critic rows 80..447 stay unwritten)
-  dim3 grid(groups4(n), (critic_obs && !skip_dump) ? kObsSections + 368 / kCopyRowsPerSection : kObsSections, unsigned(T));
-  KBS_LAUNCH(h, KBS_K_OBS, st, (obs_kernel<<<grid, kThreads, 0, st>>>(h->p, s, z, e, command, pg_carry, pg_reset, pg_lagged,
-                                                                      computed, actor_obs, critic_obs, n)));
+  if (one_step && T == 1) {
+    using S = ObsSections<true>;
+    dim3 grid(groups4(n), (critic_obs && !skip_dump) ? S::kComputed + S::kCopy : S::kComputed, 1u);
+    KBS_LAUNCH(h, KBS_K_OBS, st, (obs_kernel<true><<<grid, kThreads, 0, st>>>(h->p, s, z, e, command, pg_carry, pg_reset,
+                                                                            pg_lagged, computed, actor_obs, critic_obs, n)));
+  } else {
+    using S = ObsSections<false>;
+    dim3 grid(groups4(n), (critic_obs && !skip_dump) ? S::kComputed + S::kCopy : S::kComputed, unsigned(T));
+    KBS_LAUNCH(h, KBS_K_OBS, st, (obs_kernel<false><<<grid, kThreads, 0, st>>>(h->p, s, z, e, command, pg_carry, pg_reset,
+                                                                             pg_lagged, computed, actor_obs, critic_obs, n)));
+  }
   KBS_LAUNCH_CHECK();
   return KBS_OK;
 }
@@ -1624,6 +1649,67 @@ int kbs_launch_policy_unpack(kbs_handle* h, const float* carry_aos, const float*
   KBS_LAUNCH(h, KBS_K_POLICY_IO, st,
              (policy_unpack_kernel<<<unsigned((n + kThreads - 1) / kThreads), kThreads, 0, st>>>(
                  lpf_soa, mean_soa, carry_out, cw, action_out, ld, n)));
+  KBS_LAUNCH_CHECK();
+  return KBS_OK;
+}
+
+// ---- the online step's record (kbs_rollout_step) -------------------------------------------------------------------------
+// Moves one step's outputs into slot t of the caller's trajectories, t read from the step state, in one pass: every job is a
+// contiguous run of 32-bit words (a [F][ld] block; done / success are ld bytes), copied as float4 where both ends are 16-byte
+// aligned.  The command job also shifts the state's next-command rows into its current rows.  The last block to finish
+// advances t and flips the state's hsb slot word, so a captured launch serves every step.
+namespace {
+constexpr int kStepWordsPerBlock = 4096;
+__global__ void __launch_bounds__(256) step_record_kernel(const __grid_constant__ KbsStepRecord a) {
+  __shared__ int64_t t_s;
+  if (threadIdx.x == 0) t_s = *reinterpret_cast<volatile int64_t*>(a.t);
+  __syncthreads();
+  const int64_t t = t_s;
+  const bool in_range = t >= 0 && t < a.T;
+  if (in_range) {
+    int j = 0;
+    while (j + 1 < a.jobs && int(blockIdx.x) >= a.job[j + 1].block0) ++j;
+    const KbsStepJob& J = a.job[j];
+    const int64_t w0 = int64_t(blockIdx.x - J.block0) * kStepWordsPerBlock;
+    const int64_t w1 = w0 + kStepWordsPerBlock < J.words ? w0 + kStepWordsPerBlock : J.words;
+    const uint32_t* src = static_cast<const uint32_t*>(J.src);
+    uint32_t* dst = static_cast<uint32_t*>(J.dst) + t * J.dst_step;
+    if (J.shift) {        // command: state rows [0] -> traj[t], [1] -> traj[t + 1] and -> state rows [0]
+      uint32_t* cs = const_cast<uint32_t*>(src);
+      for (int64_t w = w0 + threadIdx.x; w < w1; w += blockDim.x) {
+        const uint32_t c0 = cs[w], c1 = cs[J.words + w];
+        dst[w] = c0; dst[J.dst_step + w] = c1; cs[w] = c1;
+      }
+    } else if (((reinterpret_cast<uintptr_t>(src) | reinterpret_cast<uintptr_t>(dst)) & 15u) == 0 && (J.words & 3) == 0) {
+      const uint4* s4 = reinterpret_cast<const uint4*>(src);
+      uint4* d4 = reinterpret_cast<uint4*>(dst);
+      for (int64_t q = w0 / 4 + threadIdx.x; q < w1 / 4; q += blockDim.x) __stcs(d4 + q, __ldcs(s4 + q));
+    } else {
+      for (int64_t w = w0 + threadIdx.x; w < w1; w += blockDim.x) dst[w] = src[w];
+    }
+  } else if (blockIdx.x == 0 && threadIdx.x == 0) {
+    atomicOr(a.status, unsigned(KBS_STATUS_STEP_RANGE));
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    __threadfence();
+    if (atomicAdd(a.ticket, 1u) == gridDim.x - 1) {       // every block has read t
+      *a.ticket = 0u;
+      if (in_range) *a.t = t + 1;
+      if (a.hsb_slot) *a.hsb_slot ^= 1;
+      __threadfence();
+    }
+  }
+}
+}  // namespace
+
+int kbs_launch_step_record(kbs_handle* h, KbsStepRecord a, cudaStream_t st) {
+  int blocks = 0;
+  for (int j = 0; j < a.jobs; ++j) {
+    a.job[j].block0 = blocks;
+    blocks += int((a.job[j].words + kStepWordsPerBlock - 1) / kStepWordsPerBlock);
+  }
+  KBS_LAUNCH(h, KBS_K_STEP_RECORD, st, (step_record_kernel<<<unsigned(blocks), 256, 0, st>>>(a)));
   KBS_LAUNCH_CHECK();
   return KBS_OK;
 }

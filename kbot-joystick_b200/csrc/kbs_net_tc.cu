@@ -759,7 +759,8 @@ struct PNet {
                                    // the packed observations themselves (kb_x0 = padded input width / block K)
   size_t x0_stride;                // bytes per step of x_sb_all
   int kb_x0;                       // K blocks of the layer-0 input operand
-  char* hsb;                       // [depth][2] x sbb: recurrent SB state (reset where done); step t reads parity t & 1
+  char* hsb;                       // [depth][2] x sbb: recurrent SB state (reset where done); step t reads parity
+                                   // (t + *hsb_slot) & 1
   char* xmid;                      // [depth][2] x sbb: un-reset SB output of layer l at step t (parity t & 1)
   float* fb;                       // [depth][c, h] x np*H: fp32 FB state
   const char* w_sb[kPMaxDepth];
@@ -794,6 +795,9 @@ struct PArgs {
   int hist;                        // 1 = SAVE instantiation: per-step buffers, no write-after-read dependencies
   int dbg;                         // profiling only (KBS_PERSIST_DBG): 1 = ignore dependencies (wrong results, timing probe)
   unsigned int* status;            // != 0: a dependency wait timed out (bug / lost CTA)
+  const int* hsb_slot;             // device 0 / 1 or nullptr (= 0): the hsb slot step 0 reads.  The online step (T = 1,
+                                   // kbs_rollout_step) keeps hsb resident and flips this word after every launch, so a
+                                   // replayed launch finds its input where the previous one left it
   long long* trace;                // per CTA [8]: total cycles, poller wait cycles, items, issuer wait-for-stage cycles,
                                    // epilogue cycles in LSTM / head items, epilogue wait-for-accumulator, issuer wait-for-TMEM
 };
@@ -891,6 +895,7 @@ rollout_persist_kernel(const __grid_constant__ kbs_params P, const __grid_consta
   const int per_slot = args.nets * args.gpanels * (args.depth * args.tiles + 1);
   const int n_g = ((args.panels + args.gpanels - 1) / args.gpanels) * (int(args.T) + args.depth) * per_slot;
   const int H = args.H;
+  const int hslot = (!SAVE && args.hsb_slot) ? *args.hsb_slot : 0;
   constexpr int kBlk = kbs_block_k(KIND);
   const int kb = H / kBlk;
   long long* tr = args.trace ? args.trace + size_t(blockIdx.x) * 16 : nullptr;
@@ -971,7 +976,7 @@ rollout_persist_kernel(const __grid_constant__ kbs_params P, const __grid_consta
         const char* xa; const char* ha; const char* wb;
         if (it.kind == 0) {
           const size_t xs = SAVE ? size_t(it.layer - 1) * size_t(args.T) + size_t(it.t) : size_t((it.layer - 1) * 2 + (it.t & 1));
-          const size_t hs = SAVE ? size_t(it.layer) * size_t(args.T + 1) + size_t(it.t) : size_t(it.layer * 2 + (it.t & 1));
+          const size_t hs = SAVE ? size_t(it.layer) * size_t(args.T + 1) + size_t(it.t) : size_t(it.layer * 2 + ((it.t + hslot) & 1));
           xa = it.layer == 0 ? N.x_sb_all + size_t(it.t) * N.x0_stride + poff / kb * kb_x : N.xmid + xs * args.sbb + poff;
           ha = N.hsb + hs * args.sbb + poff;
           wb = N.w_sb[it.layer] + size_t((args.dbg & 16) ? (blockIdx.x + it.t) % args.tiles : it.tile) * kb_total * kBBlockBytesP;
@@ -1144,7 +1149,7 @@ rollout_persist_kernel(const __grid_constant__ kbs_params P, const __grid_consta
         if (live && !(args.dbg & 2)) {
           char* x_out = N.xmid + (SAVE ? size_t(it.layer) * size_t(args.T) + size_t(it.t) : size_t(it.layer * 2 + (it.t & 1))) * args.sbb;
           char* h_out = N.hsb + (SAVE ? size_t(it.layer) * size_t(args.T + 1) + size_t(it.t + 1)
-                                      : size_t(it.layer * 2 + ((it.t + 1) & 1))) * args.sbb;
+                                      : size_t(it.layer * 2 + ((it.t + 1 + hslot) & 1))) * args.sbb;
           float* h_carry = (!SAVE && it.t == int(args.T) - 1) ? cst + npH : nullptr;
           // 8 hidden units = exactly one 16-byte SB chunk per plane (FP16 kind): every store below is a full 16 B per
           // lane, 512 contiguous bytes per warp (8-byte half-chunk stores cost the operand pipeline 2.5 K cycles per item)
@@ -4077,11 +4082,16 @@ int kbs_tc_rollout_recurrent(kbs_handle* h, const KbsTcRolloutArgs& r, cudaStrea
   const int64_t n = r.n, ld = r.ld, np = pad_rows(n);
   const size_t sbb = act_sb_bytes(h, n);
   char* hsb[2] = {r.ws.hsb[0], r.ws.hsb[1]}; char* xmid[2] = {r.ws.xmid[0], r.ws.xmid[1]};
-  float* const* h2rm = r.ws.h2rm; float* const* fb = r.ws.fb; unsigned int* const* flags = r.ws.flags;
+  float* const* h2rm = r.ws.h2rm; float* fb[2] = {r.ws.fb[0], r.ws.fb[1]}; unsigned int* const* flags = r.ws.flags;
   const size_t fbf = size_t(np) * H;
+  const bool resident = r.res_hsb_slot != nullptr;
   const char* legacy_env = getenv("KBS_TC_PER_STEP");          // A/B and cross-check against the per-step launches
-  const int legacy = (legacy_env && !r.save) ? atoi(legacy_env) : 0;
+  const int legacy = (legacy_env && !r.save && !resident) ? atoi(legacy_env) : 0;
   const bool persistent = !legacy && kbs_tc_persistent_available(h, n, r.T, nets);
+  if (resident) {                                              // the step state's own operands: nothing to convert
+    if (!persistent || r.save || r.carry_ld) return KBS_E_SHAPE;
+    for (int k = 0; k < nets; ++k) { hsb[k] = r.res_hsb[k]; fb[k] = r.res_fb[k]; }
+  }
   if (r.save) {                                                // forward pass of the PPO update: per-step history buffers
     if (!persistent || kind != KBS_KIND_F16 || r.carry_ld) return KBS_E_STATE;
     for (int k = 0; k < nets; ++k) { hsb[k] = r.hsb_hist[k]; xmid[k] = r.xmid_hist[k]; }
@@ -4091,7 +4101,9 @@ int kbs_tc_rollout_recurrent(kbs_handle* h, const KbsTcRolloutArgs& r, cudaStrea
   if (r.mean && !persistent) return KBS_E_STATE;                                   // dist.mean() output: persistent kernel only
   if (r.carry_ld && (!persistent || nets * depth * 2 > 8 || H % 8)) return KBS_E_STATE;   // flat carries: persistent kernel only
   const size_t slot_f = r.carry_ld ? size_t(H) : size_t(n) * H;                  // floats between carry slots
-  if (nets * depth * 2 <= 8 && H % 8 == 0) {                       // ABI carry: h -> SB (parity 0), c -> FB; one launch
+  if (resident) {
+    // read in place: the h slot the last step wrote, the fp32 c it left
+  } else if (nets * depth * 2 <= 8 && H % 8 == 0) {                // ABI carry: h -> SB (parity 0), c -> FB; one launch
     CarryJobs J{};
     J.ld_rm = r.carry_ld ? r.carry_ld : H;
     J.status = h->persist_status;
@@ -4159,6 +4171,7 @@ int kbs_tc_rollout_recurrent(kbs_handle* h, const KbsTcRolloutArgs& r, cudaStrea
     a.action_in = r.action_in; a.entropy = r.entropy; a.std = r.action_std; a.mean = r.mean;
     a.sraw = r.save ? r.sraw : nullptr; a.hist = r.save ? 1 : 0;
     a.status = h->persist_status;
+    a.hsb_slot = r.res_hsb_slot;
     { const char* e = getenv("KBS_PERSIST_DBG"); a.dbg = e ? atoi(e) : 0; }
     a.trace = h->trace_buf;
     cudaLaunchConfig_t cfg{};
@@ -4182,7 +4195,8 @@ int kbs_tc_rollout_recurrent(kbs_handle* h, const KbsTcRolloutArgs& r, cudaStrea
       KBS_LAUNCH(h, KBS_K_ROLLOUT_TC, st, (le = cudaLaunchKernelEx(&cfg, rollout_persist_kernel<KBS_KIND_F16, false>, h->p, a)));
     KBS_CUDA_TRY(le);
     { const int rc0 = kbs_status_publish(h, st); if (rc0) return rc0; }
-    if (r.save) { KBS_LAUNCH_CHECK(); return KBS_OK; }       // the update does not need the final carries
+    if (r.save || resident) { KBS_LAUNCH_CHECK(); return KBS_OK; }   // the update does not need the final carries; the
+                                                                      // online step leaves them in its state
     if (nets * depth * 2 <= 8 && H % 8 == 0) {                       // FB state -> ABI carry; one launch
       CarryJobs J{};
       J.ld_rm = r.carry_ld ? r.carry_ld : H;
@@ -4300,6 +4314,52 @@ int kbs_tc_debug_trace(kbs_handle* h, long long* trace_out, const KbsTcRolloutWs
     a.panels = int(np / kPanelRows);
   }
   KBS_LAUNCH(h, KBS_K_LSTM_TC, st, (launch_layer(h, tc_kind(h), a2, st)));
+  KBS_LAUNCH_CHECK();
+  return KBS_OK;
+}
+
+// ---- the online step's resident carries (kbs_step_state_*, kbs_rollout_step) -----------------------------------------------
+// One net's piece of a step state: hsb [depth][2] x act SB (the h operand; the state's slot word names the one the next step
+// reads) and fb [depth][c, h] x np*H (the fp32 cell state, and the fp32 h the last step wrote).
+KbsTcStepNet kbs_tc_step_net(KbsScratch& s, const kbs_handle* h, int64_t n) {
+  const size_t depth = size_t(h->p.depth), H = size_t(h->p.hidden_size), np = size_t(pad_rows(n));
+  KbsTcStepNet w;
+  w.hsb = s.take<char>(2 * depth * act_sb_bytes(h, n));
+  w.fb = s.take<float>(2 * depth * np * H);
+  return w;
+}
+
+// ABI carry [depth][2][n][H] <-> one net's resident operands.  to_state: h -> hsb slot 0 (split) and fb h, c -> fb c
+// (carry == nullptr: zeros); else fb c / fb h -> the ABI c / h (what kbs_tc_rollout_recurrent writes back after a call).
+int kbs_tc_step_carry(kbs_handle* h, float* carry, const KbsTcStepNet& w, int64_t n, bool to_state, cudaStream_t st) {
+  const int H = h->p.hidden_size, depth = h->p.depth;
+  const int64_t np = pad_rows(n);
+  const size_t sbb = act_sb_bytes(h, n), fbf = size_t(np) * H;
+  { const int rc0 = kbs_status_init(h); if (rc0) return rc0; }
+  if (to_state) {
+    KBS_CUDA_TRY(cudaMemsetAsync(w.hsb, 0, 2 * size_t(depth) * sbb, st));
+    if (!carry) { KBS_CUDA_TRY(cudaMemsetAsync(w.fb, 0, 2 * size_t(depth) * fbf * sizeof(float), st)); return KBS_OK; }
+  }
+  CarryJobs J{};
+  J.ld_rm = H;
+  J.status = to_state ? h->persist_status : nullptr;
+  int j = 0;
+  for (int l = 0; l < depth; ++l) {
+    float* hrm = carry + (size_t(l) * 2 + 0) * size_t(n) * H;
+    float* crm = carry + (size_t(l) * 2 + 1) * size_t(n) * H;
+    if (to_state) {
+      J.rm[j] = hrm; J.blk[j] = w.hsb + sbb * (2 * l); J.mode[j++] = 0;
+      J.rm[j] = hrm; J.blk[j] = w.fb + fbf * (2 * l + 1); J.mode[j++] = 1;
+      J.rm[j] = crm; J.blk[j] = w.fb + fbf * (2 * l); J.mode[j++] = 1;
+    } else {
+      J.rm[j] = crm; J.blk[j] = w.fb + fbf * (2 * l); J.mode[j++] = 2;
+      J.rm[j] = hrm; J.blk[j] = w.fb + fbf * (2 * l + 1); J.mode[j++] = 2;
+    }
+    if (j > 5 || l + 1 == depth) {         // at most 8 jobs per launch
+      if (const int rc = carry_convert(h, J, j, n, np, H, st)) return rc;
+      j = 0;
+    }
+  }
   KBS_LAUNCH_CHECK();
   return KBS_OK;
 }

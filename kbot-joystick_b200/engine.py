@@ -470,3 +470,55 @@ class KbotStep:
             return
         rec = L.KbsRolloutRecord(L.ptr(io.get("done_prev")), L.ptr(io.get("critic_obs")))
         L.check(self.lib.kbs_rollout_record(self._h, C.byref(r), C.byref(rec), n_envs, _stream()), "kbs_rollout_record")
+
+    # ---- the online rollout: one control step per call ----------------------------------------------------------------------
+    def step_state(self, n_envs: int, with_critic: bool = True, carry: dict | None = None) -> "StepState":
+        """A device step state for n_envs (kbs_step_state): the carries in the kernels' own layouts, lpf, pg_carry, the command,
+        done_prev and the step index, loaded from `carry` (see step_state_load; None = zeros)."""
+        nb = C.c_uint64(0)
+        L.check(self.lib.kbs_step_state_bytes(self._h, n_envs, 1 if with_critic else 0, C.byref(nb)), "kbs_step_state_bytes")
+        buf = torch.empty((int(nb.value),), dtype=torch.uint8, device=torch.device("cuda", torch.cuda.current_device()))
+        st = StepState(buf, L.KbsStepState(buf.data_ptr(), int(nb.value), n_envs, 1 if with_critic else 0))
+        self.step_state_load(st, carry or {})
+        return st
+
+    def step_state_load(self, st: "StepState", carry: dict) -> None:
+        """carry: any of actor_carry / critic_carry [depth,2,n,H], lpf [20,ld], pg_carry [3,ld], command [16,ld], done_prev u8
+        [ld] (missing = zeros).  The step index becomes 0."""
+        c = L.KbsStepCarry(*(L.ptr(carry.get(k)) for k, _ in L.KbsStepCarry._fields_))
+        L.check(self.lib.kbs_step_state_load(self._h, C.byref(st.desc), C.byref(c), _stream()), "kbs_step_state_load")
+
+    def step_state_store(self, st: "StepState", out: dict) -> dict:
+        """Write the state's carries into the tensors of `out` (same keys as step_state_load; missing = not written)."""
+        c = L.KbsStepCarry(*(L.ptr(out.get(k)) for k, _ in L.KbsStepCarry._fields_))
+        L.check(self.lib.kbs_step_state_store(self._h, C.byref(st.desc), C.byref(c), _stream()), "kbs_step_state_store")
+        return out
+
+    def step_state_rewind(self, st: "StepState") -> None:
+        """Step index back to 0; nothing else changes."""
+        L.check(self.lib.kbs_step_state_rewind(self._h, C.byref(st.desc), _stream()), "kbs_step_state_rewind")
+
+    def rollout_step(self, st: "StepState", io: dict) -> None:
+        """One control step (kbs_rollout_step).  io: state / noise / episode (dicts of this step's [F, ld] tensors), eps_action,
+        u_switch, cmd_mode, cmd_u6, cmd_u_arms of this step; trajectories command [T+1,16,ld], actor_obs, critic_obs, action,
+        log_prob, ctrl, term_codes, done, success, value ([T, ..., ld]; optional ones may be missing or None) and traj_state
+        (dict of [T, F, ld] tensors recording this step's state fields).  Slot t = the state's device step index."""
+        r = L.KbsStepIO()
+        ld = io["state"]["qpos"].shape[-1]
+        r.state = _view(L.KbsStateView, STATE_ROWS, io["state"], ld)
+        r.noise = _view(L.KbsNoiseView, NOISE_ROWS, io.get("noise"))
+        r.episode = _view(L.KbsEpisodeView, EPISODE_ROWS, io.get("episode"))
+        r.traj_state = _view(L.KbsStateView, STATE_ROWS, io.get("traj_state"), ld)
+        for k, _ in L.KbsStepIO._fields_:
+            if k not in ("state", "noise", "episode", "traj_state", "T"):
+                setattr(r, k, L.ptr(io.get(k)))
+        r.T = io["command"].shape[0] - 1 if io.get("command") is not None else 0
+        L.check(self.lib.kbs_rollout_step(self._h, C.byref(st.desc), C.byref(r), _stream()), "kbs_rollout_step")
+
+
+@dataclass
+class StepState:
+    """A step state's device buffer and its kbs_step_state descriptor (keeps the buffer alive)."""
+
+    buf: torch.Tensor
+    desc: L.KbsStepState

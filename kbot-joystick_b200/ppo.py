@@ -281,6 +281,78 @@ class PpoUpdater:
         self._iter_graph_work = (self._iwork, self._ework)     # the graph holds their addresses
         self.eng.scratch_lock(True)
 
+    # ---- the online form: one control step per call, the rollout's carries resident on the device ----------------------------
+    def begin_iteration(self, io: dict, n_envs: int) -> None:
+        """Start an iteration of the online rollout into io's trajectories (command [T+1,16,ld], actor_obs, action, log_prob,
+        ctrl, done, success, value; term_codes optional).  The first call makes the step state from io's actor_carry,
+        critic_carry, lpf, pg_carry and command[0]; later iterations continue from the state.  Every call snapshots the state's
+        carries for the epoch: the iteration's one conversion out of the kernels' layouts."""
+        T, _, ld = io["actor_obs"].shape
+        key = (id(io), T, ld, n_envs)
+        if getattr(self, "_okey", None) != key:
+            dev = self.param.device
+            self._okey, self._oio = key, io
+            self.step_st = self.eng.step_state(n_envs, True, {"actor_carry": io["actor_carry"], "critic_carry": io["critic_carry"],
+                                                              "lpf": io["lpf"], "pg_carry": io["pg_carry"],
+                                                              "command": io["command"][0]})
+            self._owork = {"actor_carry0": torch.empty_like(io["actor_carry"]), "critic_carry0": torch.empty_like(io["critic_carry"]),
+                           "lpf0": torch.empty_like(io["lpf"]), "critic_obs": torch.empty((T, L.CRITIC_OBS, ld), device=dev),
+                           "rewards": torch.empty((T, ld), device=dev),
+                           "traj_state": {k: torch.empty((T, r, ld), device=dev) for k, r in self.REWARD_STATE_ROWS.items()}}
+            self._step_graphs = {}
+            self._online_iterations = 0
+        w = self._owork
+        self.eng.step_state_store(self.step_st, {"actor_carry": w["actor_carry0"], "critic_carry": w["critic_carry0"],
+                                                 "lpf": w["lpf0"]})
+
+    REWARD_STATE_ROWS = {"qpos": 27, "qvel": 26, "sensordata": 49, "xpos": 72, "xquat": 96, "com_distance": 1}   # kbs_rewards
+
+    def _online_step(self, io_t: dict) -> None:
+        io = self._oio
+        self.eng.rollout_step(self.step_st, dict(
+            {k: io_t.get(k) for k in ("state", "noise", "episode", "eps_action", "u_switch", "cmd_mode", "cmd_u6", "cmd_u_arms")},
+            **{k: io.get(k) for k in ("command", "actor_obs", "action", "log_prob", "ctrl", "term_codes", "done", "success", "value")},
+            critic_obs=self._owork["critic_obs"], traj_state=self._owork["traj_state"]))
+
+    def step(self, io_t: dict) -> None:
+        """One control step into slot t of the iteration's trajectories.  io_t: this step's state / noise / episode (dicts of
+        [F, ld] tensors), eps_action, u_switch, cmd_mode, cmd_u6, cmd_u_arms.  After capture_step(io_t), a call with the same
+        io_t object replays the graph (refill its tensors in place between steps)."""
+        g = self._step_graphs.get(id(io_t))
+        if g is not None and g[1] is io_t:
+            g[0].replay()
+            return
+        self._online_step(io_t)
+
+    def capture_step(self, io_t: dict) -> None:
+        """Record step(io_t) as ONE CUDA graph, replayed by later step() calls with the same io_t for every t (the state's step
+        index lives on the device).  Capturing runs nothing.  The graph holds pointers into the handle's scratch, which is
+        locked here, so the scratch must already have grown to what a step AND end_iteration's epoch need: call it after one
+        whole eager iteration (begin_iteration, step x T, end_iteration) on this io; before that it raises."""
+        if not getattr(self, "_online_iterations", 0):
+            raise RuntimeError("capture_step: run one whole eager iteration (begin_iteration, step, end_iteration) first")
+        torch.cuda.synchronize()
+        g = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(g):
+            self._online_step(io_t)
+        self._step_graphs[id(io_t)] = (g, io_t)
+        self.eng.scratch_lock(True)
+
+    def end_iteration(self, reward_carry: dict, n_envs: int, batch_size: int = 512, num_passes: int = 3, seed: int = 0) -> dict:
+        """kbs_rewards on the recorded trajectory (reward_carry advanced in place), then epoch() on it; the step state is then
+        ready for the next iteration (step index 0; its command and done_prev carry over, as iteration() carries them).
+        Returns what iteration() returns."""
+        io, w = self._oio, self._owork
+        T = io["actor_obs"].shape[0]
+        self.eng.rewards(w["traj_state"], io["command"][:T], io["ctrl"], io["done"], reward_carry, total=w["rewards"], n_envs=n_envs)
+        rollout = {"actor_obs": io["actor_obs"], "critic_obs": w["critic_obs"], "action": io["action"], "done": io["done"],
+                   "success": io["success"], "rewards": w["rewards"], "actor_carry0": w["actor_carry0"],
+                   "critic_carry0": w["critic_carry0"], "lpf0": w["lpf0"]}
+        out = self._epoch(rollout, n_envs, batch_size, num_passes, seed)
+        self.eng.step_state_rewind(self.step_st)
+        self._online_iterations += 1
+        return dict(out, rewards=w["rewards"])
+
     @property
     def step_count(self) -> int:
         return int(self.step_dev.item())
