@@ -537,6 +537,53 @@ typedef struct kbs_step_io {
  * n_envs it cannot take). */
 int kbs_rollout_step(kbs_handle* h, const kbs_step_state* st, const kbs_step_io* io, void* stream);
 
+/* The physics sub-steps between two online control steps (ksim's engine loop: S = ctrl_dt / dt calls of mjx.step per control
+ * step, train.py:1775-1781: dt 0.004, ctrl_dt 0.02 => 5, action_latency_range (0.003, 0.01) s, drop_action_prob 0.05).
+ * Before each mjx.step the engine calls PositionActuators.get_ctrl on that sub-step's joint state.  The rule [U], the same as
+ * kbs_torque_substeps and oracle.position_actuator_substeps:
+ *   applied = u_drop < drop_prob ? prev_action : action         (a dropped command repeats the last applied action)
+ *   ctrl_k  = PD(k * sub_dt >= latency ? applied : prev_action, q_k, qd_k)          k = 0 .. S-1
+ *   after sub-step S-1: prev_action = applied
+ * With a simulator in the loop the joint state of sub-step k+1 depends on ctrl_k, so the sub-steps are one call each.  What
+ * crosses a sub-step stays on the device in a caller-owned ACTUATOR STATE, beside the step state: one device buffer of
+ * kbs_actuator_state_bytes bytes, 256-byte aligned, holding the sub-step index k (device int32), prev_action [20][ld] (the last
+ * applied action) and applied [20][ld] (this control step's latched action), rows at ld = n_envs rounded up to a multiple of 4. */
+typedef struct kbs_actuator_state {
+  void* buf;                  /* device, 256-byte aligned */
+  uint64_t bytes;             /* size of buf: >= kbs_actuator_state_bytes(h, n_envs) */
+  int64_t n_envs;
+  int32_t n_substeps;         /* S: sub-steps per control step (> 0) */
+} kbs_actuator_state;
+int kbs_actuator_state_bytes(kbs_handle* h, int64_t n_envs, uint64_t* bytes);
+/* prev_action [20][ld] or NULL (= zeros); sets k = 0. */
+int kbs_actuator_state_load(kbs_handle* h, const kbs_actuator_state* ast, const float* prev_action, void* stream);
+/* prev_action [20][ld] <- the state's last applied action; the state is left as it is. */
+int kbs_actuator_state_store(kbs_handle* h, const kbs_actuator_state* ast, float* prev_action, void* stream);
+
+/* One sub-step's inputs and output.  Arrays are [F][ld] at the states' ld unless stated otherwise. */
+typedef struct kbs_substep_io {
+  const float* action;        /* [T][20][ld]: the action trajectory the control steps record (kbs_step_io.action) */
+  int64_t T;
+  const float* u_drop;        /* [ld] U[0,1) of this control step */
+  const float* latency;       /* [ld] seconds, of this control step */
+  const float* qpos;          /* [27][ld] this sub-step's joint state: rows 7.. are q (as kbs_torque reads them) */
+  const float* qvel;          /* [26][ld] rows 6.. are qd */
+  kbs_episode_view episode;   /* gains, limits and biases; NULL fields = nominal / zero */
+  float* ctrl;                /* [20][ld] out */
+  float sub_dt;               /* > 0 (dt of the physics step) */
+  float drop_prob;            /* in [0, 1] */
+} kbs_substep_io;
+/* Sub-step k of the control step that kbs_rollout_step just ran, t being the step state's device index (already advanced, so
+ * the step's action is action[t-1]).  At k = 0 it latches `applied`; it writes ctrl; it then advances k, and after sub-step S-1
+ * it sets prev_action = applied and k = 0.  So S calls after a step give bitwise the S rows of ctrl, and the same prev_action,
+ * that kbs_torque_substeps gives for action[t-1] and the S joint states stacked.  t and k are read on the device: one captured
+ * sub-step replays for every sub-step of every control step.  Run the sub-steps of step T-1 before the step state is rewound.
+ * A sub-step that finds t = 0 (no step since load or rewind), t > T or k >= S writes nothing and leaves k as it is; it sets
+ * KBS_STATUS_SUBSTEP_RANGE, so the next fused call returns KBS_E_DEVICE.
+ * KBS_E_SHAPE: the two states' n_envs differ, n_substeps <= 0, T <= 0.  KBS_E_PARAM: sub_dt <= 0, drop_prob outside [0, 1]. */
+int kbs_actuator_substep(kbs_handle* h, const kbs_step_state* st, const kbs_actuator_state* ast, const kbs_substep_io* io,
+                         void* stream);
+
 /* Replaces: the jax.random draws the reference makes ON THE DEVICE during a rollout -- observation noise (train.py:1160, 1162,
  * 1176, 1194), the action sample (train.py:1564), the command resampling (train.py:725-737, 752-753, 782-783) -- for callers
  * that do not need bit parity with JAX's threefry streams (parity mode hands these arrays to kbs_rollout explicitly).
@@ -601,6 +648,7 @@ int kbs_device_status(kbs_handle* h, int* status_out);
 #define KBS_STATUS_TIMEOUT_HEAD 2
 #define KBS_STATUS_F16_RANGE 0x100
 #define KBS_STATUS_STEP_RANGE 0x200   /* kbs_rollout_step found its step index t >= T */
+#define KBS_STATUS_SUBSTEP_RANGE 0x400 /* kbs_actuator_substep found t = 0, t > T or k >= S */
 int kbs_device_status_reset(kbs_handle* h);
 
 /* Per-kernel device timing for bench.py's roofline line: while enabled, every kernel launch of this handle is
@@ -618,7 +666,7 @@ int kbs_debug_tc_trace(kbs_handle* h, long long* trace_out, int64_t n_envs, void
 /* Same stamps for LSTM layer `layer` at step `step` of subsequent kbs_rollout calls (trace_out NULL detaches). */
 int kbs_debug_tc_trace_attach(kbs_handle* h, long long* trace_out, int64_t step, int layer);
 
-#define KBS_NUM_KERNEL_IDS 25
+#define KBS_NUM_KERNEL_IDS 26
 int kbs_profile_enable(kbs_handle* h, int on);
 int kbs_profile_read(kbs_handle* h, int max_ids, double* total_ms, int64_t* launches);
 const char* kbs_kernel_name(int id);

@@ -105,6 +105,17 @@ class KbsStepIO(C.Structure):
         ("traj_state", KbsStateView), ("T", _i64)]
 
 
+class KbsActuatorState(C.Structure):
+    """kbs_actuator_state: the caller-owned device buffer of the physics sub-steps (k, prev_action, applied)."""
+    _fields_ = [("buf", _vp), ("bytes", C.c_uint64), ("n_envs", _i64), ("n_substeps", C.c_int32)]
+
+
+class KbsSubstepIO(C.Structure):
+    """kbs_substep_io: one physics sub-step's inputs and its ctrl."""
+    _fields_ = [("action", _vp), ("T", _i64), ("u_drop", _vp), ("latency", _vp), ("qpos", _vp), ("qvel", _vp),
+                ("episode", KbsEpisodeView), ("ctrl", _vp), ("sub_dt", _f), ("drop_prob", _f)]
+
+
 class KbsPpoIO(C.Structure):
     _fields_ = [(k, _vp) for k in ("actor_obs", "critic_obs", "action", "done", "actor_carry", "critic_carry", "lpf",
                                    "log_probs", "values", "entropy", "action_std", "mean")] + [("T", _i64), ("ld", _i64)] + [
@@ -157,11 +168,13 @@ EXPORTS = (
     "kbs_adamw_default_params", "kbs_adamw_step", "kbs_grad_norm", "kbs_scratch_lock", "kbs_actuator_rand_default_params",
     "kbs_sample_actuator_randomization", "kbs_device_status_reset", "kbs_ppo_grad_set_events", "kbs_generate_rollout_noise",
     "kbs_minibatch_permutation", "kbs_shuffle_minibatches", "kbs_rollout_record", "kbs_step_state_bytes", "kbs_step_state_load",
-    "kbs_step_state_store", "kbs_step_state_rewind", "kbs_rollout_step",
+    "kbs_step_state_store", "kbs_step_state_rewind", "kbs_rollout_step", "kbs_actuator_state_bytes", "kbs_actuator_state_load",
+    "kbs_actuator_state_store", "kbs_actuator_substep",
 )
 VERSION = 101
 STATUS_TIMEOUT_LSTM, STATUS_TIMEOUT_HEAD, STATUS_F16_RANGE, STATUS_STEP_RANGE = 1, 2, 0x100, 0x200
-NUM_KERNEL_IDS = 25
+STATUS_SUBSTEP_RANGE = 0x400
+NUM_KERNEL_IDS = 26
 MAX_PERMUTATION_ENVS = 16384
 
 _lib = None
@@ -226,6 +239,10 @@ def load() -> C.CDLL:
     lib.kbs_step_state_store.argtypes = [_vp, P(KbsStepState), P(KbsStepCarry), _vp]
     lib.kbs_step_state_rewind.argtypes = [_vp, P(KbsStepState), _vp]
     lib.kbs_rollout_step.argtypes = [_vp, P(KbsStepState), P(KbsStepIO), _vp]
+    lib.kbs_actuator_state_bytes.argtypes = [_vp, _i64, P(C.c_uint64)]
+    lib.kbs_actuator_state_load.argtypes = [_vp, P(KbsActuatorState), _vp, _vp]
+    lib.kbs_actuator_state_store.argtypes = [_vp, P(KbsActuatorState), _vp, _vp]
+    lib.kbs_actuator_substep.argtypes = [_vp, P(KbsStepState), P(KbsActuatorState), P(KbsSubstepIO), _vp]
     lib.kbs_launch_count.argtypes = [_vp]
     lib.kbs_launch_count.restype = _i64
     lib.kbs_device_status.argtypes = [_vp, P(C.c_int)]

@@ -460,7 +460,7 @@ const char* kbs_kernel_name(int id) {
       "reward_scan_kernel", "gae_kernel", "adv_norm_kernel", "policy_io_kernels", "gemm_nt_kernel(simt)",
       "lstm_cell_kernel", "actor_head_kernel", "critic_head_kernel", "pack_kernels", "lstm_layer_tc_kernel",
       "proj_tc_kernel", "rollout_persist_kernel", "bptt_persist_kernel", "gemm_tn_tc_kernel", "sb_to_tn_kernel", "tn_reduce_kernel",
-      "step_record_kernel", "minibatch_permutation_kernel", "shuffle_minibatches_kernels"};
+      "step_record_kernel", "actuator_substep_kernel", "minibatch_permutation_kernel", "shuffle_minibatches_kernels"};
   return (id >= 0 && id < KBS_K_COUNT) ? names[id] : "?";
 }
 
@@ -1230,6 +1230,104 @@ int kbs_rollout_step(kbs_handle* h, const kbs_step_state* st, const kbs_step_io*
   if ((rc = kbs_status_init(h))) return rc;
   R.status = h->persist_status;
   if ((rc = kbs_launch_step_record(h, R, s))) return rc;
+  return kbs_status_publish(h, s);
+}
+
+}  // extern "C"
+
+// ---- the physics sub-steps between two online control steps, on a caller-owned actuator state ------------------------------
+namespace {
+
+struct ActuatorHeader { int32_t k; uint32_t ticket; };
+// Layout of an actuator state, carved from the caller's buffer like scratch (rows at ld = round_up4(n)).
+struct ActuatorState { ActuatorHeader* hdr; float* prev_action; float* applied; };
+ActuatorState actuator_state(KbsScratch& s, int64_t n) {
+  const int64_t ld = round_up4(n);
+  ActuatorState w{};
+  w.hdr = s.take<ActuatorHeader>(1);
+  w.prev_action = s.take<float>(size_t(KBS_NUM_JOINTS) * ld);
+  w.applied = s.take<float>(size_t(KBS_NUM_JOINTS) * ld);
+  return w;
+}
+
+uint64_t actuator_state_bytes(int64_t n) {
+  KbsScratch s{nullptr};
+  actuator_state(s, n);
+  return s.bytes;
+}
+
+// the descriptor's checks, then the layout on its buffer
+int actuator_state_at(const kbs_actuator_state* ast, ActuatorState* w) {
+  REQ(ast); REQ(ast->buf);
+  if (ast->n_envs <= 0 || ast->n_substeps <= 0) return KBS_E_SHAPE;
+  if (reinterpret_cast<uintptr_t>(ast->buf) & 255u) return KBS_E_ALIGN;
+  if (ast->bytes < actuator_state_bytes(ast->n_envs)) return KBS_E_SHAPE;
+  KbsScratch s{static_cast<char*>(ast->buf)};
+  *w = actuator_state(s, ast->n_envs);
+  return KBS_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int kbs_actuator_state_bytes(kbs_handle* h, int64_t n, uint64_t* bytes) {
+  REQ(h); REQ(bytes);
+  if (n <= 0) return KBS_E_SHAPE;
+  *bytes = actuator_state_bytes(n);
+  return KBS_OK;
+}
+
+int kbs_actuator_state_load(kbs_handle* h, const kbs_actuator_state* ast, const float* prev_action, void* stream) {
+  REQ(h);
+  ActuatorState w;
+  int rc = actuator_state_at(ast, &w);
+  if (rc) return rc;
+  AL(prev_action);
+  if ((rc = kbs_enter(h))) return rc;
+  cudaStream_t s = (cudaStream_t)stream;
+  const size_t rows = size_t(KBS_NUM_JOINTS) * round_up4(ast->n_envs) * 4;
+  KBS_CUDA_TRY(cudaMemsetAsync(w.hdr, 0, sizeof(ActuatorHeader), s));
+  if ((rc = copy_or_zero(w.prev_action, prev_action, rows, s))) return rc;
+  KBS_CUDA_TRY(cudaMemsetAsync(w.applied, 0, rows, s));
+  return KBS_OK;
+}
+
+int kbs_actuator_state_store(kbs_handle* h, const kbs_actuator_state* ast, float* prev_action, void* stream) {
+  REQ(h); REQ(prev_action);
+  ActuatorState w;
+  int rc = actuator_state_at(ast, &w);
+  if (rc) return rc;
+  AL(prev_action);
+  if ((rc = kbs_enter(h))) return rc;
+  KBS_CUDA_TRY(cudaMemcpyAsync(prev_action, w.prev_action, size_t(KBS_NUM_JOINTS) * round_up4(ast->n_envs) * 4,
+                               cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+  return KBS_OK;
+}
+
+int kbs_actuator_substep(kbs_handle* h, const kbs_step_state* st, const kbs_actuator_state* ast, const kbs_substep_io* io,
+                         void* stream) {
+  REQ(h); REQ(io);
+  StepState w;
+  ActuatorState aw;
+  int rc = step_state_at(h, st, &w);
+  if (rc || (rc = actuator_state_at(ast, &aw))) return rc;
+  REQ(io->action); REQ(io->u_drop); REQ(io->latency); REQ(io->qpos); REQ(io->qvel); REQ(io->ctrl);
+  if (st->n_envs != ast->n_envs || io->T <= 0) return KBS_E_SHAPE;
+  if (!(io->sub_dt > 0.f) || !(io->drop_prob >= 0.f && io->drop_prob <= 1.f)) return KBS_E_PARAM;
+  AL(io->action); AL(io->u_drop); AL(io->latency); AL(io->qpos); AL(io->qvel); AL(io->ctrl);
+  const kbs_episode_view& ep = io->episode;
+  AL(ep.kp); AL(ep.kd); AL(ep.tau_limit); AL(ep.action_bias); AL(ep.torque_bias);
+  if ((rc = kbs_enter(h))) return rc;
+  if ((rc = kbs_status_init(h))) return rc;
+  cudaStream_t s = (cudaStream_t)stream;
+  KbsSubstepArgs a{};
+  a.action = io->action; a.T = io->T; a.t = &w.hdr->t;
+  a.k = &aw.hdr->k; a.ticket = &aw.hdr->ticket; a.prev_action = aw.prev_action; a.applied = aw.applied;
+  a.u_drop = io->u_drop; a.latency = io->latency; a.qpos = io->qpos; a.qvel = io->qvel; a.ep = ep; a.ctrl = io->ctrl;
+  a.S = ast->n_substeps; a.sub_dt = io->sub_dt; a.drop_prob = io->drop_prob;
+  a.n = st->n_envs; a.ld = round_up4(st->n_envs); a.status = h->persist_status;
+  if ((rc = kbs_launch_actuator_substep(h, a, s))) return rc;
   return kbs_status_publish(h, s);
 }
 

@@ -48,7 +48,7 @@ enum KbsKernelId {
   KBS_K_OBS = 0, KBS_K_COMMAND, KBS_K_TORQUE, KBS_K_TERMINATE, KBS_K_REWARD_ROT, KBS_K_REWARD_TERMS, KBS_K_REWARD_SCAN,
   KBS_K_GAE, KBS_K_ADV_NORM, KBS_K_POLICY_IO, KBS_K_GEMM_SIMT, KBS_K_LSTM_CELL, KBS_K_ACTOR_HEAD, KBS_K_CRITIC_HEAD,
   KBS_K_PACK, KBS_K_LSTM_TC, KBS_K_PROJ_TC, KBS_K_ROLLOUT_TC, KBS_K_BPTT_TC, KBS_K_GEMM_TN, KBS_K_PACK_TN, KBS_K_TN_REDUCE,
-  KBS_K_STEP_RECORD, KBS_K_PERMUTATION, KBS_K_SHUFFLE, KBS_K_COUNT
+  KBS_K_STEP_RECORD, KBS_K_ACTUATOR_SUBSTEP, KBS_K_PERMUTATION, KBS_K_SHUFFLE, KBS_K_COUNT
 };
 static_assert(KBS_K_COUNT == KBS_NUM_KERNEL_IDS, "kbotstep.h KBS_NUM_KERNEL_IDS");
 constexpr int kKbsProfMaxPairs = 8192;
@@ -195,6 +195,15 @@ struct KbsStepRecord {
   int64_t T; int64_t* t; int* hsb_slot; unsigned int* ticket; unsigned int* status;
 };
 int kbs_launch_step_record(kbs_handle* h, KbsStepRecord a, cudaStream_t st);
+// one physics sub-step of the online rollout (kbs_actuator_substep): t from the step state, k / ticket / prev_action /
+// applied from the actuator state; action = the [T][20][ld] trajectory
+struct KbsSubstepArgs {
+  const float* action; int64_t T; const int64_t* t;
+  int32_t* k; unsigned int* ticket; float* prev_action; float* applied;
+  const float* u_drop; const float* latency; const float* qpos; const float* qvel; kbs_episode_view ep; float* ctrl;
+  int S; float sub_dt, drop_prob; int64_t ld, n; unsigned int* status;
+};
+int kbs_launch_actuator_substep(kbs_handle* h, const KbsSubstepArgs& a, cudaStream_t st);
 // kbs_ppo_update.cu: the update phase's minibatch construction (arguments validated by the entry points in kbs_api.cu)
 int kbs_launch_minibatch_permutation(kbs_handle* h, uint64_t seed, int64_t* pass_dev, int64_t env0, int32_t* perm, int64_t n,
                                      cudaStream_t st);

@@ -832,6 +832,35 @@ torque_kernel(const __grid_constant__ kbs_params P, const float* __restrict__ ac
 // Per-physics-sub-step actuator path (SURVEY 8f-2; train.py:1775-1781: dt 0.004, ctrl_dt 0.02, action latency 3-10 ms,
 // 5 % dropped commands; ksim engine semantics [U], see oracle position_actuator_substeps): a dropped command repeats
 // the last applied action; sub-step k sees the new action once k sub_dt >= latency; PD torque on the sub-step's joint state.
+// Two kernels evaluate it: all S sub-steps of recorded joint states in one launch (torque_substeps_kernel), or one sub-step
+// per launch with the simulator in the loop (actuator_substep_kernel).  Both take the gains and the per-element rule from
+// the two functions below, so they cannot drift apart.
+
+// joint j's gains, limit and biases for 4 envs (nominal / zero where the episode view has no array)
+struct Gains4 { float kp[4], kd[4], lim[4], ab[4], tb[4]; };
+__device__ __forceinline__ void substep_gains4(const kbs_params& P, const kbs_episode_view& ep, int j, int64_t ld, int64_t n0,
+                                               Gains4& g) {
+#pragma unroll
+  for (int l = 0; l < 4; ++l) {
+    g.kp[l] = P.kp[j]; g.kd[l] = P.kd[j]; g.lim[l] = P.ctrl_limit[j]; g.ab[l] = 0.f; g.tb[l] = 0.f;
+  }
+  if (ep.kp) kbs_ld4(ep.kp, j, ld, n0, g.kp);
+  if (ep.kd) kbs_ld4(ep.kd, j, ld, n0, g.kd);
+  if (ep.tau_limit) kbs_ld4(ep.tau_limit, j, ld, n0, g.lim);
+  if (ep.action_bias) kbs_ld4(ep.action_bias, j, ld, n0, g.ab);
+  if (ep.torque_bias) kbs_ld4(ep.torque_bias, j, ld, n0, g.tb);
+}
+
+// env l of 4 at sub-step time tk = k sub_dt: the latency select, PositionActuators.get_ctrl, the clamp
+__device__ __forceinline__ float substep_torque(float applied, float prev, float tk, float lat, float q, float qd, const Gains4& g,
+                                                int l, bool has_ab, bool has_tb) {
+  const float act = (tk >= lat) ? applied : prev;
+  const float target = has_ab ? act + g.ab[l] : act;
+  float tau = g.kp[l] * (target - q) - g.kd[l] * qd;
+  if (has_tb) tau = tau + g.tb[l];
+  return fminf(fmaxf(tau, -g.lim[l]), g.lim[l]);
+}
+
 //   q_sub / qd_sub / ctrl [S][20][ld]; prev_action [20][ld] in/out
 __global__ void __launch_bounds__(kThreads)
 torque_substeps_kernel(const __grid_constant__ kbs_params P, const float* __restrict__ action, float* __restrict__ prev_action,
@@ -843,19 +872,14 @@ torque_substeps_kernel(const __grid_constant__ kbs_params P, const float* __rest
   float ud[4], lat[4];
   kbs_ld4(u_drop, 0, ld, n0, ud);
   kbs_ld4(latency, 0, ld, n0, lat);
+  const bool has_ab = ep.action_bias != nullptr, has_tb = ep.torque_bias != nullptr;
 #pragma unroll 2
   for (int j = 0; j < KBS_NUM_JOINTS; ++j) {
     float a[4], pa[4], ap[4];
-    float kp[4] = {P.kp[j], P.kp[j], P.kp[j], P.kp[j]}, kd[4] = {P.kd[j], P.kd[j], P.kd[j], P.kd[j]};
-    float lim[4] = {P.ctrl_limit[j], P.ctrl_limit[j], P.ctrl_limit[j], P.ctrl_limit[j]};
-    float ab[4] = {0, 0, 0, 0}, tb[4] = {0, 0, 0, 0};
+    Gains4 g;
     kbs_ld4(action, j, ld, n0, a);
     kbs_ld4(prev_action, j, ld, n0, pa);
-    if (ep.kp) kbs_ld4(ep.kp, j, ld, n0, kp);
-    if (ep.kd) kbs_ld4(ep.kd, j, ld, n0, kd);
-    if (ep.tau_limit) kbs_ld4(ep.tau_limit, j, ld, n0, lim);
-    if (ep.action_bias) kbs_ld4(ep.action_bias, j, ld, n0, ab);
-    if (ep.torque_bias) kbs_ld4(ep.torque_bias, j, ld, n0, tb);
+    substep_gains4(P, ep, j, ld, n0, g);
 #pragma unroll
     for (int l = 0; l < 4; ++l) ap[l] = (ud[l] < drop_prob) ? pa[l] : a[l];
     for (int k = 0; k < S; ++k) {
@@ -864,16 +888,70 @@ torque_substeps_kernel(const __grid_constant__ kbs_params P, const float* __rest
       kbs_ld4(qd_sub + int64_t(k) * KBS_NUM_JOINTS * ld, j, ld, n0, qd);
       const float tk = float(k) * sub_dt;
 #pragma unroll
-      for (int l = 0; l < 4; ++l) {
-        const float act = (tk >= lat[l]) ? ap[l] : pa[l];
-        const float target = ep.action_bias ? act + ab[l] : act;
-        float tau = kp[l] * (target - q[l]) - kd[l] * qd[l];
-        if (ep.torque_bias) tau = tau + tb[l];
-        o[l] = fminf(fmaxf(tau, -lim[l]), lim[l]);
-      }
+      for (int l = 0; l < 4; ++l) o[l] = substep_torque(ap[l], pa[l], tk, lat[l], q[l], qd[l], g, l, has_ab, has_tb);
       kbs_st4(ctrl + int64_t(k) * KBS_NUM_JOINTS * ld, j, ld, n0, o);
     }
     kbs_st4(prev_action, j, ld, n0, ap);
+  }
+}
+
+// One sub-step of the online rollout (kbs_actuator_substep): t (the step state's index, the control step that just ran is
+// t-1) and k (the actuator state's sub-step index) are read once per block.  At k = 0 the step's action is latched into
+// `applied` (or prev_action where the command is dropped); ctrl = PD on this sub-step's qpos rows 7.. / qvel rows 6..; at
+// k = S-1 prev_action = applied.  grid = (env groups, joint): one sub-step of a few thousand envs is ~3 MB, so one joint per
+// block row gives the SMs 20x the blocks a whole-env thread would.  The last block to finish advances k (ticket, as
+// step_record_kernel), so one captured launch serves every sub-step.  Out of range (t = 0, t > T, k >= S): nothing is
+// written, k stays, KBS_STATUS_SUBSTEP_RANGE is set.
+__global__ void __launch_bounds__(kThreads)
+actuator_substep_kernel(const __grid_constant__ kbs_params P, const __grid_constant__ KbsSubstepArgs a) {
+  __shared__ int64_t t_s;
+  __shared__ int k_s;
+  if (threadIdx.x == 0) {
+    t_s = *reinterpret_cast<const volatile int64_t*>(a.t);
+    k_s = *reinterpret_cast<volatile int32_t*>(a.k);
+  }
+  __syncthreads();
+  const int64_t t = t_s;
+  const int k = k_s;
+  const bool in_range = t >= 1 && t <= a.T && k >= 0 && k < a.S;
+  const int64_t n0 = (int64_t(blockIdx.x) * kThreads + threadIdx.x) * 4;
+  const int j = blockIdx.y;
+  if (in_range && n0 < a.n) {
+    const int64_t ld = a.ld;
+    const bool has_ab = a.ep.action_bias != nullptr, has_tb = a.ep.torque_bias != nullptr;
+    const float tk = float(k) * a.sub_dt;
+    float lat[4], pa[4], ap[4], q[4], qd[4], o[4];
+    Gains4 g;
+    kbs_ld4(a.latency, 0, ld, n0, lat);
+    kbs_ld4(a.prev_action, j, ld, n0, pa);
+    if (k == 0) {
+      float ud[4], x[4];
+      kbs_ld4(a.u_drop, 0, ld, n0, ud);
+      kbs_ld4(a.action + (t - 1) * KBS_NUM_JOINTS * ld, j, ld, n0, x);
+#pragma unroll
+      for (int l = 0; l < 4; ++l) ap[l] = (ud[l] < a.drop_prob) ? pa[l] : x[l];
+      kbs_st4(a.applied, j, ld, n0, ap);
+    } else {
+      kbs_ld4(a.applied, j, ld, n0, ap);
+    }
+    kbs_ld4(a.qpos, 7 + j, ld, n0, q);
+    kbs_ld4(a.qvel, 6 + j, ld, n0, qd);
+    substep_gains4(P, a.ep, j, ld, n0, g);
+#pragma unroll
+    for (int l = 0; l < 4; ++l) o[l] = substep_torque(ap[l], pa[l], tk, lat[l], q[l], qd[l], g, l, has_ab, has_tb);
+    kbs_st4(a.ctrl, j, ld, n0, o);
+    if (k == a.S - 1) kbs_st4(a.prev_action, j, ld, n0, ap);
+  } else if (!in_range && blockIdx.x == 0 && j == 0 && threadIdx.x == 0) {
+    atomicOr(a.status, unsigned(KBS_STATUS_SUBSTEP_RANGE));
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    __threadfence();
+    if (atomicAdd(a.ticket, 1u) == gridDim.x * gridDim.y - 1) {      // every block has read k
+      *a.ticket = 0u;
+      if (in_range) *a.k = (k + 1 == a.S) ? 0 : k + 1;
+      __threadfence();
+    }
   }
 }
 
@@ -1578,6 +1656,12 @@ int kbs_launch_torque_substeps(kbs_handle* h, const float* action, float* prev_a
   KBS_LAUNCH(h, KBS_K_TORQUE, st,
              (torque_substeps_kernel<<<groups4(n), kThreads, 0, st>>>(h->p, action, prev_action, u_drop, latency, q_sub, qd_sub, e,
                                                                       ctrl, S, sub_dt, drop_prob, ld, n)));
+  KBS_LAUNCH_CHECK();
+  return KBS_OK;
+}
+
+int kbs_launch_actuator_substep(kbs_handle* h, const KbsSubstepArgs& a, cudaStream_t st) {
+  KBS_LAUNCH(h, KBS_K_ACTUATOR_SUBSTEP, st, (actuator_substep_kernel<<<dim3(groups4(a.n), KBS_NUM_JOINTS), kThreads, 0, st>>>(h->p, a)));
   KBS_LAUNCH_CHECK();
   return KBS_OK;
 }

@@ -515,6 +515,44 @@ class KbotStep:
         r.T = io["command"].shape[0] - 1 if io.get("command") is not None else 0
         L.check(self.lib.kbs_rollout_step(self._h, C.byref(st.desc), C.byref(r), _stream()), "kbs_rollout_step")
 
+    # ---- the physics sub-steps between two online control steps ---------------------------------------------------------------
+    def actuator_state(self, n_envs: int, n_substeps: int, prev_action=None) -> "ActuatorState":
+        """A device actuator state for n_envs and n_substeps sub-steps per control step (kbs_actuator_state): the sub-step index,
+        the last applied action and this control step's latched one, loaded from prev_action [20, ld] (None = zeros)."""
+        nb = C.c_uint64(0)
+        L.check(self.lib.kbs_actuator_state_bytes(self._h, n_envs, C.byref(nb)), "kbs_actuator_state_bytes")
+        buf = torch.empty((int(nb.value),), dtype=torch.uint8, device=torch.device("cuda", torch.cuda.current_device()))
+        ast = ActuatorState(buf, L.KbsActuatorState(buf.data_ptr(), int(nb.value), n_envs, n_substeps))
+        self.actuator_state_load(ast, prev_action)
+        return ast
+
+    def actuator_state_load(self, ast: "ActuatorState", prev_action=None) -> None:
+        """prev_action [20, ld] (None = zeros); the sub-step index becomes 0."""
+        L.check(self.lib.kbs_actuator_state_load(self._h, C.byref(ast.desc), L.ptr(prev_action), _stream()),
+                "kbs_actuator_state_load")
+
+    def actuator_state_store(self, ast: "ActuatorState", prev_action=None):
+        """The state's last applied action, written into prev_action [20, ld] (allocated when None) and returned."""
+        if prev_action is None:
+            prev_action = torch.empty((L.NUM_JOINTS, round_up4(ast.desc.n_envs)), device=ast.buf.device)
+        L.check(self.lib.kbs_actuator_state_store(self._h, C.byref(ast.desc), L.ptr(prev_action), _stream()),
+                "kbs_actuator_state_store")
+        return prev_action
+
+    def actuator_substep(self, st: "StepState", ast: "ActuatorState", io_k: dict) -> None:
+        """One physics sub-step after the control step st just ran (kbs_actuator_substep).  io_k: action [T, 20, ld] (the
+        trajectory the steps record), u_drop / latency [ld] of this control step, qpos [27, ld] / qvel [26, ld] of this sub-step,
+        episode (dict of [F, ld] tensors, optional), ctrl [20, ld] (written); sub_dt / drop_prob (default 0.004 / 0.05).  The
+        sub-step index and the step index are read on the device."""
+        r = L.KbsSubstepIO()
+        for k in ("action", "u_drop", "latency", "qpos", "qvel", "ctrl"):
+            setattr(r, k, L.ptr(io_k.get(k)))
+        r.T = io_k["action"].shape[0] if io_k.get("action") is not None else 0
+        r.episode = _view(L.KbsEpisodeView, EPISODE_ROWS, io_k.get("episode"))
+        r.sub_dt, r.drop_prob = io_k.get("sub_dt", 0.004), io_k.get("drop_prob", 0.05)
+        L.check(self.lib.kbs_actuator_substep(self._h, C.byref(st.desc), C.byref(ast.desc), C.byref(r), _stream()),
+                "kbs_actuator_substep")
+
 
 @dataclass
 class StepState:
@@ -522,3 +560,11 @@ class StepState:
 
     buf: torch.Tensor
     desc: L.KbsStepState
+
+
+@dataclass
+class ActuatorState:
+    """An actuator state's device buffer and its kbs_actuator_state descriptor (keeps the buffer alive)."""
+
+    buf: torch.Tensor
+    desc: L.KbsActuatorState

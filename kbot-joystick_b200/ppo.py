@@ -299,7 +299,8 @@ class PpoUpdater:
                            "lpf0": torch.empty_like(io["lpf"]), "critic_obs": torch.empty((T, L.CRITIC_OBS, ld), device=dev),
                            "rewards": torch.empty((T, ld), device=dev),
                            "traj_state": {k: torch.empty((T, r, ld), device=dev) for k, r in self.REWARD_STATE_ROWS.items()}}
-            self._step_graphs = {}
+            self._step_graphs, self._substep_graphs = {}, {}
+            self.act_st = None
             self._online_iterations = 0
         w = self._owork
         self.eng.step_state_store(self.step_st, {"actor_carry": w["actor_carry0"], "critic_carry": w["critic_carry0"],
@@ -337,6 +338,43 @@ class PpoUpdater:
             self._online_step(io_t)
         self._step_graphs[id(io_t)] = (g, io_t)
         self.eng.scratch_lock(True)
+
+    def _online_substep(self, io_k: dict, n_substeps: int, sub_dt: float, drop_prob: float) -> None:
+        n = self.step_st.desc.n_envs
+        ast = getattr(self, "act_st", None)
+        if ast is None or (ast.desc.n_envs, ast.desc.n_substeps) != (n, n_substeps):
+            self.act_st = ast = self.eng.actuator_state(n, n_substeps)
+        self.eng.actuator_substep(self.step_st, ast, dict(
+            {k: io_k.get(k) for k in ("qpos", "qvel", "u_drop", "latency", "episode", "ctrl")}, action=self._oio["action"],
+            sub_dt=sub_dt, drop_prob=drop_prob))
+
+    def substep(self, io_k: dict, *, n_substeps: int = 5, sub_dt: float = 0.004, drop_prob: float = 0.05) -> None:
+        """One physics sub-step after the control step that step() just ran: ctrl [20, ld] of io_k = the PD torque on io_k's
+        qpos [27, ld] / qvel [26, ld] (gains from io_k's episode) of the action the actuators see at this sub-step -- this step's
+        action once latency [ld] has elapsed, the previous one before, the previous one throughout where u_drop [ld] <
+        drop_prob (kbs_actuator_substep).  Call it n_substeps times per step, before end_iteration.  The actuator state (sub-step
+        index, last applied action) is made on first use, from zeros.  After capture_substep(io_k), a call with the same io_k
+        object replays the graph (refill its tensors in place between sub-steps)."""
+        g = self._substep_graphs.get(id(io_k))
+        if g is not None and g[1] is io_k:
+            g[0].replay()
+            return
+        self._online_substep(io_k, n_substeps, sub_dt, drop_prob)
+
+    def capture_substep(self, io_k: dict, *, n_substeps: int = 5, sub_dt: float = 0.004, drop_prob: float = 0.05) -> None:
+        """Record substep(io_k) as ONE CUDA graph, replayed by later substep() calls with the same io_k for every sub-step of
+        every step (the sub-step and step indices live on the device), with the keyword arguments given here.  Capturing runs
+        nothing.  Like capture_step, it needs one whole eager iteration first; before that it raises."""
+        if not getattr(self, "_online_iterations", 0):
+            raise RuntimeError("capture_substep: run one whole eager iteration (begin_iteration, step, end_iteration) first")
+        n = self.step_st.desc.n_envs
+        if getattr(self, "act_st", None) is None or (self.act_st.desc.n_envs, self.act_st.desc.n_substeps) != (n, n_substeps):
+            self.act_st = self.eng.actuator_state(n, n_substeps)       # made outside the capture
+        torch.cuda.synchronize()
+        g = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(g):
+            self._online_substep(io_k, n_substeps, sub_dt, drop_prob)
+        self._substep_graphs[id(io_k)] = (g, io_k, self.act_st)      # the graph holds the state's addresses
 
     def end_iteration(self, reward_carry: dict, n_envs: int, batch_size: int = 512, num_passes: int = 3, seed: int = 0) -> dict:
         """kbs_rewards on the recorded trajectory (reward_carry advanced in place), then epoch() on it; the step state is then
