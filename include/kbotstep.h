@@ -59,7 +59,14 @@ enum { KBS_GEMM_TC_3XTF32 = 0, KBS_GEMM_SIMT_FP32 = 1, KBS_GEMM_TC_2XF16 = 2 };
  * train.py:22-70, 1206-1269; robot/kbot/metadata.json; robot/kbot/robot.mjcf. */
 typedef struct kbs_params {
   int32_t hidden_size;          /* train.py:1773 (256); 128 also supported */
-  int32_t depth;                /* train.py:82 (2) */
+  int32_t depth;                /* train.py:82 (2).  1 .. KBS_MAX_DEPTH; kbs_create refuses others with KBS_E_SHAPE.
+                                 * The persistent tensor-core kernels hold at most 2 layers.  Above 2, on the tensor-core
+                                 * datapaths (3xTF32, FP16-split), these refuse with KBS_E_SHAPE before launching anything:
+                                 *   kbs_ppo_variables with mean or the mirror pass;
+                                 *   kbs_step_state_bytes / _load and so kbs_rollout_step (no online step state);
+                                 *   kbs_ppo_grad on FP16-split: the lower layers' dG leaves the FP16 split's range
+                                 *   (3xTF32 and SIMT take any depth).
+                                 * Everything else runs the per-step launches instead of the persistent kernels. */
   int32_t gemm_path;            /* KBS_GEMM_* */
   int32_t normalize_advantages; /* ksim compute_ppo_inputs flag [unverified]: 0 none, 1 per-trajectory a/(std+eps) */
   float ctrl_dt;                /* train.py:1776 */

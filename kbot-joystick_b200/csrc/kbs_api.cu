@@ -814,7 +814,9 @@ int kbs_ppo_variables(kbs_handle* h, const kbs_ppo_io* io, int64_t n, void* stre
   cudaStream_t st = (cudaStream_t)stream;
   const int64_t ld = io->ld, T = io->T;
   const bool tc = h->p.gemm_path != KBS_GEMM_SIMT_FP32;
-  if (tc && io->mean && !kbs_tc_persistent_available(h, n, T, critic ? 2 : 1)) return KBS_E_SHAPE;
+  // dist.mean() -- asked for, or taken internally by the mirror pass -- is an output of the persistent kernel only: refuse
+  // before anything is launched, so the outputs and carries stay as they were
+  if (tc && (io->mean || mirror) && !kbs_tc_persistent_available(h, n, T, critic ? 2 : 1)) return KBS_E_SHAPE;
   // the mirror pass's intermediates: mean, mean_m [T][20][ld], value_m, lp_m, ent_m [T][ld]; then both passes' workspace
   float *mean = nullptr, *mean_m = nullptr, *value_m = nullptr, *lp_m = nullptr, *ent_m = nullptr;
   VarsWs ws;
@@ -1068,6 +1070,8 @@ extern "C" {
 int kbs_step_state_bytes(kbs_handle* h, int64_t n, int with_critic, uint64_t* bytes) {
   REQ(h); REQ(bytes);
   if (n <= 0) return KBS_E_SHAPE;
+  // the tensor-core datapaths keep the carries in the persistent kernel's layouts: a shape it cannot run has no state
+  if (h->p.gemm_path != KBS_GEMM_SIMT_FP32 && !kbs_tc_persistent_available(h, n, 1, with_critic ? 2 : 1)) return KBS_E_SHAPE;
   *bytes = step_state_bytes(h, n, with_critic != 0);
   return KBS_OK;
 }

@@ -291,10 +291,12 @@ class PpoUpdater:
         key = (id(io), T, ld, n_envs)
         if getattr(self, "_okey", None) != key:
             dev = self.param.device
-            self._okey, self._oio = key, io
+            # made first: where the handle has no step state (a tensor-core datapath at depth > 2) this raises and the
+            # updater keeps no half-made iteration
             self.step_st = self.eng.step_state(n_envs, True, {"actor_carry": io["actor_carry"], "critic_carry": io["critic_carry"],
                                                               "lpf": io["lpf"], "pg_carry": io["pg_carry"],
                                                               "command": io["command"][0]})
+            self._okey, self._oio = key, io
             self._owork = {"actor_carry0": torch.empty_like(io["actor_carry"]), "critic_carry0": torch.empty_like(io["critic_carry"]),
                            "lpf0": torch.empty_like(io["lpf"]), "critic_obs": torch.empty((T, L.CRITIC_OBS, ld), device=dev),
                            "rewards": torch.empty((T, ld), device=dev),

@@ -254,6 +254,15 @@ def compare_grads_blockwise(got: dict, ref: dict, net: str, H: int, depth: int) 
     return bad
 
 
+def grad_block_ratios(got: dict, ref: dict, net: str, H: int, depth: int) -> dict:
+    """{"net.tensor": its largest block error over that block's block_bound}: <= 1 passes the block check; the margin."""
+    out = {}
+    for (name, key, g), (_, _, r) in zip(grad_tensors(got, depth), grad_tensors(ref, depth)):
+        out[f"{net}.{name}"] = max(float(np.abs(g[rows] - r[rows]).max()) / block_bound(r[rows], r)
+                                   for _, rows in grad_blocks(net, key, H))
+    return out
+
+
 def ppo_device_batch(b: dict, dev, carry0=None) -> dict:
     """The library's form of a ppo_batch minibatch: SoA arrays, carries at the first step in the ABI layout."""
     d = lambda a, dt=None: synth.to_soa(a if dt is None else a.astype(dt), 1, dev)
@@ -267,10 +276,11 @@ def ppo_device_batch(b: dict, dev, carry0=None) -> dict:
     return batch
 
 
-def ppo_grad_compare(e, wa, wc, b: dict, p, dev, N: int, carry0=None, hyper=None) -> tuple:
+def ppo_grad_compare(e, wa, wc, b: dict, p, dev, N: int, carry0=None, hyper=None, ratios: dict | None = None) -> tuple:
     """kbs_ppo_grad on minibatch b (from carry0, with loss hyper-parameters hyper) against torch.autograd in float64
     (oracle/ppo_grad_torch.py): asserts log-probs, values and loss statistics; returns (the list of gradient tensors /
-    blocks outside their bound, the reference (loss, stats, grads_actor, grads_critic, log_probs, values))."""
+    blocks outside their bound, the reference (loss, stats, grads_actor, grads_critic, log_probs, values)).  ratios, when
+    given, receives grad_block_ratios of both nets."""
     import ppo_grad_torch as G
 
     S = synth.from_soa
@@ -292,6 +302,9 @@ def ppo_grad_compare(e, wa, wc, b: dict, p, dev, N: int, carry0=None, hyper=None
     close(out["stats"].cpu().numpy(), np.array((loss,) + stats, np.float32), "loss stats", rtol=2e-5, atol=1e-5)
     bad = (compare_grads_blockwise(ga, ga_ref, "actor", p.hidden_size, p.depth) +
            compare_grads_blockwise(gc, gc_ref, "critic", p.hidden_size, p.depth))
+    if ratios is not None:
+        ratios.update(grad_block_ratios(ga, ga_ref, "actor", p.hidden_size, p.depth))
+        ratios.update(grad_block_ratios(gc, gc_ref, "critic", p.hidden_size, p.depth))
     return bad, ref
 
 
