@@ -52,7 +52,9 @@ enum { KBS_NET_ACTOR = 0, KBS_NET_CRITIC = 1 };
 /* GEMM datapath for the LSTM/MLP contractions.  All are sm_100a CUDA in this library (no vendor library, no
  * fallback).  TC_* = tcgen05.mma with fp32 TMEM accumulators on operands split into two tensor-core-exact planes
  * (fp32-accurate: hi.hi + hi.lo + lo.hi): 3XTF32 = TF32 planes, 2XF16 = FP16 planes (lo scaled by 2^11; operands must
- * stay below 65504 in magnitude; half the bytes and twice the MMA rate).  SIMT = plain fp32 FFMA. */
+ * stay below 65504 in magnitude; half the bytes and twice the MMA rate).  The FP16 split represents an operand element x
+ * to within 2^-22 |x| + 2^-36: below fp16's normal range (|x| < 2^-14) the floor 2^-36 is absolute, so an operand whose
+ * elements all sit near it keeps only its leading bits.  SIMT = plain fp32 FFMA. */
 enum { KBS_GEMM_TC_3XTF32 = 0, KBS_GEMM_SIMT_FP32 = 1, KBS_GEMM_TC_2XF16 = 2 };
 
 /* Scalars of the path.  Defaults = the reference launch config (train.py:1761-1791) and tables
@@ -63,9 +65,7 @@ typedef struct kbs_params {
                                  * The persistent tensor-core kernels hold at most 2 layers.  Above 2, on the tensor-core
                                  * datapaths (3xTF32, FP16-split), these refuse with KBS_E_SHAPE before launching anything:
                                  *   kbs_ppo_variables with mean or the mirror pass;
-                                 *   kbs_step_state_bytes / _load and so kbs_rollout_step (no online step state);
-                                 *   kbs_ppo_grad on FP16-split: the lower layers' dG leaves the FP16 split's range
-                                 *   (3xTF32 and SIMT take any depth).
+                                 *   kbs_step_state_bytes / _load and so kbs_rollout_step (no online step state).
                                  * Everything else runs the per-step launches instead of the persistent kernels. */
   int32_t gemm_path;            /* KBS_GEMM_* */
   int32_t normalize_advantages; /* ksim compute_ppo_inputs flag [unverified]: 0 none, 1 per-trajectory a/(std+eps) */
@@ -256,7 +256,7 @@ int kbs_adam_step(kbs_handle* h, float* param, const float* grad, float* m, floa
  * and the step counter untouched.  step_dev: device int64 = number of updates applied so far (read, then advanced by one
  * when the update is applied), so that the whole update can be replayed as one CUDA graph; NULL = use `step` (>= 1). */
 typedef struct kbs_adamw_params {
-  double b1, b2;   /* doubles: optax forms (1 - b) in Python double precision and only then rounds to fp32 (1.0f - 0.999f != 0.001f) */
+  double b1, b2;   /* doubles: (1 - b) is formed in double (1.0f - 0.999f != 0.001f); m and v are updated in double and rounded once */
   float lr, eps, weight_decay, grad_scale, max_grad_norm;
 } kbs_adamw_params;
 int kbs_adamw_default_params(kbs_adamw_params* p);   /* lr 5e-4, b1 0.9, b2 0.999, eps 1e-8, wd 1e-5 [R]; clip 10.0 [U] */
@@ -663,7 +663,8 @@ int kbs_device_status_reset(kbs_handle* h);
  * kbs_profile_read sums elapsed ms and launch counts per kernel id (ids 0..KBS_NUM_KERNEL_IDS-1, names from
  * kbs_kernel_name); returns 1 if the event pool overflowed (totals partial), 0 ok. */
 /* Test hook of the tcgen05 datapath: pre-activation gates [n][4H] (eqx order i,f,g,o, bias added) of LSTM layer
- * `layer` of `net` for row-major x [n][H], h [n][H].  Needs gemm_path = KBS_GEMM_TC_3XTF32 and packed weights. */
+ * `layer` of `net` for row-major x [n][H], h [n][H].  Needs a tensor-core gemm_path (KBS_GEMM_TC_3XTF32 or
+ * KBS_GEMM_TC_2XF16) and packed weights: x and h are split as that datapath splits its operands. */
 int kbs_debug_tc_gates(kbs_handle* h, int net, int layer, const float* x_rm, const float* h_rm, float* gates_out,
                        int64_t n_envs, void* stream);
 

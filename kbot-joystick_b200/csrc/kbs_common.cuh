@@ -395,6 +395,12 @@ __device__ __forceinline__ float tf32_rn(float x) {
   asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
   return __uint_as_float(r);
 }
+// float(a) + c rounded once to fp32: sm_100's mixed-precision add (one FHADD, no separate f16 -> f32 conversion)
+__device__ __forceinline__ float kbs_add_f16_f32(__half a, float c) {
+  float d;
+  asm("add.rn.f32.f16 %0, %1, %2;" : "=f"(d) : "h"(__half_as_ushort(a)), "f"(c));
+  return d;
+}
 // byte offset of the 16-byte chunk holding (row, k) in plane `part`
 // WB = weight-block variant: [k-block][chunk][hi|lo][row][16 B], i.e. the hi and lo rows of one k-chunk are adjacent, so
 // ONE N = 2R descriptor (LBO = 2R*16 B) presents [W_hi | W_lo] to the tensor core and x_hi . [W_hi | W_lo]^T comes out of a
@@ -420,17 +426,17 @@ __device__ __forceinline__ KbsSplit4 sb_split4(const float (&x)[4]) {
     s.hi = make_uint4(__float_as_uint(h[0]), __float_as_uint(h[1]), __float_as_uint(h[2]), __float_as_uint(h[3]));
     s.lo = make_uint4(__float_as_uint(l[0]), __float_as_uint(l[1]), __float_as_uint(l[2]), __float_as_uint(l[3]));
   } else {
-    // hi = x rounded to 11 significant bits with integer ops (exactly an fp16 value for |x| in the normal range; below
-    // 6e-5 the conversion rounds once more, an absolute error < 3e-8 that nothing downstream resolves); the f32 -> f16
-    // conversions run on the quarter-rate XU pipe shared with ex2/rcp, so they are issued packed (cvt.rn.f16x2.f32).
-    float h[4], l[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      h[i] = __uint_as_float((__float_as_uint(x[i]) + 0x1000u) & 0xFFFFE000u);
-      l[i] = (x[i] - h[i]) * kKbsF16LoScale;
-    }
-    const __half2 h01 = __floats2half2_rn(h[0], h[1]), h23 = __floats2half2_rn(h[2], h[3]);
-    const __half2 l01 = __floats2half2_rn(l[0], l[1]), l23 = __floats2half2_rn(l[2], l[3]);
+    // hi = fp16(x), and lo = (x - hi) 2^11 is taken from that same fp16 value (hi - x is exact in fp32), so lo carries the
+    // whole residual at every magnitude: within fp16's normal range (|x| >= 2^-14) hi keeps 11 significant bits; below it hi
+    // is a multiple of 2^-24, the subnormal spacing.  A hi rounded to 11 bits in fp32 and only then converted would round a
+    // second time below 2^-14, up to 2^-25 that neither plane holds.  The split's error is <= 2^-22 |x| + 2^-36 (the last
+    // term: lo's own rounding in fp16's subnormal range).  The f32 -> f16 conversions run on the quarter-rate XU pipe shared
+    // with ex2/rcp, so they are issued packed (cvt.rn.f16x2.f32); hi - x is one mixed-precision add (kbs_add_f16_f32).
+    const __half2 h01 = __floats2half2_rn(x[0], x[1]), h23 = __floats2half2_rn(x[2], x[3]);
+    const float d0 = kbs_add_f16_f32(__low2half(h01), -x[0]), d1 = kbs_add_f16_f32(__high2half(h01), -x[1]);
+    const float d2 = kbs_add_f16_f32(__low2half(h23), -x[2]), d3 = kbs_add_f16_f32(__high2half(h23), -x[3]);
+    const __half2 l01 = __floats2half2_rn(d0 * -kKbsF16LoScale, d1 * -kKbsF16LoScale);
+    const __half2 l23 = __floats2half2_rn(d2 * -kKbsF16LoScale, d3 * -kKbsF16LoScale);
     s.hi = make_uint4(*reinterpret_cast<const uint32_t*>(&h01), *reinterpret_cast<const uint32_t*>(&h23), 0u, 0u);
     s.lo = make_uint4(*reinterpret_cast<const uint32_t*>(&l01), *reinterpret_cast<const uint32_t*>(&l23), 0u, 0u);
   }

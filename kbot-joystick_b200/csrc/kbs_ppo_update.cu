@@ -611,19 +611,22 @@ adamw_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restri
              const kbs_adamw_params o, const float* __restrict__ norm, const long long* __restrict__ step_dev, long long step) {
   const int64_t i = int64_t(blockIdx.x) * kT + threadIdx.x;
   if (i >= count) return;
-  float scale = o.grad_scale;
+  double scale = o.grad_scale;
   if (norm) {
     const float nn = norm[0] * o.grad_scale;                     // norm of the gradient the optimiser sees
     if (!(fabsf(nn) <= 3.0e38f)) return;                         // NaN / inf: ksim skips the update, optimiser state untouched
-    if (o.max_grad_norm > 0.0f && nn > o.max_grad_norm) scale = scale * (o.max_grad_norm / fmaxf(nn, 1e-6f));
+    if (o.max_grad_norm > 0.0f && nn > o.max_grad_norm)
+      scale = scale * (double(o.max_grad_norm) / fmax(double(norm[0]) * double(o.grad_scale), 1e-6));
   }
   const float s = float(step_dev ? step_dev[0] + 1 : step);
-  // optax.scale_by_adam: decay and (1 - decay) are Python doubles rounded to fp32 separately; bias correction 1 - decay^count in fp32
-  const float b1 = float(o.b1), b2 = float(o.b2), omb1 = float(1.0 - o.b1), omb2 = float(1.0 - o.b2);
+  // optax.scale_by_adam with the moments formed in double from the fp32 state and rounded once: b1 m and (1 - b1) g have
+  // either sign, and where they cancel an fp32 sum would keep an error of an ulp of the terms, many ulps of m.  Bias
+  // corrections 1 - decay^count in fp32 (decay rounded to fp32 as optax does).
+  const float b1 = float(o.b1), b2 = float(o.b2);
   const float bc1 = 1.0f - powf(b1, s), bc2 = 1.0f - powf(b2, s);
-  const float gi = g[i] * scale;
-  const float mi = b1 * m[i] + omb1 * gi;
-  const float vi = b2 * v[i] + omb2 * (gi * gi);
+  const double gi = double(g[i]) * scale;
+  const float mi = float(o.b1 * double(m[i]) + (1.0 - o.b1) * gi);
+  const float vi = float(o.b2 * double(v[i]) + (1.0 - o.b2) * (gi * gi));
   m[i] = mi; v[i] = vi;
   const float pi = p[i];
   p[i] = pi - o.lr * ((mi / bc1) / (sqrtf(vi / bc2) + o.eps) + o.weight_decay * pi);
@@ -1339,11 +1342,6 @@ int kbs_ppo_grad(kbs_handle* h, const kbs_ppo_loss_params* params, const kbs_ppo
   if (b->T <= 0 || n <= 0 || b->ld < n || (b->ld & 3)) return KBS_E_SHAPE;
   for (int k = 0; k < 2; ++k)
     if (!h->net[k].packed) return KBS_E_STATE;
-  // FP16-split above two layers: dG is pre-scaled by one power of two chosen from T n before its FP16 split, and the
-  // gradients of the lower layers of a deeper stack are orders of magnitude smaller than the top layer's.  Their dG lands in
-  // fp16's subnormal range: at depth 4, T = 1, n = 5 the critic's layer-0 blocks came out 3x beyond the bound the tests hold
-  // every other case to.  Refused rather than silently imprecise; 3xTF32 and SIMT take any depth.
-  if (h->p.gemm_path == KBS_GEMM_TC_2XF16 && h->p.depth > 2) return KBS_E_SHAPE;
   { const int rc0 = kbs_enter(h); if (rc0) return rc0; }
   cudaStream_t st = (cudaStream_t)stream;
   {

@@ -6,10 +6,9 @@ Depth is a task setting.  At depth 2 a layer loop that reads the wrong ping-pong
 two layers only, still gives the right answer.  The persistent tensor-core kernels hold at most two layers, so above depth 2
 the tensor-core datapaths run the per-step launches: the rollout's layer loop over the xmid slots (l - 1) & 1, the ABI-carry
 fallback (pack_rows + fb_convert, taken when nets x depth x 2 > 8: depth >= 3 with the critic), kbs_tc_lstm_stack's
-x_sb[l & 1] ping-pong (actor / critic / policy step), and the per-step PPO gradient on 3xTF32.  Depth 1 runs the persistent
-kernels with one layer.  Where a tensor-core entry point has no per-step form above depth 2 (dist.mean(), the mirror pass, the
-online step), and for the FP16-split PPO gradient above depth 2 (the lower layers' dG leaves the split's range), it refuses
-with KBS_E_SHAPE before it launches anything.
+x_sb[l & 1] ping-pong (actor / critic / policy step), and the per-step PPO gradient on 3xTF32 and FP16-split.  Depth 1 runs
+the persistent kernels with one layer.  Where a tensor-core entry point has no per-step form above depth 2 (dist.mean(), the
+mirror pass, the online step), it refuses with KBS_E_SHAPE before it launches anything.
 
 The worst scaled errors of the rollouts and the gradient block margins (block error / harness.block_bound, per layer) are
 printed, so `pytest -s` puts the precision margin of each datapath and depth on record."""
@@ -303,16 +302,18 @@ def test_ppo_variables(dev, path, depth, T, N, H, mirror):
 
 # ---- kbs_ppo_grad -------------------------------------------------------------------------------------------------------------
 
-# (path, per_step, depth, T, N, H, start); FP16-split at depth 1 runs the persistent update unless KBS_PPO_PER_STEP=1, and is
-# refused above depth 2 (test_ppo_grad_fp16_split_refused_above_depth_2)
+# (path, per_step, depth, T, N, H, start); FP16-split at depth 1 runs the persistent update unless KBS_PPO_PER_STEP=1; above
+# depth 2 it always runs the per-step launches.  The lower layers of a deeper stack have the smallest dG: at depth 4, T = 1,
+# n = 5 the critic's layer 0 sits deep below fp16's normal range in the FP16 split.
 GRAD_CASES = []
 for _d, _shapes in ((1, {"zero": (7, 70, 256), "warm": (6, 77, 256)}), (3, {"zero": (6, 129, 256), "warm": (5, 130, 128)}),
                     (4, {"zero": (7, 77, 256), "warm": (1, 5, 256)})):
-    for _path, _per_step in ((SIMT, False), (TF32, False)) + (((F16, False), (F16, True)) if _d == 1 else ()):
+    for _path, _per_step in ((SIMT, False), (TF32, False), (F16, False)) + (((F16, True),) if _d == 1 else ()):
         for _start, (_T, _N, _H) in _shapes.items():
             GRAD_CASES.append(pytest.param(_path, _per_step, _d, _T, _N, _H, _start,
                                            id=f"{NAMES[_path]}{'-per-step' if _per_step else ''}-d{_d}-{_start}-T{_T}xN{_N}xH{_H}"))
-GRAD_CASES.append(pytest.param(TF32, False, 4, 33, 300, 256, "warm", id="tc3xtf32-d4-warm-T33xN300xH256"))
+for _path in (TF32, F16):
+    GRAD_CASES.append(pytest.param(_path, False, 4, 33, 300, 256, "warm", id=f"{NAMES[_path]}-d4-warm-T33xN300xH256"))
 
 
 @pytest.mark.parametrize("path,per_step,depth,T,N,H,start", GRAD_CASES)
@@ -348,45 +349,12 @@ def test_ppo_grad(dev, path, per_step, depth, T, N, H, start, monkeypatch):
         assert_start_state_matters(ref, G.ppo_minibatch_grads(wa, wc, b, p), depth)
 
 
-@pytest.mark.parametrize("depth", [3, 4])
-@pytest.mark.parametrize("per_step", [False, True], ids=["default", "per-step"])
-def test_ppo_grad_fp16_split_refused_above_depth_2(dev, depth, per_step, monkeypatch):
-    """FP16-split splits dG after one power-of-two pre-scale chosen from T n; the lower layers of a 3- or 4-layer stack have
-    gradients small enough to land in fp16's subnormal range (at depth 4, T = 1, n = 5 the critic's layer 0 measured 3x
-    beyond its block bound).  kbs_ppo_grad refuses the shape with KBS_E_SHAPE, in either form, before launching anything:
-    the gradients stay as they were, the health word clear; PpoUpdater.update raises and its state does not move."""
-    monkeypatch.setenv("KBS_PPO_PER_STEP", "1" if per_step else "0")
-    T, N, H = 5, 77, 256
-    e, wa, wc = Hn.make_engine(hidden=H, depth=depth, gemm_path=F16, device=dev)
-    try:
-        b = Hn.ppo_batch(np.random.default_rng(5), T, N, H, O.OracleParams(hidden_size=H, depth=depth), wa, wc)
-        db = Hn.ppo_device_batch(b, dev)
-        up = PpoUpdater(e, wa, wc)
-        torch.cuda.synchronize()
-        ga, gc = up.pa.as_dict(torch.full_like(up.grad, float("nan"))[:up.na]), up.pc.as_dict(torch.full_like(up.grad, float("nan"))[up.na:])
-        snap = snapshot(up)
-        l0 = e.launches
-        with pytest.raises(RuntimeError, match=r"kbs_ppo_grad failed: \[-2\]"):
-            e.ppo_grad(db, ga, gc, n_envs=N)
-        with pytest.raises(RuntimeError, match=r"kbs_ppo_grad failed: \[-2\]"):
-            up.update(db, N)
-        torch.cuda.synchronize()
-        assert e.launches == l0
-        for g in (ga, gc):
-            for _, _, a in Hn.grad_tensors(g, depth):
-                assert np.isnan(a).all()
-        for k in ("param", "m", "v"):
-            assert torch.equal(getattr(up, k), snap[k]), k
-        assert up.step_count == 0 and e.device_status() == 0
-    finally:
-        e.close()
-
-
 # ---- PpoUpdater.update / epoch ---------------------------------------------------------------------------------------------------
 
 
 @pytest.mark.parametrize("path,depth,H", [pytest.param(TF32, 3, 128, id="tc3xtf32-d3"), pytest.param(TF32, 4, 256, id="tc3xtf32-d4"),
-                                          pytest.param(F16, 1, 256, id="tc2xf16-d1-persistent")])
+                                          pytest.param(F16, 1, 256, id="tc2xf16-d1-persistent"),
+                                          pytest.param(F16, 4, 256, id="tc2xf16-d4")])
 def test_ppo_update_against_float64_each_update(dev, path, depth, H, monkeypatch):
     """PpoUpdater with 1, 3 or 4 layers (its flat parameter vector, AdamW, the re-pack of every layer) update by update, each
     from the state the updater had before it, as test_gpu_ppo_update.test_ppo_update_against_float64_each_update; minibatches
