@@ -239,6 +239,26 @@ int kbs_ppo_grad(kbs_handle* h, const kbs_ppo_loss_params* params, const kbs_ppo
  * that point, so the caller can start reducing the critic's gradients on another stream while the actor's weight-gradient
  * GEMMs still run.  NULL clears it.  (The torch datapaths without the persistent kernels record it at the end.) */
 int kbs_ppo_grad_set_events(kbs_handle* h, void* critic_ready);
+/* Vector-Jacobian product of get_ppo_variables (train.py:1484-1487) on one minibatch: the gradient of a caller's loss, given
+ * its cotangents d loss / d (log_probs, values, entropy, action_std), back-propagated through the same forward and BPTT as
+ * kbs_ppo_grad.  Writes into actor / critic (layout of kbs_ppo_grad) sum_{t,e} ct . d var / d theta at the weights packed in
+ * the handle, and the forward's log_probs / values / entropy [T][ld] (bitwise those of kbs_ppo_grad on the same batch).
+ *   batch: as kbs_ppo_grad; old_log_probs, advantages, value_targets and old_values are not read (may be NULL).  The start
+ *          carries, observations, actions and done are constants.  No mirror pass.
+ *   ct: any member may be NULL (= zero cotangent).
+ * Same datapaths as kbs_ppo_grad, selected the same way; honours kbs_ppo_grad_set_events; no host synchronisation (capturable).
+ * Each network's cotangents are scaled on the device by a power of two chosen from their largest magnitude, and its gradients
+ * by the inverse (exact), so any loss scale suits the FP16-split datapath: VJP(2^k ct) == 2^k VJP(ct) bitwise while nothing
+ * leaves the normal range.  All-zero cotangents give zero gradients; a non-finite one propagates into its network's gradient. */
+typedef struct kbs_ppo_cotangents {
+  const float* log_probs;   /* [T][ld] */
+  const float* values;      /* [T][ld] */
+  const float* entropy;     /* [T][ld] */
+  const float* action_std;  /* [T][20][ld] */
+} kbs_ppo_cotangents;
+int kbs_ppo_variables_vjp(kbs_handle* h, const kbs_ppo_batch* batch, const kbs_ppo_cotangents* ct, const kbs_net_grads* actor,
+                          const kbs_net_grads* critic, float* log_probs, float* values, float* entropy, int64_t n_envs,
+                          void* stream);
 /* Replaces: optax.adam -- the adam_weight_decay == 0.0 branch of get_optimizer (train.py:1062-1063; NOT the branch the launch
  * config takes: see kbs_adamw_step): scale_by_adam, eps_root = 0, then -learning_rate, on one flat parameter array: g = grad * grad_scale (1 / world_size after a sum all-reduce, or a global-norm clip factor);
  * m = b1 m + (1 - b1) g; v = b2 v + (1 - b2) g^2; p -= lr (m / (1 - b1^step)) / (sqrt(v / (1 - b2^step)) + eps).  step >= 1. */

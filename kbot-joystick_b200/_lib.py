@@ -159,6 +159,10 @@ class KbsNetGrads(C.Structure):
                 ("w_out", _vp), ("b_out", _vp)]
 
 
+class KbsPpoCotangents(C.Structure):
+    _fields_ = [(k, _vp) for k in ("log_probs", "values", "entropy", "action_std")]
+
+
 # every symbol include/kbotstep.h declares (tests check the .so exports all of them)
 EXPORTS = (
     "kbs_version", "kbs_error_string", "kbs_default_params", "kbs_create", "kbs_destroy", "kbs_get_params",
@@ -169,7 +173,7 @@ EXPORTS = (
     "kbs_sample_actuator_randomization", "kbs_device_status_reset", "kbs_ppo_grad_set_events", "kbs_generate_rollout_noise",
     "kbs_minibatch_permutation", "kbs_shuffle_minibatches", "kbs_rollout_record", "kbs_step_state_bytes", "kbs_step_state_load",
     "kbs_step_state_store", "kbs_step_state_rewind", "kbs_rollout_step", "kbs_actuator_state_bytes", "kbs_actuator_state_load",
-    "kbs_actuator_state_store", "kbs_actuator_substep",
+    "kbs_actuator_state_store", "kbs_actuator_substep", "kbs_ppo_variables_vjp",
 )
 VERSION = 101
 STATUS_TIMEOUT_LSTM, STATUS_TIMEOUT_HEAD, STATUS_F16_RANGE, STATUS_STEP_RANGE = 1, 2, 0x100, 0x200
@@ -210,6 +214,8 @@ def load() -> C.CDLL:
     lib.kbs_adamw_default_params.argtypes = [P(KbsAdamwParams)]
     lib.kbs_adamw_step.argtypes = [_vp, _vp, _vp, _vp, _vp, _i64, P(KbsAdamwParams), _vp, _vp, _i64, _vp]
     lib.kbs_ppo_grad_set_events.argtypes = [_vp, _vp]
+    lib.kbs_ppo_variables_vjp.argtypes = [_vp, P(KbsPpoBatch), P(KbsPpoCotangents), P(KbsNetGrads), P(KbsNetGrads), _vp, _vp,
+                                          _vp, _i64, _vp]
     lib.kbs_generate_rollout_noise.argtypes = [_vp, C.c_uint64, _i64, P(KbsNoiseView), _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _vp]
     lib.kbs_grad_norm.argtypes = [_vp, _vp, _i64, _vp, _vp]
     lib.kbs_minibatch_permutation.argtypes = [_vp, C.c_uint64, _vp, _i64, _vp, _i64, _vp]

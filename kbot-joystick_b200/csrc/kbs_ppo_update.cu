@@ -213,14 +213,67 @@ __device__ __forceinline__ float policy_dlogp(float r, float rc, float dr, float
   return (inside || r * a < rc * a) ? a * dr : (isfinite(a) ? 0.0f : a);
 }
 
+// Cotangent mode of the heads (kbs_ppo_variables_vjp, template flag CT): d / d(log-prob, value, entropy, action std) come from
+// the caller instead of the loss.  Each network's cotangents are multiplied by a power of two s taken from their largest
+// magnitude (ct_scale), so that the BPTT sees them at the size a mean loss gives them -- the FP16-split planes (and gscale)
+// assume that size -- and the finished gradients are multiplied by 1 / s (grad_rescale_kernel).  Both products are exact, so
+// VJP(2^k ct) == 2^k VJP(ct) bitwise while everything stays in the normal range.
+struct HeadCt {
+  kbs_ppo_cotangents c;
+  const unsigned int* amax;   // [2]: float bits of max |ct| over the actor's (log-prob, entropy, std) / the critic's (value)
+  int rexp;                   // ceil(log2(T n))
+};
+
+// s with s max|ct| in [1, 2) / 2^rexp (a mean over T n rows of per-row cotangents of order one).  All-zero cotangents, and a
+// non-finite one (its bits are >= those of inf, and atomicMax keeps them), give s = 1: a NaN propagates into the gradient,
+// where the updater's non-finite skip sees it.
+__device__ __forceinline__ float ct_scale(unsigned int bits, int rexp) {
+  if (bits == 0u || bits >= 0x7f800000u) return 1.0f;
+  int e;
+  frexpf(__uint_as_float(bits), &e);                    // max = f 2^e, f in [0.5, 1)
+  const int k = max(-126, min(127, 1 - e - rexp));
+  return __int_as_float((k + 127) << 23);
+}
+
+// max |ct| per network as float bits (order-free, so deterministic).  blockIdx.y = array (log-prob, entropy, std, value), the
+// grid strides over its rows x n; rows of the padding (e >= n) are never read.
+__global__ void __launch_bounds__(kT)
+ct_absmax_kernel(const kbs_ppo_cotangents c, unsigned int* __restrict__ amax, int64_t T, int64_t ld, int64_t n) {
+  const int a = blockIdx.y;
+  const float* p = a == 0 ? c.log_probs : a == 1 ? c.entropy : a == 2 ? c.action_std : c.values;
+  if (!p) return;
+  const int64_t count = (a == 2 ? T * KBS_NUM_JOINTS : T) * n;
+  unsigned int m = 0u;
+  for (int64_t i = int64_t(blockIdx.x) * kT + threadIdx.x; i < count; i += int64_t(gridDim.x) * kT) {
+    const int64_t r = i / n, e = i - r * n;
+    m = max(m, __float_as_uint(p[r * ld + e]) & 0x7fffffffu);
+  }
+#pragma unroll
+  for (int s = 16; s > 0; s >>= 1) m = max(m, __shfl_xor_sync(0xffffffffu, m, s));
+  if ((threadIdx.x & 31) == 0 && m) atomicMax(amax + (a == 3 ? 1 : 0), m);
+}
+
+// the gradient tensors of one network, multiplied by 1 / s once they are final (blockIdx.y = tensor)
+struct GradList {
+  float* p[3 * KBS_MAX_DEPTH + 4];
+  int64_t count[3 * KBS_MAX_DEPTH + 4];
+};
+__global__ void __launch_bounds__(kT)
+grad_rescale_kernel(const GradList g, const unsigned int* __restrict__ amax, int rexp) {
+  const float inv = 1.0f / ct_scale(amax[0], rexp);     // a power of two: exact
+  float* p = g.p[blockIdx.y];
+  for (int64_t i = int64_t(blockIdx.x) * kT + threadIdx.x; i < g.count[blockIdx.y]; i += int64_t(gridDim.x) * kT) p[i] *= inv;
+}
+
 // The same head with one WARP per env (lane j = joint j, log-prob / entropy by warp shuffles): the one-thread-per-env form
 // above was 3.5 ms of an 18 ms update (512 threads walking 2 x T steps x 20 joints of libm math and strided loads).
 // The steps are taken in chunks of kHC: every input of a chunk is loaded first (none depends on the filter's recurrence), then
 // the chunk's steps run out of registers -- one L2 round trip per chunk instead of per step (there are only ~3 warps per SM at
 // 512 envs, so nothing else hides the latency: 0.24 -> 0.07 ms per 512 x 100).  Same operations in the same order as before.
 constexpr int kHC = 10;
+template <bool CT>
 __global__ void __launch_bounds__(128)
-actor_head_fwd_bwd_warp_kernel(const __grid_constant__ kbs_params P, kbs_ppo_loss_params L, const float* __restrict__ out,
+actor_head_fwd_bwd_warp_kernel(const __grid_constant__ kbs_params P, kbs_ppo_loss_params L, const HeadCt ct, const float* __restrict__ out,
                                const float* __restrict__ actor_obs, const float* __restrict__ action,
                                const uint8_t* __restrict__ done, const float* __restrict__ lpf0, const float* __restrict__ old_lp,
                                const float* __restrict__ adv, float* __restrict__ y_s, float* __restrict__ sd_s,
@@ -278,16 +331,26 @@ actor_head_fwd_bwd_warp_kernel(const __grid_constant__ kbs_params P, kbs_ppo_los
   __syncwarp();
   const float inv = 1.0f / (float(T) * float(n));
   float gy = 0.0f;
+  float cs = 1.0f;
+  if constexpr (CT) cs = ct_scale(ct.amax[0], ct.rexp);
   for (int64_t t1 = T; t1 > 0; t1 -= kHC) {             // chunk = steps t1 - 1 down to t1 - kHC
-    float lp[kHC], ol[kHC], av[kHC], sdv[kHC], yv[kHC], ac[kHC], os[kHC];
+    float lp[kHC], ol[kHC], av[kHC], sdv[kHC], yv[kHC], ac[kHC], os[kHC], cst[kHC];
     uint8_t dn[kHC];
 #pragma unroll
     for (int i = 0; i < kHC; ++i) {
       const int64_t t = (t1 - 1 - i >= 0) ? t1 - 1 - i : 0;
       const int64_t so = (t * KBS_NUM_JOINTS + jj) * ld + e;
-      lp[i] = log_prob[t * ld + e];
-      ol[i] = old_lp[t * ld + e];
-      av[i] = adv[t * ld + e];
+      if constexpr (CT) {                               // ol / av hold the log-prob / entropy cotangents
+        lp[i] = 0.0f;
+        ol[i] = ct.c.log_probs ? ct.c.log_probs[t * ld + e] : 0.0f;
+        av[i] = ct.c.entropy ? ct.c.entropy[t * ld + e] : 0.0f;
+        cst[i] = ct.c.action_std ? ct.c.action_std[so] : 0.0f;
+      } else {
+        lp[i] = log_prob[t * ld + e];
+        ol[i] = old_lp[t * ld + e];
+        av[i] = adv[t * ld + e];
+        cst[i] = 0.0f;
+      }
       dn[i] = done[t * ld + e];
       sdv[i] = sd_s[so];
       yv[i] = y_s[so];
@@ -298,22 +361,29 @@ actor_head_fwd_bwd_warp_kernel(const __grid_constant__ kbs_params P, kbs_ppo_los
     for (int i = 0; i < kHC; ++i) {
       const int64_t t = t1 - 1 - i;
       if (t < 0) break;
-      const float lr = lp[i] - ol[i];
-      const float lrc = fminf(fmaxf(lr, -L.log_clip_value), L.log_clip_value);
-      const float r = expf(lrc);
-      const float a = av[i];
-      const float dr = (fabsf(lr) <= L.log_clip_value) ? r : 0.0f;
-      const bool inside = r >= 1.0f - L.clip_param && r <= 1.0f + L.clip_param;
-      const float rc = fminf(fmaxf(r, 1.0f - L.clip_param), 1.0f + L.clip_param);
-      const float dpol = policy_dlogp(r, rc, dr, a, inside);
-      const float glp = -inv * dpol, gent = -inv * L.entropy_coef;
+      float glp, gent;
+      if constexpr (CT) {
+        glp = cs * ol[i];
+        gent = cs * av[i];
+      } else {
+        const float lr = lp[i] - ol[i];
+        const float lrc = fminf(fmaxf(lr, -L.log_clip_value), L.log_clip_value);
+        const float r = expf(lrc);
+        const float a = av[i];
+        const float dr = (fabsf(lr) <= L.log_clip_value) ? r : 0.0f;
+        const bool inside = r >= 1.0f - L.clip_param && r <= 1.0f + L.clip_param;
+        const float rc = fminf(fmaxf(r, 1.0f - L.clip_param), 1.0f + L.clip_param);
+        const float dpol = policy_dlogp(r, rc, dr, a, inside);
+        glp = -inv * dpol; gent = -inv * L.entropy_coef;
+      }
       const float keep = dn[i] ? 0.0f : 1.0f;
       float* d = dout + (t * n + e) * 64;
       if (act) {
         const float sd = sdv[i], yy = yv[i];
         const float z = (ac[i] - yy) / sd;
         const float dmu = glp * z / sd;
-        const float dsd = (glp * (z * z - 1.0f) + gent) / sd;
+        float dsd = (glp * (z * z - 1.0f) + gent) / sd;
+        if constexpr (CT) { if (ct.c.action_std) dsd += cs * cst[i]; }
         const float sraw = os[i];
         const float sp = fmaxf(sraw, 0.0f) + log1pf(expf(-fabsf(sraw)));
         const bool clamped = (sp + P.min_std) * P.var_scale > P.max_std;
@@ -331,8 +401,9 @@ actor_head_fwd_bwd_warp_kernel(const __grid_constant__ kbs_params P, kbs_ppo_los
 // around two cheap sequential scans by warp 0 (the filter forward: one FMA per step; its adjoint backward).  Every element sees
 // the same operations in the same order as in the warp-per-env form: identical results; 0.115 -> 0.05 ms per 512 x 100.
 // Shared memory: 3 x [T][32] floats + [T] bytes (38.5 KB at T = 100); the launcher falls back to the warp form beyond 48 KB.
+template <bool CT>
 __global__ void __launch_bounds__(128)
-actor_head_fwd_bwd_block_kernel(const __grid_constant__ kbs_params P, kbs_ppo_loss_params L, const float* __restrict__ out,
+actor_head_fwd_bwd_block_kernel(const __grid_constant__ kbs_params P, kbs_ppo_loss_params L, const HeadCt ct, const float* __restrict__ out,
                                 const float* __restrict__ actor_obs, const float* __restrict__ action,
                                 const uint8_t* __restrict__ done, const float* __restrict__ lpf0, const float* __restrict__ old_lp,
                                 const float* __restrict__ adv, float* __restrict__ y_s, float* __restrict__ sd_s,
@@ -396,14 +467,23 @@ actor_head_fwd_bwd_block_kernel(const __grid_constant__ kbs_params P, kbs_ppo_lo
   __syncthreads();
   // ---- phase 3: log-prob / entropy, the loss gradient, its way back through the Gaussian and softplus + clamp ----
   const float inv = 1.0f / (float(T) * float(n));
+  float cs = 1.0f;
+  if constexpr (CT) cs = ct_scale(ct.amax[0], ct.rexp);
   for (int64_t tb = w; tb < T; tb += 4 * kPB) {
-    float i_ac[kPB], i_ol[kPB], i_av[kPB], i_os[kPB];
+    float i_ac[kPB], i_ol[kPB], i_av[kPB], i_os[kPB], i_cs[kPB];
 #pragma unroll
     for (int i = 0; i < kPB; ++i) {
       const int64_t t = (tb + 4 * i < T) ? tb + 4 * i : T - 1;
       i_ac[i] = action[(t * KBS_NUM_JOINTS + jj) * ld + e];
-      i_ol[i] = old_lp[t * ld + e];
-      i_av[i] = adv[t * ld + e];
+      if constexpr (CT) {                               // i_ol / i_av hold the log-prob / entropy cotangents
+        i_ol[i] = ct.c.log_probs ? ct.c.log_probs[t * ld + e] : 0.0f;
+        i_av[i] = ct.c.entropy ? ct.c.entropy[t * ld + e] : 0.0f;
+        i_cs[i] = ct.c.action_std ? ct.c.action_std[(t * KBS_NUM_JOINTS + jj) * ld + e] : 0.0f;
+      } else {
+        i_ol[i] = old_lp[t * ld + e];
+        i_av[i] = adv[t * ld + e];
+        i_cs[i] = 0.0f;
+      }
       i_os[i] = out[(t * n + e) * 64 + KBS_NUM_JOINTS + jj];
     }
 #pragma unroll
@@ -424,20 +504,27 @@ actor_head_fwd_bwd_block_kernel(const __grid_constant__ kbs_params P, kbs_ppo_lo
         log_prob[t * ld + e] = lp;
         entropy[t * ld + e] = tl + float(KBS_NUM_JOINTS) * (0.5f + kHalfLog2Pi);
       }
-      const float lr = lp - i_ol[i];
-      const float lrc = fminf(fmaxf(lr, -L.log_clip_value), L.log_clip_value);
-      const float r = expf(lrc);
-      const float a = i_av[i];
-      const float dr = (fabsf(lr) <= L.log_clip_value) ? r : 0.0f;
-      const bool inside = r >= 1.0f - L.clip_param && r <= 1.0f + L.clip_param;
-      const float rc = fminf(fmaxf(r, 1.0f - L.clip_param), 1.0f + L.clip_param);
-      const float dpol = policy_dlogp(r, rc, dr, a, inside);
-      const float glp = -inv * dpol, gent = -inv * L.entropy_coef;
+      float glp, gent;
+      if constexpr (CT) {
+        glp = cs * i_ol[i];
+        gent = cs * i_av[i];
+      } else {
+        const float lr = lp - i_ol[i];
+        const float lrc = fminf(fmaxf(lr, -L.log_clip_value), L.log_clip_value);
+        const float r = expf(lrc);
+        const float a = i_av[i];
+        const float dr = (fabsf(lr) <= L.log_clip_value) ? r : 0.0f;
+        const bool inside = r >= 1.0f - L.clip_param && r <= 1.0f + L.clip_param;
+        const float rc = fminf(fmaxf(r, 1.0f - L.clip_param), 1.0f + L.clip_param);
+        const float dpol = policy_dlogp(r, rc, dr, a, inside);
+        glp = -inv * dpol; gent = -inv * L.entropy_coef;
+      }
       float* d = dout + (t * n + e) * 64;
       float dmu = 0.0f;
       if (act) {
         dmu = glp * z / sd;
-        const float dsd = (glp * (z * z - 1.0f) + gent) / sd;
+        float dsd = (glp * (z * z - 1.0f) + gent) / sd;
+        if constexpr (CT) { if (ct.c.action_std) dsd += cs * i_cs[i]; }
         const float sraw = i_os[i];
         const float sp = fmaxf(sraw, 0.0f) + log1pf(expf(-fabsf(sraw)));
         const bool clamped = (sp + P.min_std) * P.var_scale > P.max_std;
@@ -463,8 +550,9 @@ actor_head_fwd_bwd_block_kernel(const __grid_constant__ kbs_params P, kbs_ppo_lo
 // produced log-prob / entropy / std / filtered mean / raw std output per step ([T][.][ld]); one warp per env (lane = joint)
 // walks the steps backwards through the loss gradient, the Gaussian, softplus + clamp and the low-pass filter's recurrence
 // (done-resets included).  dout [T*n][64] row-major: columns 0..19 = d loss / d mean output, 20..39 = d / d std output, rest 0.
+template <bool CT>
 __global__ void __launch_bounds__(128)
-actor_head_bwd_warp_kernel(const __grid_constant__ kbs_params P, kbs_ppo_loss_params L, const float* __restrict__ action,
+actor_head_bwd_warp_kernel(const __grid_constant__ kbs_params P, kbs_ppo_loss_params L, const HeadCt ct, const float* __restrict__ action,
                            const uint8_t* __restrict__ done, const float* __restrict__ old_lp, const float* __restrict__ adv,
                            const float* __restrict__ y_s, const float* __restrict__ sd_s, const float* __restrict__ sraw_s,
                            const float* __restrict__ log_prob, float* __restrict__ dout, int64_t T, int64_t ld, int64_t n) {
@@ -473,17 +561,25 @@ actor_head_bwd_warp_kernel(const __grid_constant__ kbs_params P, kbs_ppo_loss_pa
   const int j = threadIdx.x & 31;
   const bool act = j < KBS_NUM_JOINTS;
   const float inv = 1.0f / (float(T) * float(n));
+  float cs = 1.0f;
+  if constexpr (CT) cs = ct_scale(ct.amax[0], ct.rexp);
   float gy = 0.0f;
   for (int64_t t = T - 1; t >= 0; --t) {
-    const float lr = log_prob[t * ld + e] - old_lp[t * ld + e];
-    const float lrc = fminf(fmaxf(lr, -L.log_clip_value), L.log_clip_value);
-    const float r = expf(lrc);
-    const float a = adv[t * ld + e];
-    const float dr = (fabsf(lr) <= L.log_clip_value) ? r : 0.0f;
-    const bool inside = r >= 1.0f - L.clip_param && r <= 1.0f + L.clip_param;
-    const float rc = fminf(fmaxf(r, 1.0f - L.clip_param), 1.0f + L.clip_param);
-    const float dpol = policy_dlogp(r, rc, dr, a, inside);
-    const float glp = -inv * dpol, gent = -inv * L.entropy_coef;
+    float glp, gent;
+    if constexpr (CT) {
+      glp = ct.c.log_probs ? cs * ct.c.log_probs[t * ld + e] : 0.0f;
+      gent = ct.c.entropy ? cs * ct.c.entropy[t * ld + e] : 0.0f;
+    } else {
+      const float lr = log_prob[t * ld + e] - old_lp[t * ld + e];
+      const float lrc = fminf(fmaxf(lr, -L.log_clip_value), L.log_clip_value);
+      const float r = expf(lrc);
+      const float a = adv[t * ld + e];
+      const float dr = (fabsf(lr) <= L.log_clip_value) ? r : 0.0f;
+      const bool inside = r >= 1.0f - L.clip_param && r <= 1.0f + L.clip_param;
+      const float rc = fminf(fmaxf(r, 1.0f - L.clip_param), 1.0f + L.clip_param);
+      const float dpol = policy_dlogp(r, rc, dr, a, inside);
+      glp = -inv * dpol; gent = -inv * L.entropy_coef;
+    }
     const float keep = done[t * ld + e] ? 0.0f : 1.0f;
     float* d = dout + (t * n + e) * 64;
     if (act) {
@@ -491,7 +587,8 @@ actor_head_bwd_warp_kernel(const __grid_constant__ kbs_params P, kbs_ppo_loss_pa
       const float sd = sd_s[so], yy = y_s[so];
       const float z = (action[so] - yy) / sd;
       const float dmu = glp * z / sd;
-      const float dsd = (glp * (z * z - 1.0f) + gent) / sd;
+      float dsd = (glp * (z * z - 1.0f) + gent) / sd;
+      if constexpr (CT) { if (ct.c.action_std) dsd += cs * ct.c.action_std[so]; }
       const float sraw = sraw_s[so];
       const float sp = fmaxf(sraw, 0.0f) + log1pf(expf(-fabsf(sraw)));
       const bool clamped = (sp + P.min_std) * P.var_scale > P.max_std;
@@ -504,31 +601,37 @@ actor_head_bwd_warp_kernel(const __grid_constant__ kbs_params P, kbs_ppo_loss_pa
 }
 
 // ... and of the critic head: values [T][ld] came from the forward pass
+template <bool CT>
 __global__ void __launch_bounds__(kT)
-critic_head_bwd_kernel(kbs_ppo_loss_params L, const float* __restrict__ values, const float* __restrict__ old_values,
+critic_head_bwd_kernel(kbs_ppo_loss_params L, const HeadCt ct, const float* __restrict__ values, const float* __restrict__ old_values,
                        const float* __restrict__ targets, float* __restrict__ dout, int64_t T, int64_t ld, int64_t n) {
   const int64_t idx = int64_t(blockIdx.x) * kT + threadIdx.x;
   if (idx >= T * n) return;
   const int64_t t = idx / n, e = idx - t * n;
-  const float v = values[t * ld + e];
-  const float tgt = targets[t * ld + e];
-  const float err = tgt - v;
-  float dval = -err;
-  if (L.use_clipped_value_loss) {
-    const float vo = old_values[t * ld + e];
-    const float dv = v - vo;
-    const float errc = tgt - (vo + fminf(fmaxf(dv, -L.clip_param), L.clip_param));
-    if (fabsf(dv) > L.clip_param) dval = (err * err > errc * errc) ? -err : 0.0f;
-  }
   float* d = dout + idx * 64;
-  d[0] = L.value_loss_coef * dval / (float(T) * float(n));
+  if constexpr (CT) {
+    d[0] = ct.c.values ? ct_scale(ct.amax[1], ct.rexp) * ct.c.values[t * ld + e] : 0.0f;
+  } else {
+    const float v = values[t * ld + e];
+    const float tgt = targets[t * ld + e];
+    const float err = tgt - v;
+    float dval = -err;
+    if (L.use_clipped_value_loss) {
+      const float vo = old_values[t * ld + e];
+      const float dv = v - vo;
+      const float errc = tgt - (vo + fminf(fmaxf(dv, -L.clip_param), L.clip_param));
+      if (fabsf(dv) > L.clip_param) dval = (err * err > errc * errc) ? -err : 0.0f;
+    }
+    d[0] = L.value_loss_coef * dval / (float(T) * float(n));
+  }
 #pragma unroll
   for (int j = 1; j < 64; ++j) d[j] = 0.0f;
 }
 
 // Critic head: value_t = out[t][e][0]; dout[.][0] = d loss / d value (clipped value loss), other columns zero.
+template <bool CT>
 __global__ void __launch_bounds__(kT)
-critic_head_fwd_bwd_kernel(kbs_ppo_loss_params L, const float* __restrict__ out, const float* __restrict__ old_values,
+critic_head_fwd_bwd_kernel(kbs_ppo_loss_params L, const HeadCt ct, const float* __restrict__ out, const float* __restrict__ old_values,
                            const float* __restrict__ targets, float* __restrict__ values, float* __restrict__ dout, int64_t T,
                            int64_t ld, int64_t n) {
   const int64_t idx = int64_t(blockIdx.x) * kT + threadIdx.x;
@@ -536,17 +639,21 @@ critic_head_fwd_bwd_kernel(kbs_ppo_loss_params L, const float* __restrict__ out,
   const int64_t t = idx / n, e = idx - t * n;
   const float v = out[idx * 64];
   values[t * ld + e] = v;
-  const float tgt = targets[t * ld + e];
-  const float err = tgt - v;
-  float dval = -err;                                        // d (0.5 err^2) / d v
-  if (L.use_clipped_value_loss) {
-    const float vo = old_values[t * ld + e];
-    const float dv = v - vo;
-    const float errc = tgt - (vo + fminf(fmaxf(dv, -L.clip_param), L.clip_param));
-    if (fabsf(dv) > L.clip_param) dval = (err * err > errc * errc) ? -err : 0.0f;   // the clipped branch has no gradient
-  }
   float* d = dout + idx * 64;
-  d[0] = L.value_loss_coef * dval / (float(T) * float(n));
+  if constexpr (CT) {
+    d[0] = ct.c.values ? ct_scale(ct.amax[1], ct.rexp) * ct.c.values[t * ld + e] : 0.0f;
+  } else {
+    const float tgt = targets[t * ld + e];
+    const float err = tgt - v;
+    float dval = -err;                                        // d (0.5 err^2) / d v
+    if (L.use_clipped_value_loss) {
+      const float vo = old_values[t * ld + e];
+      const float dv = v - vo;
+      const float errc = tgt - (vo + fminf(fmaxf(dv, -L.clip_param), L.clip_param));
+      if (fabsf(dv) > L.clip_param) dval = (err * err > errc * errc) ? -err : 0.0f;   // the clipped branch has no gradient
+    }
+    d[0] = L.value_loss_coef * dval / (float(T) * float(n));
+  }
 #pragma unroll
   for (int j = 1; j < 64; ++j) d[j] = 0.0f;
 }
@@ -555,8 +662,9 @@ critic_head_fwd_bwd_kernel(kbs_ppo_loss_params L, const float* __restrict__ out,
 // the padded 64-column GEMM), the clipped value loss' gradient, dout row (column 0 = d loss / d value: the A operand of the
 // dW_out GEMM) and dv [T * n] -- the backward kernel forms dh_top = dv w_out itself (rank 1), so neither `out` nor `dh_top` of
 // the critic exist.  One warp per (t, env) row.
+template <bool CT>
 __global__ void __launch_bounds__(256)
-critic_value_head_kernel(kbs_ppo_loss_params L, const float* __restrict__ h_top, const float* __restrict__ w_out,
+critic_value_head_kernel(kbs_ppo_loss_params L, const HeadCt ct, const float* __restrict__ h_top, const float* __restrict__ w_out,
                          const float* __restrict__ b_out, const float* __restrict__ old_values, const float* __restrict__ targets,
                          float* __restrict__ values, float* __restrict__ dout, float* __restrict__ dv, int H, int64_t T, int64_t ld,
                          int64_t n) {
@@ -574,7 +682,11 @@ critic_value_head_kernel(kbs_ppo_loss_params L, const float* __restrict__ h_top,
   const int64_t t = idx / n, e = idx - t * n;
   const float v = acc + b_out[0];
   float dval = 0.0f;
-  if (lane == 0) {
+  if (lane == 0 && CT) {
+    values[t * ld + e] = v;
+    dval = ct.c.values ? ct_scale(ct.amax[1], ct.rexp) * ct.c.values[t * ld + e] : 0.0f;
+    dv[idx] = dval;
+  } else if (lane == 0) {
     values[t * ld + e] = v;
     const float tgt = targets[t * ld + e];
     const float err = tgt - v;
@@ -863,6 +975,40 @@ int run_net(kbs_handle* h, int net, const kbs_ppo_batch& b, const float* carry0,
   return run_net_k<KBS_KIND_F16>(h, net, b, carry0, w, gates_pre, dc_rec, part, splits, n, st, backward, g, tc);
 }
 
+// ---- cotangent mode (kbs_ppo_variables_vjp): the heads' HeadCt, max |ct| per network before the heads, 1 / s after the
+// weight-gradient reductions.  c == nullptr: loss mode (kbs_ppo_grad), nothing is launched. ----
+int ct_begin(kbs_handle* h, const kbs_ppo_cotangents* c, unsigned int* amax, int64_t T, int64_t ld, int64_t n, cudaStream_t st,
+             HeadCt* hc) {
+  *hc = HeadCt{};
+  if (!c) return KBS_OK;
+  hc->c = *c;
+  hc->amax = amax;
+  while ((int64_t(1) << hc->rexp) < T * n) ++hc->rexp;
+  KBS_CUDA_TRY(cudaMemsetAsync(amax, 0, 2 * sizeof(unsigned int), st));
+  const int64_t gx = (T * KBS_NUM_JOINTS * n + kT - 1) / kT;
+  KBS_LAUNCH(h, KBS_K_ADV_NORM, st, (ct_absmax_kernel<<<dim3(unsigned(gx < 592 ? gx : 592), 4), kT, 0, st>>>(*c, amax, T, ld, n)));
+  KBS_LAUNCH_CHECK();
+  return KBS_OK;
+}
+int ct_rescale(kbs_handle* h, const HeadCt& hc, int net, const kbs_net_grads* g, cudaStream_t st) {
+  if (!hc.amax) return KBS_OK;
+  const KbsNet& N = h->net[net];
+  const int64_t H = h->p.hidden_size;
+  GradList L{};
+  int k = 0;
+  auto add = [&](float* p, int64_t count) { L.p[k] = p; L.count[k] = count; ++k; };
+  add(g->w_in, H * N.num_in);
+  add(g->b_in, H);
+  for (int l = 0; l < h->p.depth; ++l) { add(g->w_ih[l], 4 * H * H); add(g->w_hh[l], 4 * H * H); add(g->b[l], 4 * H); }
+  add(g->w_out, int64_t(N.num_out) * H);
+  add(g->b_out, N.num_out);
+  const int64_t gx = (4 * H * H + kT - 1) / kT;
+  KBS_LAUNCH(h, KBS_K_ADV_NORM, st,
+             (grad_rescale_kernel<<<dim3(unsigned(gx < 128 ? gx : 128), unsigned(k)), kT, 0, st>>>(L, hc.amax + net, hc.rexp)));
+  KBS_LAUNCH_CHECK();
+  return KBS_OK;
+}
+
 // ---- the persistent form of kbs_ppo_grad (FP16-split datapath) ---------------------------------------------------------
 // main stream: input projections (tensor core, straight from the SoA observations) -> lstm_fwd_save_kernel (ALL T steps of both
 // networks' LSTM stacks, one launch; keeps operands, cell states, activated gates) -> heads (actor: FFMA GEMM + one warp per env
@@ -887,7 +1033,8 @@ struct PersistWork {
 };
 
 int ppo_grad_persistent(kbs_handle* h, const kbs_ppo_loss_params& L, const kbs_ppo_batch& b, const kbs_net_grads* const* grads,
-                        float* log_probs, float* values, float* entropy, float* stats_out, int64_t n, cudaStream_t st) {
+                        float* log_probs, float* values, float* entropy, float* stats_out, int64_t n, cudaStream_t st,
+                        const kbs_ppo_cotangents* ct) {
   const int H = h->p.hidden_size, depth = h->p.depth;
   const int64_t T = b.T, ld = b.ld, rows = T * n, np = (n + 127) / 128 * 128;
   const size_t npH = size_t(np) * H;
@@ -896,6 +1043,7 @@ int ppo_grad_persistent(kbs_handle* h, const kbs_ppo_loss_params& L, const kbs_p
   KbsTcRolloutWs rws;
   float* osb[2]; float *y_s, *sd_s, *sraw_s, *lpf;
   double* loss_part;
+  unsigned int* amax;
   PersistWork w[2];
   int rc = kbs_scratch(h, [&](KbsScratch& s) {
     rws = kbs_tc_rollout_ws(s, h, n, 2);
@@ -933,8 +1081,11 @@ int ppo_grad_persistent(kbs_handle* h, const kbs_ppo_loss_params& L, const kbs_p
       w[k].tnb_obs = s.take<char>(kpp / 128 * plan.col_bytes);
       for (int l = 0; l < depth; ++l) w[k].tna_dG[l] = s.take<char>(size_t(4 * H / 128) * plan.col_bytes);
     }
+    amax = s.take<unsigned int>(2);
   });
   if (rc) return rc;
+  HeadCt hc;
+  if ((rc = ct_begin(h, ct, amax, T, ld, n, st, &hc))) return rc;
   // ---- forward ----
   // narrow-tile kernel (lstm_fwd_save_kernel: LSTM stacks only, heads as a batched GEMM + per-env scan afterwards) unless
   // KBS_PPO_FWD_WIDE=1 asks for rollout_persist_kernel<SAVE> (128 x 256 tiles, heads fused: the first version, kept for A/B)
@@ -1011,24 +1162,24 @@ int ppo_grad_persistent(kbs_handle* h, const kbs_ppo_loss_params& L, const kbs_p
       if (block_head < 0) { const char* e = getenv("KBS_PPO_HEAD_BLOCK"); block_head = e ? atoi(e) : 1; }
       if (block_head && head_smem <= 48 * 1024)
         KBS_LAUNCH(h, KBS_K_ACTOR_HEAD, st,
-                   (actor_head_fwd_bwd_block_kernel<<<unsigned(n), 128, head_smem, st>>>(
-                       h->p, L, w[0].out, b.actor_obs, b.action, b.done, b.lpf0, b.old_log_probs, b.advantages, y_s, sd_s, log_probs,
+                   ((ct ? actor_head_fwd_bwd_block_kernel<true> : actor_head_fwd_bwd_block_kernel<false>)<<<unsigned(n), 128, head_smem, st>>>(
+                       h->p, L, hc, w[0].out, b.actor_obs, b.action, b.done, b.lpf0, b.old_log_probs, b.advantages, y_s, sd_s, log_probs,
                        entropy, w[0].dout, T, ld, n)));
       else
         KBS_LAUNCH(h, KBS_K_ACTOR_HEAD, st,
-                   (actor_head_fwd_bwd_warp_kernel<<<unsigned((n + 3) / 4), 128, 0, st>>>(
-                       h->p, L, w[0].out, b.actor_obs, b.action, b.done, b.lpf0, b.old_log_probs, b.advantages, y_s, sd_s, log_probs,
+                   ((ct ? actor_head_fwd_bwd_warp_kernel<true> : actor_head_fwd_bwd_warp_kernel<false>)<<<unsigned((n + 3) / 4), 128, 0, st>>>(
+                       h->p, L, hc, w[0].out, b.actor_obs, b.action, b.done, b.lpf0, b.old_log_probs, b.advantages, y_s, sd_s, log_probs,
                        entropy, w[0].dout, T, ld, n)));
     }
     if (rank1_critic) {
       KBS_LAUNCH(h, KBS_K_CRITIC_HEAD, st,
-                 (critic_value_head_kernel<<<unsigned((rows + 7) / 8), 256, 0, st>>>(L, w[1].h_top_rm, h->net[1].w_out, h->net[1].b_out,
+                 ((ct ? critic_value_head_kernel<true> : critic_value_head_kernel<false>)<<<unsigned((rows + 7) / 8), 256, 0, st>>>(L, hc, w[1].h_top_rm, h->net[1].w_out, h->net[1].b_out,
                                                                                     b.old_values, b.value_targets, values, w[1].dout,
                                                                                     w[1].out /*dv*/, H, T, ld, n)));
     } else {
       if ((rc = kbs_simt_gemm_nt(h, w[1].h_top_rm, H, h->net[1].w_out, H, h->net[1].b_out, w[1].out, 64, rows, 64, H, 0, st))) return rc;
       KBS_LAUNCH(h, KBS_K_CRITIC_HEAD, st,
-                 (critic_head_fwd_bwd_kernel<<<blocks(rows), kT, 0, st>>>(L, w[1].out, b.old_values, b.value_targets, values, w[1].dout, T, ld, n)));
+                 ((ct ? critic_head_fwd_bwd_kernel<true> : critic_head_fwd_bwd_kernel<false>)<<<blocks(rows), kT, 0, st>>>(L, hc, w[1].out, b.old_values, b.value_targets, values, w[1].dout, T, ld, n)));
     }
   } else {
     KbsTcRolloutArgs r{};
@@ -1046,10 +1197,10 @@ int ppo_grad_persistent(kbs_handle* h, const kbs_ppo_loss_params& L, const kbs_p
     for (int k = 0; k < 2; ++k) { r.xmid_hist[k] = w[k].xmid; r.hsb_hist[k] = w[k].hsb; r.c_hist[k] = w[k].c_hist; r.save_g[k] = w[k].save_g; }
     if ((rc = kbs_tc_rollout_recurrent(h, r, st))) return rc;
     KBS_LAUNCH(h, KBS_K_ACTOR_HEAD, st,
-               (actor_head_bwd_warp_kernel<<<unsigned((n + 3) / 4), 128, 0, st>>>(h->p, L, b.action, b.done, b.old_log_probs, b.advantages,
+               ((ct ? actor_head_bwd_warp_kernel<true> : actor_head_bwd_warp_kernel<false>)<<<unsigned((n + 3) / 4), 128, 0, st>>>(h->p, L, hc, b.action, b.done, b.old_log_probs, b.advantages,
                                                                                  y_s, sd_s, sraw_s, log_probs, w[0].dout, T, ld, n)));
     KBS_LAUNCH(h, KBS_K_CRITIC_HEAD, st,
-               (critic_head_bwd_kernel<<<blocks(rows), kT, 0, st>>>(L, values, b.old_values, b.value_targets, w[1].dout, T, ld, n)));
+               ((ct ? critic_head_bwd_kernel<true> : critic_head_bwd_kernel<false>)<<<blocks(rows), kT, 0, st>>>(L, hc, values, b.old_values, b.value_targets, w[1].dout, T, ld, n)));
   }
   // ---- side stream, second part: what the forward pass produced and the weight-gradient GEMMs read with K = row (the
   // top layer's outputs; [x | h_in] of every layer unless the forward kernel re-packed them itself), while the backward
@@ -1144,13 +1295,14 @@ int ppo_grad_persistent(kbs_handle* h, const kbs_ppo_loss_params& L, const kbs_p
       float* const dst2[2] = {g->w_in, g->b_in};
       if ((rc = kbs_tc_tn_reduce_multi(h, plan, w[k].tn_partial, mp, kpp, H, 2, sg2, dst2, sk))) return rc;
     }
+    if ((rc = ct_rescale(h, hc, k, g, sk))) return rc;
     if (k == 1) {
       if (h->ev_critic_ready) KBS_CUDA_TRY(cudaEventRecord(h->ev_critic_ready, sk));   // the critic's gradients are final
       if (side_pack) KBS_CUDA_TRY(cudaEventRecord(h->ev_chunk[0], ss));
     }
   }
   if (side_pack) KBS_CUDA_TRY(cudaStreamWaitEvent(st, h->ev_chunk[0], 0));        // join: both networks' gradients are final
-  {
+  if (!ct) {
     kbs_ppo_loss_io io{};
     io.log_probs = log_probs; io.old_log_probs = b.old_log_probs; io.advantages = b.advantages; io.values = values;
     io.old_values = b.old_values; io.value_targets = b.value_targets; io.entropy = entropy; io.out = stats_out;
@@ -1330,16 +1482,13 @@ int kbs_launch_shuffle_minibatches(kbs_handle* h, const int32_t* perm, const kbs
   return KBS_OK;
 }
 
-extern "C" {
+namespace {
 
-int kbs_ppo_grad(kbs_handle* h, const kbs_ppo_loss_params* params, const kbs_ppo_batch* b, const kbs_net_grads* actor,
+// kbs_ppo_grad (ct == nullptr: d loss / d head outputs from the loss, statistics into stats_out) and kbs_ppo_variables_vjp (ct:
+// the caller's cotangents; L and stats_out unused).  Both entry points check their arguments first.
+int ppo_grad_run(kbs_handle* h, const kbs_ppo_loss_params& L, const kbs_ppo_batch* b, const kbs_net_grads* actor,
                  const kbs_net_grads* critic, float* log_probs, float* values, float* entropy, float* stats_out, int64_t n,
-                 void* stream) {
-  if (!h || !params || !b || !actor || !critic || !log_probs || !values || !entropy || !stats_out) return KBS_E_NULL;
-  if (!b->actor_obs || !b->critic_obs || !b->action || !b->done || !b->old_log_probs || !b->advantages || !b->value_targets ||
-      !b->old_values)
-    return KBS_E_NULL;
-  if (b->T <= 0 || n <= 0 || b->ld < n || (b->ld & 3)) return KBS_E_SHAPE;
+                 void* stream, const kbs_ppo_cotangents* ct) {
   for (int k = 0; k < 2; ++k)
     if (!h->net[k].packed) return KBS_E_STATE;
   { const int rc0 = kbs_enter(h); if (rc0) return rc0; }
@@ -1350,7 +1499,7 @@ int kbs_ppo_grad(kbs_handle* h, const kbs_ppo_loss_params* params, const kbs_ppo
     const char* e = getenv("KBS_PPO_PER_STEP");
     if (!(e && atoi(e)) && h->p.gemm_path == KBS_GEMM_TC_2XF16 && h->p.depth <= 2 && kbs_tc_bptt_available(h, n, b->T)) {
       const kbs_net_grads* gr[2] = {actor, critic};
-      return ppo_grad_persistent(h, *params, *b, gr, log_probs, values, entropy, stats_out, n, st);
+      return ppo_grad_persistent(h, L, *b, gr, log_probs, values, entropy, stats_out, n, st, ct);
     }
   }
   const int H = h->p.hidden_size, depth = h->p.depth;
@@ -1362,6 +1511,7 @@ int kbs_ppo_grad(kbs_handle* h, const kbs_ppo_loss_params* params, const kbs_ppo
   const bool tc = h->p.gemm_path != KBS_GEMM_SIMT_FP32;
   const size_t part_f = size_t(chunks) * 4 * H + size_t(splits) * size_t(4 * H) * size_t(kp_max) + size_t(H) * kp_max + 64 * H + 4096;
   float* gates_pre[2]; float* dc_rec[2]; float* part[2]; float *y_s, *sd_s;
+  unsigned int* amax;
   NetWork w[2];
   int rc = kbs_scratch(h, [&](KbsScratch& s) {
     for (int k = 0; k < 2; ++k) {            // per net: actor and critic run concurrently on two streams
@@ -1408,12 +1558,15 @@ int kbs_ppo_grad(kbs_handle* h, const kbs_ppo_loss_params* params, const kbs_ppo
         w[k].tn_ones = s.take<char>(4096 * sizeof(float));
       }
     }
+    amax = s.take<unsigned int>(2);
   });
   if (rc) return rc;
   // The two networks share nothing until the loss statistics: the critic runs on the handle's side stream, forked from
   // and joined into the caller's stream with events (capturable: the whole call can be replayed as one CUDA graph).
   { const int rc0 = kbs_side_stream_init(h); if (rc0) return rc0; }
   cudaStream_t sc = h->side_stream;
+  HeadCt hc;
+  if ((rc = ct_begin(h, ct, amax, T, ld, n, st, &hc))) return rc;
   KBS_CUDA_TRY(cudaEventRecord(h->ev_pre, st));
   KBS_CUDA_TRY(cudaStreamWaitEvent(sc, h->ev_pre, 0));
   // forward with saved activations
@@ -1425,29 +1578,55 @@ int kbs_ppo_grad(kbs_handle* h, const kbs_ppo_loss_params* params, const kbs_ppo
     return rc;
   // heads: outputs, loss gradient wrt the head outputs
   KBS_LAUNCH(h, KBS_K_ACTOR_HEAD, st,
-             (actor_head_fwd_bwd_warp_kernel<<<unsigned((n + 3) / 4), 128, 0, st>>>(
-                 h->p, *params, w[0].out, b->actor_obs, b->action, b->done, b->lpf0, b->old_log_probs, b->advantages, y_s, sd_s,
+             ((ct ? actor_head_fwd_bwd_warp_kernel<true> : actor_head_fwd_bwd_warp_kernel<false>)<<<unsigned((n + 3) / 4), 128, 0, st>>>(
+                 h->p, L, hc, w[0].out, b->actor_obs, b->action, b->done, b->lpf0, b->old_log_probs, b->advantages, y_s, sd_s,
                  log_probs, entropy, w[0].dout, T, ld, n)));
   KBS_LAUNCH(h, KBS_K_CRITIC_HEAD, sc,
-             (critic_head_fwd_bwd_kernel<<<blocks(rows), kT, 0, sc>>>(*params, w[1].out, b->old_values, b->value_targets, values,
+             ((ct ? critic_head_fwd_bwd_kernel<true> : critic_head_fwd_bwd_kernel<false>)<<<blocks(rows), kT, 0, sc>>>(L, hc, w[1].out, b->old_values, b->value_targets, values,
                                                                       w[1].dout, T, ld, n)));
   // critic backward on the side stream
   if ((rc = run_net(h, KBS_NET_CRITIC, *b, nullptr, w[1], gates_pre[1], dc_rec[1], part[1], splits, n, sc, true, critic)))
     return rc;
+  if ((rc = ct_rescale(h, hc, 1, critic, sc))) return rc;
   KBS_CUDA_TRY(cudaEventRecord(h->ev_head[0], sc));
   if ((rc = run_net(h, KBS_NET_ACTOR, *b, nullptr, w[0], gates_pre[0], dc_rec[0], part[0], splits, n, st, true, actor)))
     return rc;
+  if ((rc = ct_rescale(h, hc, 0, actor, st))) return rc;
   KBS_CUDA_TRY(cudaStreamWaitEvent(st, h->ev_head[0], 0));       // join: values + critic gradients are complete
   if (h->ev_critic_ready) KBS_CUDA_TRY(cudaEventRecord(h->ev_critic_ready, st));
   // loss statistics (same kernel as kbs_ppo_loss; partials in the actor's reduction scratch, free again by now)
-  {
+  if (!ct) {
     kbs_ppo_loss_io io{};
     io.log_probs = log_probs; io.old_log_probs = b->old_log_probs; io.advantages = b->advantages; io.values = values;
     io.old_values = b->old_values; io.value_targets = b->value_targets; io.entropy = entropy; io.out = stats_out;
     io.T = T; io.ld = ld;
-    if ((rc = kbs_launch_ppo_loss_at(h, *params, io, n, reinterpret_cast<double*>(part[0]), st))) return rc;
+    if ((rc = kbs_launch_ppo_loss_at(h, L, io, n, reinterpret_cast<double*>(part[0]), st))) return rc;
   }
   return KBS_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int kbs_ppo_grad(kbs_handle* h, const kbs_ppo_loss_params* params, const kbs_ppo_batch* b, const kbs_net_grads* actor,
+                 const kbs_net_grads* critic, float* log_probs, float* values, float* entropy, float* stats_out, int64_t n,
+                 void* stream) {
+  if (!h || !params || !b || !actor || !critic || !log_probs || !values || !entropy || !stats_out) return KBS_E_NULL;
+  if (!b->actor_obs || !b->critic_obs || !b->action || !b->done || !b->old_log_probs || !b->advantages || !b->value_targets ||
+      !b->old_values)
+    return KBS_E_NULL;
+  if (b->T <= 0 || n <= 0 || b->ld < n || (b->ld & 3)) return KBS_E_SHAPE;
+  return ppo_grad_run(h, *params, b, actor, critic, log_probs, values, entropy, stats_out, n, stream, nullptr);
+}
+
+int kbs_ppo_variables_vjp(kbs_handle* h, const kbs_ppo_batch* b, const kbs_ppo_cotangents* ct, const kbs_net_grads* actor,
+                          const kbs_net_grads* critic, float* log_probs, float* values, float* entropy, int64_t n, void* stream) {
+  if (!h || !b || !ct || !actor || !critic || !log_probs || !values || !entropy) return KBS_E_NULL;
+  if (!b->actor_obs || !b->critic_obs || !b->action || !b->done) return KBS_E_NULL;
+  if (b->T <= 0 || n <= 0 || b->ld < n || (b->ld & 3)) return KBS_E_SHAPE;
+  const kbs_ppo_loss_params unused{};
+  return ppo_grad_run(h, unused, b, actor, critic, log_probs, values, entropy, nullptr, n, stream, ct);
 }
 
 int kbs_adam_step(kbs_handle* h, float* param, const float* grad, float* m, float* v, int64_t count, float lr, float b1, float b2,

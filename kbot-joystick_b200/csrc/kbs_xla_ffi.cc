@@ -277,6 +277,14 @@ ffi::Error RewardsImpl(cudaStream_t stream, int64_t handle, int64_t n_envs, F32 
 
 // ---- jax.grad of the PPO minibatch loss (train.py:1435-1524 under jax.grad; ksim.compute_ppo_loss) ----------------------------
 // grads: ONE flat f32 buffer per network in the order w_in, b_in, (w_ih, w_hh, b) per layer, w_out, b_out (ppo.NetParams)
+void GradViews(float* p, int64_t hidden, int64_t depth, int64_t num_in, int64_t num_out, kbs_net_grads* g) {
+  const int64_t Hh = hidden;
+  g->w_in = p; p += Hh * num_in; g->b_in = p; p += Hh;
+  for (int64_t l = 0; l < depth && l < KBS_MAX_DEPTH; ++l) {
+    g->w_ih[l] = p; p += 4 * Hh * Hh; g->w_hh[l] = p; p += 4 * Hh * Hh; g->b[l] = p; p += 4 * Hh;
+  }
+  g->w_out = p; p += num_out * Hh; g->b_out = p;
+}
 ffi::Error PpoGradImpl(cudaStream_t stream, int64_t handle, int64_t n_envs, int64_t hidden, int64_t depth, F32 actor_obs,
                        F32 critic_obs, F32 action, U8 done, F32 old_log_probs, F32 advantages, F32 value_targets, F32 old_values,
                        F32 actor_carry0, F32 critic_carry0, F32 lpf0, RF32 grad_actor, RF32 grad_critic, RF32 log_probs, RF32 values,
@@ -289,19 +297,30 @@ ffi::Error PpoGradImpl(cudaStream_t stream, int64_t handle, int64_t n_envs, int6
   b.value_targets = value_targets.typed_data(); b.old_values = old_values.typed_data();
   b.actor_carry0 = actor_carry0.typed_data(); b.critic_carry0 = critic_carry0.typed_data(); b.lpf0 = lpf0.typed_data();
   b.T = Dim(actor_obs, 0); b.ld = Dim(actor_obs, 2);
-  auto views = [&](float* p, int64_t num_in, int64_t num_out, kbs_net_grads* g) {
-    const int64_t Hh = hidden;
-    g->w_in = p; p += Hh * num_in; g->b_in = p; p += Hh;
-    for (int64_t l = 0; l < depth && l < KBS_MAX_DEPTH; ++l) {
-      g->w_ih[l] = p; p += 4 * Hh * Hh; g->w_hh[l] = p; p += 4 * Hh * Hh; g->b[l] = p; p += 4 * Hh;
-    }
-    g->w_out = p; p += num_out * Hh; g->b_out = p;
-  };
   kbs_net_grads ga{}, gc{};
-  views(grad_actor->typed_data(), KBS_ACTOR_OBS, KBS_ACTOR_OUT, &ga);
-  views(grad_critic->typed_data(), KBS_CRITIC_OBS, 1, &gc);
+  GradViews(grad_actor->typed_data(), hidden, depth, KBS_ACTOR_OBS, KBS_ACTOR_OUT, &ga);
+  GradViews(grad_critic->typed_data(), hidden, depth, KBS_CRITIC_OBS, 1, &gc);
   return Rc(kbs_ppo_grad(H(handle), &lp, &b, &ga, &gc, log_probs->typed_data(), values->typed_data(), entropy->typed_data(),
                          stats->typed_data(), n_envs, stream));
+}
+
+// ---- VJP of get_ppo_variables (train.py:1484-1487): the backward rule of a jax.custom_vjp around it (INTEGRATION.md) ----------
+// ct_*: the cotangents of log_probs / values / entropy [T][ld] and action_std [T][20][ld]; grads flat as for KbsPpoGrad
+ffi::Error PpoVariablesVjpImpl(cudaStream_t stream, int64_t handle, int64_t n_envs, int64_t hidden, int64_t depth, F32 actor_obs,
+                               F32 critic_obs, F32 action, U8 done, F32 actor_carry0, F32 critic_carry0, F32 lpf0, F32 ct_log_probs,
+                               F32 ct_values, F32 ct_entropy, F32 ct_action_std, RF32 grad_actor, RF32 grad_critic, RF32 log_probs,
+                               RF32 values, RF32 entropy) {
+  kbs_ppo_batch b{};
+  b.actor_obs = actor_obs.typed_data(); b.critic_obs = critic_obs.typed_data(); b.action = action.typed_data();
+  b.done = done.typed_data();
+  b.actor_carry0 = actor_carry0.typed_data(); b.critic_carry0 = critic_carry0.typed_data(); b.lpf0 = lpf0.typed_data();
+  b.T = Dim(actor_obs, 0); b.ld = Dim(actor_obs, 2);
+  kbs_ppo_cotangents ct{ct_log_probs.typed_data(), ct_values.typed_data(), ct_entropy.typed_data(), ct_action_std.typed_data()};
+  kbs_net_grads ga{}, gc{};
+  GradViews(grad_actor->typed_data(), hidden, depth, KBS_ACTOR_OBS, KBS_ACTOR_OUT, &ga);
+  GradViews(grad_critic->typed_data(), hidden, depth, KBS_CRITIC_OBS, 1, &gc);
+  return Rc(kbs_ppo_variables_vjp(H(handle), &b, &ct, &ga, &gc, log_probs->typed_data(), values->typed_data(),
+                                  entropy->typed_data(), n_envs, stream));
 }
 
 // ---- optax.global_norm + optax.adamw with ksim's clip (train.py:1059-1065) on one flat parameter vector ------------------------
@@ -375,6 +394,10 @@ XLA_FFI_DEFINE_HANDLER_SYMBOL(KbsPpoGrad, PpoGradImpl,
                               KBS_BIND_N().Attr<int64_t>("hidden").Attr<int64_t>("depth")
                                   .Arg<F32>().Arg<F32>().Arg<F32>().Arg<U8>().Arg<F32>().Arg<F32>().Arg<F32>().Arg<F32>().Arg<F32>()
                                   .Arg<F32>().Arg<F32>().Ret<F32>().Ret<F32>().Ret<F32>().Ret<F32>().Ret<F32>().Ret<F32>());
+XLA_FFI_DEFINE_HANDLER_SYMBOL(KbsPpoVariablesVjp, PpoVariablesVjpImpl,
+                              KBS_BIND_N().Attr<int64_t>("hidden").Attr<int64_t>("depth")
+                                  .Arg<F32>().Arg<F32>().Arg<F32>().Arg<U8>().Arg<F32>().Arg<F32>().Arg<F32>().Arg<F32>().Arg<F32>()
+                                  .Arg<F32>().Arg<F32>().Ret<F32>().Ret<F32>().Ret<F32>().Ret<F32>().Ret<F32>());
 XLA_FFI_DEFINE_HANDLER_SYMBOL(KbsGradNorm, GradNormImpl, KBS_BIND().Arg<F32>().Ret<F32>());
 XLA_FFI_DEFINE_HANDLER_SYMBOL(KbsAdamwStep, AdamwStepImpl,
                               KBS_BIND().Attr<float>("lr").Attr<float>("weight_decay").Attr<float>("grad_scale").Attr<float>("max_grad_norm")

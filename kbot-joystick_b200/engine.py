@@ -45,6 +45,26 @@ def _view(cls, rows: dict, tensors: dict | None, ld: int | None = None, host: bo
     return v
 
 
+def _ppo_batch(batch: dict):
+    """kbs_ppo_batch over a minibatch dict ([T, F, ld] arrays; missing keys are NULL)."""
+    T, _, ld = batch["actor_obs"].shape
+    b = L.KbsPpoBatch()
+    for k in ("actor_obs", "critic_obs", "action", "done", "old_log_probs", "advantages", "value_targets", "old_values",
+              "actor_carry0", "critic_carry0", "lpf0"):
+        setattr(b, k, L.ptr(batch.get(k)))
+    b.T, b.ld = T, ld
+    return b
+
+
+def _net_grads(g: dict):
+    """kbs_net_grads over an eqx-layout dict of gradient tensors."""
+    s = L.KbsNetGrads()
+    s.w_in, s.b_in, s.w_out, s.b_out = (L.ptr(g[k]) for k in ("w_in", "b_in", "w_out", "b_out"))
+    for i, lw in enumerate(g["layers"]):
+        s.w_ih[i], s.w_hh[i], s.b[i] = L.ptr(lw["w_ih"]), L.ptr(lw["w_hh"]), L.ptr(lw["b"])
+    return s
+
+
 @dataclass
 class KbotStep:
     """One handle of the B200 control-step library bound to the current CUDA device."""
@@ -171,20 +191,8 @@ class KbotStep:
         L.check(self.lib.kbs_ppo_loss_default_params(C.byref(lp)), "kbs_ppo_loss_default_params")
         for k, v in hyper.items():
             setattr(lp, k, v)
-        b = L.KbsPpoBatch()
-        for k in ("actor_obs", "critic_obs", "action", "done", "old_log_probs", "advantages", "value_targets", "old_values",
-                  "actor_carry0", "critic_carry0", "lpf0"):
-            setattr(b, k, L.ptr(batch.get(k)))
-        b.T, b.ld = T, ld
-
-        def gview(g):
-            s = L.KbsNetGrads()
-            s.w_in, s.b_in, s.w_out, s.b_out = (L.ptr(g[k]) for k in ("w_in", "b_in", "w_out", "b_out"))
-            for i, lw in enumerate(g["layers"]):
-                s.w_ih[i], s.w_hh[i], s.b[i] = L.ptr(lw["w_ih"]), L.ptr(lw["w_hh"]), L.ptr(lw["b"])
-            return s
-
-        ga, gc = gview(grads_actor), gview(grads_critic)
+        b = _ppo_batch(batch)
+        ga, gc = _net_grads(grads_actor), _net_grads(grads_critic)
         # critic_ready: a torch.cuda.Event the library records on the stream once the critic's gradients are final (its
         # all-reduce can then overlap the actor's weight-gradient GEMMs)
         L.check(self.lib.kbs_ppo_grad_set_events(self._h, critic_ready.cuda_event if critic_ready is not None else None),
@@ -194,6 +202,28 @@ class KbotStep:
         L.check(self.lib.kbs_ppo_grad(self._h, C.byref(lp), C.byref(b), C.byref(ga), C.byref(gc), L.ptr(out["log_probs"]),
                                       L.ptr(out["values"]), L.ptr(out["entropy"]), L.ptr(out["stats"]), n_envs or ld, _stream()),
                 "kbs_ppo_grad")
+        return out
+
+    def ppo_variables_vjp(self, batch: dict, cotangents: dict, grads_actor: dict, grads_critic: dict, n_envs: int | None = None,
+                          critic_ready=None) -> dict:
+        """Vector-Jacobian product of the PPO variables (kbs_ppo_variables_vjp): grads_* (written, eqx layout) = the gradient
+        of sum(ct * var) over the minibatch for cotangents {"log_probs", "values", "entropy": [T, ld], "action_std":
+        [T, 20, ld]} (a missing key is a zero cotangent), through the same forward and BPTT as ppo_grad.  batch as for
+        ppo_grad; old_log_probs / advantages / value_targets / old_values are not read.  critic_ready as for ppo_grad.
+        Returns the forward's {"log_probs", "values", "entropy": [T, ld]}."""
+        T, _, ld = batch["actor_obs"].shape
+        dev = batch["actor_obs"].device
+        b = _ppo_batch(batch)
+        ct = L.KbsPpoCotangents()
+        for k in ("log_probs", "values", "entropy", "action_std"):
+            setattr(ct, k, L.ptr(cotangents.get(k)))
+        ga, gc = _net_grads(grads_actor), _net_grads(grads_critic)
+        L.check(self.lib.kbs_ppo_grad_set_events(self._h, critic_ready.cuda_event if critic_ready is not None else None),
+                "kbs_ppo_grad_set_events")
+        out = {k: torch.empty((T, ld), device=dev) for k in ("log_probs", "values", "entropy")}
+        L.check(self.lib.kbs_ppo_variables_vjp(self._h, C.byref(b), C.byref(ct), C.byref(ga), C.byref(gc),
+                                               L.ptr(out["log_probs"]), L.ptr(out["values"]), L.ptr(out["entropy"]),
+                                               n_envs or ld, _stream()), "kbs_ppo_variables_vjp")
         return out
 
     def adam_step(self, param, grad, m, v, step: int, lr=5e-4, b1=0.9, b2=0.999, eps=1e-8, grad_scale=1.0) -> None:

@@ -28,7 +28,7 @@ _TARGETS = {
     "kbs_rollout_record": "KbsRolloutRecord", "kbs_ppo_variables": "KbsPpoVariables",
     "kbs_mirror_observations": "KbsMirrorObservations", "kbs_mirror_joints": "KbsMirrorJoints",
     "kbs_com_distance": "KbsComDistance", "kbs_rewards": "KbsRewards", "kbs_ppo_grad": "KbsPpoGrad",
-    "kbs_grad_norm": "KbsGradNorm", "kbs_adamw_step": "KbsAdamwStep",
+    "kbs_grad_norm": "KbsGradNorm", "kbs_adamw_step": "KbsAdamwStep", "kbs_ppo_variables_vjp": "KbsPpoVariablesVjp",
 }
 STATE_ROWS = (("qpos", 27), ("qvel", 26), ("sensordata", 49), ("xpos", 72), ("xquat", 96), ("cinert", 240), ("cvel", 144),
               ("actuator_force", 20))
@@ -254,6 +254,23 @@ def ppo_grad(handle: int, batch: dict, actor_carry0, critic_carry0, lpf0, n_envs
     return jax.ffi.ffi_call("kbs_ppo_grad", out)(
         batch["actor_obs"], batch["critic_obs"], batch["action"], batch["done"].astype(jnp.uint8), batch["old_log_probs"],
         batch["advantages"], batch["value_targets"], batch["old_values"], actor_carry0, critic_carry0, lpf0,
+        **_h(np, handle, n_envs=n_envs, hidden=hidden, depth=depth))
+
+
+def ppo_variables_vjp(handle: int, batch: dict, actor_carry0, critic_carry0, lpf0, cotangents: dict, n_envs: int, hidden: int = 256,
+                      depth: int = 2):
+    """VJP of the PPO variables (kbs_ppo_variables_vjp), the backward rule of a jax.custom_vjp around get_ppo_variables:
+    batch = {actor_obs [T, 65, ld], critic_obs [T, 475, ld], action, done}, cotangents = {log_probs, values, entropy [T, ld],
+    action_std [T, 20, ld]} -> (grad_actor flat, grad_critic flat, log_probs, values, entropy [T, ld]); flat layout as ppo_grad.
+    The parameter cotangent is summed over the minibatch's envs: under vmap it must not be reduced again."""
+    jax, jnp, np = _j()
+    T, _, ld = batch["actor_obs"].shape
+    f32 = jnp.float32
+    out = (_sds(jax, (net_param_count(65, 40, hidden, depth),), f32), _sds(jax, (net_param_count(475, 1, hidden, depth),), f32)) + \
+        (_sds(jax, (T, ld), f32),) * 3
+    return jax.ffi.ffi_call("kbs_ppo_variables_vjp", out)(
+        batch["actor_obs"], batch["critic_obs"], batch["action"], batch["done"].astype(jnp.uint8), actor_carry0, critic_carry0, lpf0,
+        cotangents["log_probs"], cotangents["values"], cotangents["entropy"], cotangents["action_std"],
         **_h(np, handle, n_envs=n_envs, hidden=hidden, depth=depth))
 
 

@@ -102,20 +102,45 @@ class PpoUpdater:
         self.eng.pack_weights(L.NET_ACTOR, self.pa.as_dict(), sync=False)
         cur.wait_event(self.ev_comm)
 
-    def grads(self, batch: dict, n_envs: int, critic_ready=None) -> dict:
-        return self.eng.ppo_grad(batch, self.pa.as_dict(self.grad[:self.na]), self.pc.as_dict(self.grad[self.na:]), n_envs=n_envs,
-                                 critic_ready=critic_ready, **self.loss_hyper)
+    def grads(self, batch: dict, n_envs: int, critic_ready=None, loss_fn=None) -> dict:
+        ga, gc = self.pa.as_dict(self.grad[:self.na]), self.pc.as_dict(self.grad[self.na:])
+        if loss_fn is None:
+            return self.eng.ppo_grad(batch, ga, gc, n_envs=n_envs, critic_ready=critic_ready, **self.loss_hyper)
+        return self._loss_fn_grads(batch, n_envs, critic_ready, loss_fn, ga, gc)
 
-    def _step(self, batch: dict, n_envs: int) -> dict:
+    VARIABLES = ("log_probs", "values", "entropy", "action_std")
+
+    def _loss_fn_grads(self, batch: dict, n_envs: int, critic_ready, loss_fn, ga: dict, gc: dict) -> dict:
+        """The gradient of a caller's loss: kbs_ppo_variables from copies of the minibatch's start carries, the loss and its
+        cotangents by torch autograd, then kbs_ppo_variables_vjp.  The loss sees kbs_ppo_variables' forward and the gradient
+        is taken at the VJP's own forward; the two agree to fp32 rounding (as epoch() mixes kbs_ppo_variables' old values
+        with kbs_ppo_grad's gradients)."""
+        T, _, ld = batch["actor_obs"].shape
+        dev = batch["actor_obs"].device
+        shape = (self.eng.depth, 2, n_envs, self.eng.hidden_size)
+        carry = lambda k, s: batch[k].clone() if batch.get(k) is not None else torch.zeros(s, device=dev)
+        v = self.eng.ppo_variables(batch["actor_obs"], batch["action"], batch["done"], carry("actor_carry0", shape),
+                                   carry("lpf0", (L.NUM_JOINTS, ld)), batch["critic_obs"], carry("critic_carry0", shape),
+                                   n_envs=n_envs)
+        var = {k: v[k].detach().requires_grad_(True) for k in self.VARIABLES}
+        loss = loss_fn(var, batch)
+        cts = torch.autograd.grad(loss, [var[k] for k in self.VARIABLES], allow_unused=True)
+        out = self.eng.ppo_variables_vjp(batch, {k: c for k, c in zip(self.VARIABLES, cts) if c is not None}, ga, gc,
+                                         n_envs=n_envs, critic_ready=critic_ready)
+        nan = torch.full((3,), float("nan"), device=dev)
+        out["stats"] = torch.cat([loss.detach().reshape(1).float(), nan])
+        return out
+
+    def _step(self, batch: dict, n_envs: int, loss_fn=None) -> dict:
         """One whole update, enqueued on the current stream (+ the communication stream, forked from / joined into it)."""
         import torch.distributed as dist
 
         world = dist.get_world_size() if (dist.is_available() and dist.is_initialized()) else 1
         if world == 1:
-            out = self.grads(batch, n_envs)
+            out = self.grads(batch, n_envs, loss_fn=loss_fn)
         else:
             cur = torch.cuda.current_stream()
-            out = self.grads(batch, n_envs, critic_ready=self.ev_critic)
+            out = self.grads(batch, n_envs, critic_ready=self.ev_critic, loss_fn=loss_fn)
             with torch.cuda.stream(self.comm_stream):
                 self.comm_stream.wait_event(self.ev_critic)          # the critic's gradients are final: reduce them now
                 dist.all_reduce(self.grad[self.na:], op=dist.ReduceOp.SUM)
@@ -128,21 +153,27 @@ class PpoUpdater:
         self._repack()
         return out
 
-    def capture(self, batch: dict, n_envs: int) -> None:
-        """Record one whole update on `batch` as ONE CUDA graph; later update() calls with the same batch object replay it
-        (refill the batch tensors in place between updates).  Call after at least one eager update (allocations, NCCL)."""
+    def capture(self, batch: dict, n_envs: int, loss_fn=None) -> None:
+        """Record one whole update on `batch` as ONE CUDA graph; later update() calls with the same batch object and loss_fn
+        replay it (refill the batch tensors in place between updates).  Call after at least one eager update (allocations,
+        NCCL).  A loss_fn is captured with it: it must enqueue device work only."""
         torch.cuda.synchronize()
         self._graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self._graph):
-            self._graph_out = self._step(batch, n_envs)
-        self._graph_batch = batch
+            self._graph_out = self._step(batch, n_envs, loss_fn)
+        self._graph_batch, self._graph_loss_fn = batch, loss_fn
         self.eng.scratch_lock(True)        # the graph holds pointers into the library's scratch: it must not be reallocated
 
-    def update(self, batch: dict, n_envs: int) -> dict:
-        if self._graph is not None and batch is self._graph_batch:
+    def update(self, batch: dict, n_envs: int, loss_fn=None) -> dict:
+        """One whole update on a minibatch.  loss_fn=None: the library's PPO loss (kbs_ppo_grad).  Otherwise
+        loss = loss_fn(vars, batch), a scalar tensor, where vars holds "log_probs", "values", "entropy" [T, ld] and "action_std"
+        [T, 20, ld] as tensors that require grad and batch is the minibatch dict (old_log_probs, advantages, ...): its gradient
+        comes from torch autograd for the cotangents and kbs_ppo_variables_vjp for the parameters (see _loss_fn_grads).  Only
+        columns < n_envs reach the gradient.  Returns the forward outputs and "stats" ([loss, nan, nan, nan] with a loss_fn)."""
+        if self._graph is not None and batch is self._graph_batch and loss_fn is self._graph_loss_fn:
             self._graph.replay()
             return self._graph_out
-        return self._step(batch, n_envs)
+        return self._step(batch, n_envs, loss_fn)
 
     # ---- the update phase of an epoch -----------------------------------------------------------------------------------------
     def _epoch_work(self, rollout: dict, n_envs: int, batch_size: int, num_passes: int) -> dict:
@@ -163,7 +194,7 @@ class PpoUpdater:
         self._ework = w
         return w
 
-    def _epoch(self, rollout: dict, n_envs: int, batch_size: int, num_passes: int, seed: int) -> dict:
+    def _epoch(self, rollout: dict, n_envs: int, batch_size: int, num_passes: int, seed: int, loss_fn=None) -> dict:
         """One epoch's update phase, enqueued on the current stream (SURVEY 3.1): kbs_ppo_variables from the rollout's start
         carries -> kbs_gae -> per pass: permutation, shuffle into minibatches, one whole update per minibatch."""
         import torch.distributed as dist
@@ -185,35 +216,37 @@ class PpoUpdater:
             self.eng.minibatch_permutation(self.pass_dev, n_envs, seed=seed, env0=rank * n_envs, out=w["perm"][p])
             self.eng.shuffle_minibatches(w["perm"][p], src, n_envs, batch_size, dst=mb)
             for b in range(nb):
-                out = self._step({k: t[b] for k, t in mb.items()}, batch_size)
+                out = self._step({k: t[b] for k, t in mb.items()}, batch_size, loss_fn)
                 w["stats"][p * nb + b].copy_(out["stats"])
                 w["norms"][p * nb + b:p * nb + b + 1].copy_(self.norm)
         return {"stats": w["stats"], "norms": w["norms"], "perm": w["perm"]}
 
-    def epoch(self, rollout: dict, n_envs: int, batch_size: int = 512, num_passes: int = 3, seed: int = 0) -> dict:
+    def epoch(self, rollout: dict, n_envs: int, batch_size: int = 512, num_passes: int = 3, seed: int = 0, loss_fn=None) -> dict:
         """The update phase of one PPO epoch on a stored rollout: num_passes x (n_envs / batch_size) updates (train.py:1763-1766),
         each on a minibatch of whole trajectories taken from a fresh device-drawn permutation of the env axis.
         rollout: actor_obs [T,65,ld], critic_obs [T,475,ld], action [T,20,ld], done / success u8 [T,ld], rewards [T,ld], and the
         carries at the rollout's first step (snapshot them before kbs_rollout, which advances them): actor_carry0 /
         critic_carry0 [depth,2,n_envs,H], lpf0 [20,ld].  Returns device tensors, overwritten by the next epoch: "stats"
         [P*B, 4] loss statistics and "norms" [P*B] gradient norms per update, "perm" [P, n_envs] the permutations.  No host
-        synchronisation.  After capture_epoch, a call on the same rollout object with the same arguments replays the graph."""
+        synchronisation.  After capture_epoch, a call on the same rollout object with the same arguments replays the graph.
+        loss_fn: as for update(), for every update of the epoch."""
         if self._epoch_graph is not None and rollout is self._epoch_rollout and \
-                self._epoch_args == (n_envs, batch_size, num_passes, seed):
+                self._epoch_args == (n_envs, batch_size, num_passes, seed, loss_fn):
             self._epoch_graph.replay()
             return self._epoch_out
-        return self._epoch(rollout, n_envs, batch_size, num_passes, seed)
+        return self._epoch(rollout, n_envs, batch_size, num_passes, seed, loss_fn)
 
-    def capture_epoch(self, rollout: dict, n_envs: int, batch_size: int = 512, num_passes: int = 3, seed: int = 0) -> None:
+    def capture_epoch(self, rollout: dict, n_envs: int, batch_size: int = 512, num_passes: int = 3, seed: int = 0,
+                      loss_fn=None) -> None:
         """Record one whole epoch() on `rollout` as ONE CUDA graph; later epoch() calls with the same rollout object and
         arguments replay it (refill the rollout tensors in place between epochs).  Call after one eager epoch with the same
         arguments: the handle's scratch has then grown to what kbs_ppo_variables and kbs_ppo_grad need, and is locked here."""
         torch.cuda.synchronize()
         self._epoch_graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self._epoch_graph):
-            self._epoch_out = self._epoch(rollout, n_envs, batch_size, num_passes, seed)
+            self._epoch_out = self._epoch(rollout, n_envs, batch_size, num_passes, seed, loss_fn)
         self._epoch_rollout = rollout
-        self._epoch_args = (n_envs, batch_size, num_passes, seed)
+        self._epoch_args = (n_envs, batch_size, num_passes, seed, loss_fn)
         self._epoch_graph_work = self._ework       # the graph holds its buffers' addresses: keep them if the shapes change
         self.eng.scratch_lock(True)
 
